@@ -2,6 +2,7 @@
 """Benchmark of the mc3 sampling hot path (BASELINE.json metric: chain-steps/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 Workload (N=1 and per GPU at N>1, weak scaling): BASELINE config 2 -- DEMC,
 4096 chains per GPU, 5-parameter sinusoid+line model, 1e5 data points, fp64
@@ -23,6 +24,10 @@ One JSON line on stdout (rank 0):
              the host cores: a bounded sample of the same workload
 
 --impl reference prints the same line for the CPU reference arm.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed generation
+computed (posterior rows, log-posterior, chi-squared, best parameters) as
+DIR/<name>.npy in float64; the inputs are seeded, so two builds can be compared.
 """
 import argparse
 import contextlib
@@ -310,7 +315,10 @@ def run_ours(args):
     ms_total = float(t.item())
     launches = pop.launches - launches0
     value = nchains*K/(ms_total*1e-3)
-    acc = pop.counters()['numaccept']
+    cnt = pop.counters()
+    acc = cnt['numaccept']
+    if args.dump_outputs:
+        dump_outputs(pop, cnt, rank, args.dump_outputs)
 
     # ---- roofline of the dominant kernel, timed alone -------------------
     roof = None
@@ -472,6 +480,22 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(pop, counters, rank, outdir):
+    """Write what the last timed generation computed, as a caller of Population.run()
+    reads it: the history rows it wrote (posterior sample, log-posterior and chi-squared
+    of every chain) and the best parameters so far.  The inputs are seeded, so two
+    builds run with the same arguments can be compared array for array."""
+    posterior, _, log_post, chisq = pop.history_host(dst=0)    # collective at world > 1
+    if rank != 0:
+        return
+    n = pop.nchains                      # thinning 1: one row per chain and generation
+    out = {'posterior': posterior[-n:], 'log_post': log_post[-n:], 'chisq': chisq[-n:],
+           'bestp': counters['bestp']}
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(outdir, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 def multi_gpu_parity(args, w, model, rank, world, dev):
     """Driver-visible check that N devices compute what one device computes: a short
     fixed-seed config-2 population (4096 chains in total, N=1e5: TMA path, decreasing
@@ -553,7 +577,11 @@ def main():
     ap.add_argument('--dtype', default='f64', choices=['f64', 'f32'])
     ap.add_argument('--cpu-steps', type=int, default=2000)
     ap.add_argument('--no-cpu', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     # stdout carries exactly one JSON line: everything libraries print on fd 1 while
     # the run lasts (NCCL's version banner, the hub's greeting) goes to stderr.
     global _OUT
