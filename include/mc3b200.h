@@ -4,7 +4,8 @@
  * Every entry point returns an int status (MC3B_OK on success); the message of
  * the last failure on the calling thread is available from mc3b_last_error().
  * All pointers are DEVICE pointers unless a parameter is marked [host].  The
- * caller owns every buffer; the library allocates nothing persistent.
+ * caller owns every buffer; the library allocates nothing persistent except the
+ * peer buffers and user-model handles it hands out (see below).
  * `stream` is a cudaStream_t passed as void* (NULL = default stream).  Calls
  * are asynchronous with respect to the host and re-entrant per stream.
  *
@@ -22,7 +23,18 @@
 #ifndef MC3B200_H
 #define MC3B200_H
 
+#ifdef __CUDACC_RTC__
+/* NVRTC (user models compiled at run time) has no <stdint.h>: the LP64 types */
+typedef signed char int8_t;
+typedef unsigned char uint8_t;
+typedef int int32_t;
+typedef unsigned int uint32_t;
+typedef long int64_t;
+typedef unsigned long uint64_t;
+typedef unsigned long uintptr_t;
+#else
 #include <stdint.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -221,6 +233,50 @@ int mc3b_model_eval(int model_id, const double* params, int64_t ldp,
                     int64_t nchains, int nmodel, const double* x, int64_t n,
                     double* out, void* stream);
 
+/* ------------------------------------------------------------------------
+ * User models compiled at run time   (the user's own `func`, chain.py:316-319)
+ *
+ * The source defines  __device__ real model(real x, const real* p)  (p[0..nmodel)),
+ * with `real` = double (dtype F64) or float (F32); helpers above it are allowed and
+ * models.cuh (fast_sin, fast_sincos_core, ...) is included.  NVRTC compiles it into
+ * the kernels of the built-in models (csrc/chisq_kernel.cuh), so the model runs on the
+ * same fused, TMA-staged, graph-capturable path.
+ * ---------------------------------------------------------------------- */
+typedef struct mc3b_user_model mc3b_user_model_t;          /* opaque */
+
+/* source -> sm_100a CUBIN, with the NVRTC library at nvrtc_path (dlopen'ed; 12.8 or
+ * newer).  Host only, needs no device.  *size always receives the size needed; the
+ * CUBIN is written when cap >= *size.  log [host, logcap] receives the NVRTC log.
+ * MC3B_ERR_ARG: the source does not compile (see the log), defines no `model`, or the
+ * buffer is too small; MC3B_ERR_CUDA: NVRTC cannot be loaded or is too old. */
+int mc3b_user_model_compile(const char* nvrtc_path, const char* source, int nmodel,
+                            int dtype, void* cubin /*[host]*/, int64_t cap,
+                            int64_t* size /*[host]*/, char* log /*[host]*/,
+                            int64_t logcap);
+
+/* Load a CUBIN of mc3b_user_model_compile (same nmodel and dtype) into every device
+ * of the process and return a handle (allocates; release it with
+ * mc3b_user_model_free).  A module built against other headers or another library
+ * version is refused (MC3B_ERR_ARG). */
+int mc3b_user_model_load(const void* cubin /*[host]*/, int64_t size, int nmodel,
+                         int dtype, mc3b_user_model_t** out /*[host]*/);
+int mc3b_user_model_free(mc3b_user_model_t* m);
+
+/* mc3b_model_chisq_ex for a user model: the same partial layout, plan
+ * (mc3b_model_chisq_plan) and fuse semantics; dtype and nmodel come from the
+ * handle.  Of the options, plan_chains, uniform_sigma and fuse / fuse_done / c_off /
+ * gen / zrow0 / advance apply; folded, work, moment and tile_x are refused. */
+int mc3b_user_model_chisq_ex(const mc3b_user_model_t* m, const double* params,
+                             int64_t ldp, int64_t nchains, const void* x,
+                             const void* data, const void* invsig, int64_t n,
+                             double* partial, int64_t ldpartial, int nsplit,
+                             const mc3b_chisq_opts_t* opts, void* stream);
+
+/* mc3b_model_eval for a user model: fp64 values, out is [nchains, n] row-major. */
+int mc3b_user_model_eval(const mc3b_user_model_t* m, const double* params,
+                         int64_t ldp, int64_t nchains, const double* x, int64_t n,
+                         double* out, void* stream);
+
 /* chisq[c] = sum_s partial[s*ldpartial + c] (fixed order s = 0..nsplit-1)
  *          + sum over j with priorlow_j > 0 and priorup_j > 0 of
  *            ((p_cj - prior_j) / (p_cj > prior_j ? priorup_j : priorlow_j))^2
@@ -349,8 +405,8 @@ int mc3b_metropolis(const mc3b_sampler_t* s, const double* partial,
  * one box).  mc3b_peer_alloc: zero-filled device buffer on the current device +
  * its 64-byte IPC handle [host].  mc3b_peer_open: map another process's buffer
  * into this one (peer access is enabled on demand); *ptr [host] receives the local
- * address.  mc3b_peer_close / mc3b_peer_free undo them.  These four are the only
- * entry points that allocate. */
+ * address.  mc3b_peer_close / mc3b_peer_free undo them.  These four and
+ * mc3b_user_model_load are the only entry points that allocate. */
 int mc3b_peer_alloc(int64_t nbytes, void** ptr, unsigned char* handle64);
 int mc3b_peer_open(const unsigned char* handle64, void** ptr);
 int mc3b_peer_close(void* ptr);

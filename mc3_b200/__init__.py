@@ -10,7 +10,7 @@ torch.distributed); the arithmetic is hand-written CUDA in libmc3b200.so, bound
 through a C ABI (include/mc3b200.h) with ctypes.  There is no CPU fallback.
 """
 from . import models
-from .models import BuiltinModel, TorchModel
+from .models import BuiltinModel, CudaModel, TorchModel
 from .sampler_driver import sample, __version__
 from .fit_driver import fit
 from . import stats
@@ -18,4 +18,4 @@ from . import utils
 from .utils import Log
 
 __all__ = ['sample', 'fit', 'stats', 'utils', 'models', 'BuiltinModel',
-           'TorchModel', 'Log', '__version__']
+           'CudaModel', 'TorchModel', 'Log', '__version__']

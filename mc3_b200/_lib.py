@@ -87,6 +87,13 @@ _SIGS = {
     'mc3b_moment_prepare': (c_int, [c_vp, c_i64, c_dbl, c_dbl, c_vp, c_dbl, c_dbl, c_int, c_vp, c_vp, c_vp]),
     'mc3b_model_eval': (c_int, [c_int, c_vp, c_i64, c_i64, c_int, c_vp, c_i64,
                                 c_vp, c_vp]),
+    'mc3b_user_model_compile': (c_int, [ctypes.c_char_p, ctypes.c_char_p, c_int, c_int, c_vp, c_i64,
+                                        ctypes.POINTER(c_i64), ctypes.c_char_p, c_i64]),
+    'mc3b_user_model_load': (c_int, [ctypes.c_char_p, c_i64, c_int, c_int, ctypes.POINTER(c_vp)]),
+    'mc3b_user_model_free': (c_int, [c_vp]),
+    'mc3b_user_model_chisq_ex': (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64,
+                                         c_int, ctypes.POINTER(ChisqOpts), c_vp]),
+    'mc3b_user_model_eval': (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp]),
     'mc3b_chisq_finish': (c_int, [c_vp, c_i64, c_int, c_i64, c_vp, c_i64, c_int,
                                   c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mc3b_chisq_batch': (c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp]),

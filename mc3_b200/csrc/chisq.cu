@@ -1,214 +1,17 @@
 // mc3_b200 -- chi-squared family (replaces src_c/_chisq.c and the model +
 // chi-squared half of Chain.eval_model, mc3/chain.py:302-340).
 //
-// k_model_chisq is the hot kernel of the sampler: one launch evaluates the
-// built-in model and the data chi-squared of EVERY chain of the population.
-//
-//   grid  = (chain groups, data splits); block = 4 warps.
-//   warp  = LC chains x LP = 32/LC point lanes.  LC = 32: one chain per lane,
-//           every lane walks all points of a tile (shared-memory broadcast);
-//           LC = 8 / 1: fewer chains, lanes share the points of the tile.
-//   data  = x, data, 1/sigma tiles of TILE points, staged into shared memory
-//           by 1-D TMA bulk copies (cp.async.bulk + mbarrier, 3 stages), so a
-//           tile is fetched once per CTA and serves all its chains; the
-//           per-chain constants live in registers for the whole launch.
-//   sum   = per lane in registers, then a fixed-order xor-shuffle over the
-//           point lanes, one partial per (split, chain): deterministic.
-//
-// Bound: FP64 (or FP32) pipe -- nchains*F flops per 24 bytes of data.
+// The model + chi-squared kernel k_model_chisq and the model-value kernel live in
+// chisq_kernel.cuh, which user models compiled at run time share (jit.cu); this file
+// instantiates them for the built-in models, plans their launch shape and checks
+// their arguments (mc3b_chisq_setup, used by both paths).
 #include <stdlib.h>
 #include <string.h>
 #include <stdio.h>
 #include <type_traits>
-#include "models.cuh"
-#include "sampler_dev.cuh"
-
-#include "chisq_args.cuh"
+#include "chisq_kernel.cuh"
 
 namespace {
-
-// USIG: one uncertainty for all points (w[0]): residuals are plain differences
-// (a two-register DADD instead of a multiply or a three-register FMA) and the sum
-// is scaled by w[0]^2 once per partial.
-template <class M, typename T, int LC, int CPT, bool USIG>
-__global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESIDENT)) k_model_chisq(ChisqArgs<T> a) {
-    constexpr int TILE = tilecfg<T>::TILE;
-    constexpr int LP = 32 / LC;
-    asm volatile("griddepcontrol.launch_dependents;");   // the next proposal kernel may start its draws
-    __shared__ __align__(128) T sx[STAGES][TILE];
-    __shared__ __align__(128) T sd[STAGES][TILE];
-    __shared__ __align__(128) T sw[STAGES][TILE];
-    __shared__ __align__(8) uint64_t bar[STAGES];
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int lc = lane % LC, lp = lane / LC;
-    const int64_t cbase = ((int64_t)blockIdx.x * WARPS + warp) * (LC * CPT) + lc;
-
-    M mdl[CPT];
-#pragma unroll
-    for (int k = 0; k < CPT; k++) {
-        int64_t c = cbase + (int64_t)k * LC;
-        if (c >= a.nchains) c = a.nchains - 1;      // idle lanes shadow the last chain
-        if constexpr (M::TILE_STATE) {
-            const double dx = ((double)a.x[a.n - 1] - (double)a.x[0]) / (double)(a.n - 1);
-            mdl[k].load(a.params + c * a.ldp, dx, TILE);
-        } else {
-            mdl[k].load(a.params + c * a.ldp);
-        }
-    }
-    double acc[CPT];
-#pragma unroll
-    for (int k = 0; k < CPT; k++) acc[k] = 0.0;
-
-    // Tiles of this split: balanced contiguous ranges of FULL tiles; the
-    // ragged tail (n % TILE points) belongs to the last split.
-    const int64_t nfull = a.n / TILE;
-    int64_t tb, te;
-    if (a.nsched > 0) { tb = a.tstart[blockIdx.y]; te = a.tstart[blockIdx.y + 1]; }
-    else { tb = nfull * blockIdx.y / gridDim.y; te = nfull * (blockIdx.y + 1) / gridDim.y; }
-    const int64_t nt = te - tb;
-
-    if (a.use_tma) {
-        if (threadIdx.x == 0) {
-            for (int s = 0; s < STAGES; s++) mbar_init(&bar[s], 1);
-            mbar_fence_init();
-        }
-        __syncthreads();
-        auto issue = [&](int64_t t, int s) {
-            const int64_t off = t * TILE;
-            mbar_expect_tx(&bar[s], (USIG ? 2u : 3u) * TILE * sizeof(T));
-            bulk_g2s(sx[s], a.x + off, TILE * sizeof(T), &bar[s]);
-            bulk_g2s(sd[s], a.d + off, TILE * sizeof(T), &bar[s]);
-            if constexpr (!USIG) bulk_g2s(sw[s], a.w + off, TILE * sizeof(T), &bar[s]);
-        };
-        if (threadIdx.x == 0)
-            for (int s = 0; s < STAGES && s < nt; s++) issue(tb + s, s);
-        constexpr bool PM = premul_of<M>::value && !USIG;
-        // PM keeps d/sigma in a buffer of its own: TMA never writes it, so no generic-proxy
-        // store ever meets an async-proxy refill of the same bytes (no proxy fence needed)
-        __shared__ __align__(128) T sdw[PM ? STAGES : 1][PM ? TILE : 2];
-        // PM: data tile <- data / sigma, once for all chains of the CTA.  Tile it+1 is
-        // scaled at the end of tile it, so that the stage-release barrier publishes it.
-        auto premul = [&](int64_t t) {
-            const int s1 = (int)(t % STAGES);
-            mbar_wait(&bar[s1], (uint32_t)((t / STAGES) & 1));
-            for (int i = threadIdx.x; i < TILE; i += WARPS * 32) sdw[PM ? s1 : 0][PM ? i : 0] = sd[s1][i] * sw[s1][i];
-        };
-        if constexpr (PM) {
-            if (nt > 0) premul(0);
-            __syncthreads();
-        }
-        for (int64_t it = 0; it < nt; it++) {
-            const int s = (int)(it % STAGES);
-            if constexpr (!PM) mbar_wait(&bar[s], (uint32_t)((it / STAGES) & 1));
-            constexpr int U = 4;                // points in flight per lane
-            static_assert(TILE % (U * LP) == 0, "tile must hold whole groups");
-            if constexpr (M::TILE_STATE) {
-                static_assert(LP == 1, "stateful models walk a tile in order: one chain per lane");
-#pragma unroll
-                for (int k = 0; k < CPT; k++) mdl[k].begin_tile((double)sx[s][0], TILE);
-            }
-            T tacc[CPT], uacc[CPT][U];          // one accumulator per point slot: no serial tail
-#pragma unroll
-            for (int k = 0; k < CPT; k++) {
-#pragma unroll
-                for (int u = 0; u < U; u++) uacc[k][u] = (T)0;
-            }
-#pragma unroll(LOOP_UNROLL)
-            for (int i = lp; i < TILE; i += U * LP) {
-                T x[U], y[U];
-#pragma unroll
-                for (int u = 0; u < U; u++) x[u] = sx[s][i + u * LP];
-#pragma unroll
-                for (int k = 0; k < CPT; k++) {
-                    eval_points<M, T, U>(mdl[k], x, y, 0);
-#pragma unroll
-                    for (int u = 0; u < U; u++) {
-                        const T r = USIG ? y[u] - sd[s][i + u * LP]
-                                    : PM ? fma(y[u], sw[s][i + u * LP], -sdw[PM ? s : 0][PM ? i + u * LP : 0])
-                                         : (y[u] - sd[s][i + u * LP]) * sw[s][i + u * LP];
-                        uacc[k][u] = fma(r, r, uacc[k][u]);
-                    }
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < CPT; k++) tacc[k] = (uacc[k][0] + uacc[k][1]) + (uacc[k][2] + uacc[k][3]);
-            if (M::GUARD) {                     // extreme model arguments: redo the tile safely
-#pragma unroll
-                for (int k = 0; k < CPT; k++) {
-                    if (mdl[k].flagged()) {
-                        mdl[k].clear();
-                        tacc[k] = (T)0;
-                        for (int i = lp; i < TILE; i += LP) {
-                            const T r = USIG ? mdl[k].eval_safe(sx[s][i]) - sd[s][i]
-                                        : PM ? fma(mdl[k].eval_safe(sx[s][i]), sw[s][i], -sdw[PM ? s : 0][PM ? i : 0])
-                                             : (mdl[k].eval_safe(sx[s][i]) - sd[s][i]) * sw[s][i];
-                            tacc[k] = fma(r, r, tacc[k]);
-                        }
-                    }
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < CPT; k++) acc[k] += (double)tacc[k];
-            if constexpr (PM) {
-                if (it + 1 < nt) premul(it + 1);
-            }
-            __syncthreads();                    // everyone is done reading stage s
-            if (threadIdx.x == 0 && it + STAGES < nt) issue(tb + it + STAGES, s);
-        }
-    } else {
-        for (int64_t it = 0; it < nt; it++) {   // unaligned inputs: plain staged loads
-            const int64_t off = (tb + it) * TILE;
-            __syncthreads();
-            for (int i = threadIdx.x; i < TILE; i += WARPS * 32) {
-                sx[0][i] = a.x[off + i]; sd[0][i] = a.d[off + i]; sw[0][i] = USIG ? (T)1 : a.w[off + i];
-            }
-            __syncthreads();
-            T tacc[CPT];
-#pragma unroll
-            for (int k = 0; k < CPT; k++) tacc[k] = (T)0;
-            for (int i = lp; i < TILE; i += LP) {
-                const T x = sx[0][i], d = sd[0][i], w = sw[0][i];
-#pragma unroll
-                for (int k = 0; k < CPT; k++) {
-                    const T r = (mdl[k].eval_safe(x) - d) * w;
-                    tacc[k] = fma(r, r, tacc[k]);
-                }
-            }
-#pragma unroll
-            for (int k = 0; k < CPT; k++) acc[k] += (double)tacc[k];
-        }
-    }
-
-    // Ragged tail, straight from global memory (last split only).
-    if (blockIdx.y == gridDim.y - 1) {
-        T tacc[CPT];
-#pragma unroll
-        for (int k = 0; k < CPT; k++) tacc[k] = (T)0;
-        for (int64_t i = nfull * TILE + lp; i < a.n; i += LP) {
-            const T x = a.x[i], d = a.d[i], w = USIG ? (T)1 : a.w[i];
-#pragma unroll
-            for (int k = 0; k < CPT; k++) {
-                const T r = (mdl[k].eval_safe(x) - d) * w;
-                tacc[k] = fma(r, r, tacc[k]);
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < CPT; k++) acc[k] += (double)tacc[k];
-    }
-
-    double w2 = 1.0;
-    if constexpr (USIG) { const double w0 = (double)a.w[0]; w2 = w0 * w0; }
-#pragma unroll
-    for (int k = 0; k < CPT; k++) {
-        double v = acc[k];
-#pragma unroll
-        for (int o = 16; o >= LC; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        const int64_t c = cbase + (int64_t)k * LC;
-        if (lp == 0 && c < a.nchains) a.partial[(int64_t)blockIdx.y * a.ldpartial + c] = USIG ? v * w2 : v;
-    }
-    if (a.f.on) fused_metropolis(a.f, a.partial, a.ldpartial, a.nchains, WARPS * LC * CPT);
-}
 
 // Shape policy: a pure function of (plan_chains, n, dtype, SM count).  plan_chains
 // is the chain count the shape is planned FOR -- by default the chains of the
@@ -216,11 +19,6 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
 // spread over launches or devices plans for the whole population and launches any
 // subset of it with that plan (the split boundaries, hence the order in which a
 // chain's terms are added, then do not depend on the subset).
-struct Shape {
-    int lc, nsplit;
-    int nsched; int32_t tstart[SCHED_MAX + 1];
-};
-
 // kind: MC3B_PLAN_GENERAL, or MC3B_PLAN_MOMENT for the sufficient-statistics kernel: it runs 4
 // CTAs per SM and its CTAs are short, so its waves are planned for 4 and its splits shrink
 // more slowly and stop at 8 tiles (measured at config 2: 0.0954 against 0.0985 ms; the same plan
@@ -287,33 +85,14 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
                   const void* x, const void* d, const void* w, int64_t n, double* partial, int64_t ldpartial,
                   int nsplit, int dtype, const mc3b_chisq_opts_t& o, cudaStream_t st) {
     ChisqArgs<T> A;
-    A.params = params; A.ldp = ldp; A.nchains = nchains;
-    A.x = (const T*)x; A.d = (const T*)d; A.w = (const T*)w; A.fold = (const T*)o.folded; A.consts = nullptr; A.ldc = 0; A.consts_wait = 0; A.m = MomentArgs{}; A.n = n;
-    A.xt = nullptr; A.dxg = 0.0; A.ntiles = 0; A.partial = partial; A.ldpartial = ldpartial;
+    Shape sh;
+    dim3 grid;
+    const int rc = mc3b_chisq_setup<T>(params, ldp, nchains, x, d, w, n, partial, ldpartial, nsplit, dtype, o, A, sh,
+                                       grid);
+    if (rc != MC3B_OK) return rc;
     const bool usig = o.uniform_sigma != 0;
-    A.use_tma = ((((uintptr_t)x | (uintptr_t)d | (usig ? 0 : (uintptr_t)w)) & 15) == 0) ? 1 : 0;
-    const int64_t plan_chains = o.plan_chains > 0 ? o.plan_chains : nchains;
-    MC3B_CHECK_ARG(plan_chains >= nchains, "plan_chains (%lld) is smaller than the launch (%lld chains)",
-                   (long long)plan_chains, (long long)nchains);
-    const Shape sh = plan_shape(plan_chains, n, dtype, mc3b_sm_count(),
-                                o.moment != nullptr && usig ? MC3B_PLAN_MOMENT : MC3B_PLAN_GENERAL);
-    A.nsched = sh.nsched;
-    if (sh.nsched > 0) memcpy(A.tstart, sh.tstart, sizeof(int32_t) * (sh.nsched + 1));
-    MC3B_CHECK_ARG(nsplit == sh.nsplit, "nsplit %d does not match the plan (%d)", nsplit, sh.nsplit);
-    const int64_t groups = ceil_div64(nchains, (int64_t)WARPS * sh.lc);
-    MC3B_CHECK_ARG(groups <= 0x7fffffff, "too many chains for one launch");
-    A.f.on = 0;
-    if (o.fuse != nullptr) {
-        MC3B_CHECK_ARG(o.fuse_done != nullptr, "the fused Metropolis epilogue needs its counters (fuse_done)");
-        MC3B_CHECK_ARG(o.gen >= 0 || (o.fuse->gen_dev && o.fuse->thinning > 0),
-                       "device-driven generations need gen_dev and thinning");
-        MC3B_CHECK_ARG(!o.advance || o.fuse->gen_dev, "advance needs gen_dev");
-        MC3B_CHECK_ARG(o.c_off >= o.fuse->chain0 && o.c_off + nchains <= o.fuse->chain0 + o.fuse->nlocal,
-                       "chain range outside this device's slice");
-        A.f.on = 1; A.f.advance = o.advance; A.f.done = o.fuse_done; A.f.c_off = o.c_off;
-        A.f.gen = o.gen; A.f.zrow0 = o.zrow0; A.f.S = *o.fuse;
-    }
-    dim3 grid((unsigned)groups, (unsigned)nsplit), block(WARPS * 32);
+    const unsigned groups = grid.x;
+    dim3 block(WARPS * 32);
     if (model_id == MC3B_MODEL_SINUSOID_GRID) {
         if constexpr (std::is_same<T, double>::value) {
             if (sh.lc == 32 && A.use_tma && n >= 2) {
@@ -349,15 +128,6 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
     if (usig) { MC3B_DISPATCH_MODEL(T, model_id, nmodel, return (launch_model_chisq<M, T, true>(sh, A, grid, st))); }
     else { MC3B_DISPATCH_MODEL(T, model_id, nmodel, return (launch_model_chisq<M, T, false>(sh, A, grid, st))); }
     return MC3B_OK;
-}
-
-// ---- model values (best_model, func(params) shape probe) -------------------
-template <class M>
-__global__ void k_model_eval(const double* params, int64_t ldp, const double* x, int64_t n, double* out) {
-    M m;
-    m.load(params + (int64_t)blockIdx.y * ldp);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        out[(int64_t)blockIdx.y * n + i] = m.eval_safe(x[i]);
 }
 
 // ---- sum of partials + priors ----------------------------------------------
@@ -416,6 +186,48 @@ __global__ void k_residuals(const double* model, const double* data, const doubl
 }
 
 }  // namespace
+
+// Argument block, launch shape and argument checks of one model + chi-squared launch:
+// the part shared by the built-in models (above) and user models (jit.cu).
+template <typename T>
+int mc3b_chisq_setup(const double* params, int64_t ldp, int64_t nchains, const void* x, const void* d, const void* w,
+                     int64_t n, double* partial, int64_t ldpartial, int nsplit, int dtype, const mc3b_chisq_opts_t& o,
+                     ChisqArgs<T>& A, Shape& sh, dim3& grid) {
+    A.params = params; A.ldp = ldp; A.nchains = nchains;
+    A.x = (const T*)x; A.d = (const T*)d; A.w = (const T*)w; A.fold = (const T*)o.folded; A.consts = nullptr; A.ldc = 0; A.consts_wait = 0; A.m = MomentArgs{}; A.n = n;
+    A.xt = nullptr; A.dxg = 0.0; A.ntiles = 0; A.partial = partial; A.ldpartial = ldpartial;
+    const bool usig = o.uniform_sigma != 0;
+    A.use_tma = ((((uintptr_t)x | (uintptr_t)d | (usig ? 0 : (uintptr_t)w)) & 15) == 0) ? 1 : 0;
+    const int64_t plan_chains = o.plan_chains > 0 ? o.plan_chains : nchains;
+    MC3B_CHECK_ARG(plan_chains >= nchains, "plan_chains (%lld) is smaller than the launch (%lld chains)",
+                   (long long)plan_chains, (long long)nchains);
+    sh = plan_shape(plan_chains, n, dtype, mc3b_sm_count(),
+                    o.moment != nullptr && usig ? MC3B_PLAN_MOMENT : MC3B_PLAN_GENERAL);
+    A.nsched = sh.nsched;
+    if (sh.nsched > 0) memcpy(A.tstart, sh.tstart, sizeof(int32_t) * (sh.nsched + 1));
+    MC3B_CHECK_ARG(nsplit == sh.nsplit, "nsplit %d does not match the plan (%d)", nsplit, sh.nsplit);
+    const int64_t groups = ceil_div64(nchains, (int64_t)WARPS * sh.lc);
+    MC3B_CHECK_ARG(groups <= 0x7fffffff, "too many chains for one launch");
+    A.f.on = 0;
+    if (o.fuse != nullptr) {
+        MC3B_CHECK_ARG(o.fuse_done != nullptr, "the fused Metropolis epilogue needs its counters (fuse_done)");
+        MC3B_CHECK_ARG(o.gen >= 0 || (o.fuse->gen_dev && o.fuse->thinning > 0),
+                       "device-driven generations need gen_dev and thinning");
+        MC3B_CHECK_ARG(!o.advance || o.fuse->gen_dev, "advance needs gen_dev");
+        MC3B_CHECK_ARG(o.c_off >= o.fuse->chain0 && o.c_off + nchains <= o.fuse->chain0 + o.fuse->nlocal,
+                       "chain range outside this device's slice");
+        A.f.on = 1; A.f.advance = o.advance; A.f.done = o.fuse_done; A.f.c_off = o.c_off;
+        A.f.gen = o.gen; A.f.zrow0 = o.zrow0; A.f.S = *o.fuse;
+    }
+    grid = dim3((unsigned)groups, (unsigned)nsplit);
+    return MC3B_OK;
+}
+template int mc3b_chisq_setup<double>(const double*, int64_t, int64_t, const void*, const void*, const void*, int64_t,
+                                      double*, int64_t, int, int, const mc3b_chisq_opts_t&, ChisqArgs<double>&, Shape&,
+                                      dim3&);
+template int mc3b_chisq_setup<float>(const double*, int64_t, int64_t, const void*, const void*, const void*, int64_t,
+                                     double*, int64_t, int, int, const mc3b_chisq_opts_t&, ChisqArgs<float>&, Shape&,
+                                     dim3&);
 
 extern "C" int mc3b_model_chisq_plan_kind(int kind, int64_t nchains, int64_t n, int dtype, int* nsplit) {
     MC3B_CHECK_ARG(nchains > 0 && n > 0 && nsplit != nullptr, "bad plan arguments");

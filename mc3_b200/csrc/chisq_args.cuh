@@ -173,8 +173,25 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
     }
 }
 
+#ifndef __CUDACC_RTC__
+// Launch shape of a model + chi-squared launch (chisq.cu plan_shape): chains per warp,
+// data splits and, for large populations, the split boundaries in tiles.
+struct Shape {
+    int lc, nsplit;
+    int nsched; int32_t tstart[SCHED_MAX + 1];
+};
+#endif
+
 }  // namespace mc3b_chisq
 using namespace mc3b_chisq;
+
+#ifndef __CUDACC_RTC__
+// chisq.cu: argument block, launch shape and argument checks of a k_model_chisq launch
+// (plan, TMA alignment, fuse, nsplit), shared by the built-in and the user-model paths.
+template <typename T>
+int mc3b_chisq_setup(const double* params, int64_t ldp, int64_t nchains, const void* x, const void* d, const void* w,
+                     int64_t n, double* partial, int64_t ldpartial, int nsplit, int dtype, const mc3b_chisq_opts_t& o,
+                     ChisqArgs<T>& A, Shape& sh, dim3& grid);
 
 // chisq_grid.cu
 int mc3b_launch_sinegrid(const ChisqArgs<double>& a, bool usig, unsigned groups, unsigned nsplit, cudaStream_t st);
@@ -184,3 +201,4 @@ int mc3b_launch_moment_finish(const ChisqArgs<double>& a, int nsplit, int npars,
                               const double* pup, double* chisq, cudaStream_t st);
 int mc3b_launch_moment_prepare(const double* d, int64_t ntiles, double x0, double dx, const double* tile_x,
                                double c0ref, double slref, double* folded, double* tiles, int layout, cudaStream_t st);
+#endif

@@ -1,14 +1,17 @@
 // mc3_b200 -- shared device helpers (sm_100a only).
 #pragma once
+#ifndef __CUDACC_RTC__          // NVRTC (user models, jit.cu) has none of these headers
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#endif
 #include "../../include/mc3b200.h"
 
 #ifndef __CUDA_ARCH__
 #define MC3B_HOST 1
 #endif
 
+#ifndef __CUDACC_RTC__
 // ---- error plumbing (C-ABI returns int, message via mc3b_last_error) ------
 void mc3b_set_error(const char* fmt, ...);
 #define MC3B_CHECK_ARG(cond, ...)                                      \
@@ -26,6 +29,7 @@ void mc3b_set_error(const char* fmt, ...);
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 int mc3b_sm_count();
+#endif
 
 // ---- TMA bulk copy (1-D, no tensor map) + mbarrier -------------------------
 // cp.async.bulk global->shared completes on an mbarrier by byte count; SASS:

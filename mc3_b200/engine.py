@@ -7,6 +7,7 @@ launches through the C ABI (include/mc3b200.h):
 
     mc3b_propose      draws, jump, bounds, shared fill        chain.py:185-247
     mc3b_model_chisq  built-in model + chi-squared, all chains  chain.py:249, 302-340
+                      (mc3b_user_model_chisq_ex for a CudaModel: the same kernel)
     mc3b_metropolis   partial sums + priors, accept, write    chain.py:251-289
 
 advancing every chain in lock-step (SURVEY.md finding 6: within one generation
@@ -34,7 +35,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .models import BuiltinModel, TorchModel, SINUSOID, SINUSOID_GRID
+from .models import BuiltinModel, CudaModel, TorchModel, SINUSOID, SINUSOID_GRID
 from . import gridseg
 from .parallel import chain_slice, allgather_rows, gather_history, sum_owned
 
@@ -160,13 +161,22 @@ class Population:
         self.d_data = torch.from_numpy(data).to(self.dev)
         self.d_uncert = torch.from_numpy(uncert).to(self.dev)
         self.nfunc = npars - 3 if self.wlike else npars
-        if isinstance(func, BuiltinModel):
-            self.kind = 'builtin'
+        if isinstance(func, CudaModel) and self.shard == 'data':
+            raise ValueError("shard='data' needs a built-in model (a CudaModel runs with "
+                             "shard='chains')")
+        if isinstance(func, (BuiltinModel, CudaModel)):
+            # a CudaModel takes the built-in path with its own compiled kernels
+            # (mc3b_user_model_*): never the sinusoid grid, fold or moment kernels
+            user = isinstance(func, CudaModel)
+            self.kind = 'cuda' if user else 'builtin'
             self.nmodel = func.nmodel(self.nfunc)
+            self.jit = func.handle(self.dtype) if user else None
+            # model values are fp64 whatever the dtype, as mc3b_model_eval's
+            self.jit_eval = func.handle(_lib.F64) if user else None
             x = np.ascontiguousarray(self.indparams[0], dtype=np.double)
             if x.size != self.ndata_total or x.ndim != 1:
-                raise ValueError('built-in models need indparams=[x] with the '
-                                 'same shape as data')
+                raise ValueError(f'{"CUDA" if user else "built-in"} models need indparams=[x] '
+                                 'with the same shape as data')
             x = x[lo:hi]
             self.d_x = torch.from_numpy(x).to(self.dev)
             self.d_invsig = 1.0/self.d_uncert
@@ -176,13 +186,13 @@ class Population:
                              and not os.environ.get('MC3B_NO_USIG'))
             # A sinusoid on a uniform abscissa grid takes the rotation-recurrence
             # kernel (models.cuh SineGridModel); MC3B_NO_GRID=1 forces the plain one.
-            self.chisq_model_id = func.model_id
+            self.chisq_model_id = None if user else func.model_id
             self.grid = False
             self.seg = None                    # piecewise-uniform layout (gridseg.tile_layout) or None
             kx, kd, kw = self.d_x, self.d_data, self.d_invsig     # what the model kernels read
             nfold = self.ndata                 # leading entries of kd that form whole tiles
             fold_ok = self.usig and not os.environ.get('MC3B_NO_FOLD')
-            if func.model_id == SINUSOID and self.dtype == _lib.F64 and x.size >= 8 \
+            if not user and func.model_id == SINUSOID and self.dtype == _lib.F64 and x.size >= 8 \
                     and not os.environ.get('MC3B_NO_GRID'):
                 ideal = x[0] + np.arange(x.size)*((x[-1] - x[0])/(x.size - 1))
                 if x[-1] != x[0] and np.max(np.abs(x - ideal)) <= 8*np.finfo(float).eps*np.max(np.abs(x)):
@@ -335,7 +345,7 @@ class Population:
         self.plan_chains = int(plan_chains) if plan_chains else 0
         # Metropolis step fused into the tail of the model kernel (2 launches per
         # generation instead of 4); MC3B_NO_FUSE=1 keeps the separate kernels
-        self.fused = (self.kind == 'builtin' and not self.wlike and self.shard == 'chains'
+        self.fused = (self.kind in ('builtin', 'cuda') and not self.wlike and self.shard == 'chains'
                       and not os.environ.get('MC3B_NO_FUSE'))
         self.fuse_done = torch.zeros(self.nlocal//8 + 8, dtype=torch.int32, device=self.dev)
         self.S = self._make_struct()
@@ -443,6 +453,12 @@ class Population:
 
     def _model_rows(self, P):
         """Model values [nb, N] on the device for non-built-in models."""
+        if self.kind == 'cuda':
+            rows = self._workspace(('mrows', P.shape[0]), (P.shape[0], self.ndata))
+            _lib.call('mc3b_user_model_eval', self.jit_eval, P.data_ptr(), _lib.ld(P), P.shape[0],
+                      self.d_x.data_ptr(), self.ndata, rows.data_ptr(), _lib.stream_ptr())
+            self.launches += 1
+            return rows
         if self.kind == 'torch':
             Pm = P[:, :self.nfunc]
             m = self.func.fn(Pm, *self.t_indparams, **self.indparams_dict)
@@ -516,7 +532,7 @@ class Population:
                           out.data_ptr(), st)
             self.launches += 2
             return out, nb, 1
-        if self.kind == 'builtin':
+        if self.kind in ('builtin', 'cuda'):
             moment = bool(getattr(self, 'use_moment', False)) and self.d_fold is not None \
                 and (fuse is not None or moment_ok)
             ns = self._plan(nb, moment)
@@ -541,11 +557,16 @@ class Population:
                 o.advance = 1 if adv else 0
                 o.fuse = ctypes.pointer(self.S)
                 o.fuse_done = self.fuse_done.data_ptr()
-            _lib.call('mc3b_model_chisq_ex', self.chisq_model_id, self.dtype,
-                      P.data_ptr(), _lib.ld(P), nb, self.nmodel,
-                      self.k_x.data_ptr(), self.k_d.data_ptr(),
-                      self.k_w.data_ptr(), self.ndata, part.data_ptr(), nb, ns,
-                      ctypes.byref(o), st)
+            if self.kind == 'cuda':
+                _lib.call('mc3b_user_model_chisq_ex', self.jit, P.data_ptr(), _lib.ld(P), nb,
+                          self.k_x.data_ptr(), self.k_d.data_ptr(), self.k_w.data_ptr(),
+                          self.ndata, part.data_ptr(), nb, ns, ctypes.byref(o), st)
+            else:
+                _lib.call('mc3b_model_chisq_ex', self.chisq_model_id, self.dtype,
+                          P.data_ptr(), _lib.ld(P), nb, self.nmodel,
+                          self.k_x.data_ptr(), self.k_d.data_ptr(),
+                          self.k_w.data_ptr(), self.ndata, part.data_ptr(), nb, ns,
+                          ctypes.byref(o), st)
             self.launches += 1
             return part, nb, ns
         m = self._model_rows(P)
@@ -558,13 +579,17 @@ class Population:
 
     @on_device
     def model_eval(self, fpar):
-        """Built-in model at one parameter vector over the (device-resident)
+        """Built-in or CUDA model at one parameter vector over the (device-resident)
         abscissa, as a host array (chain.py:316-319 `func(params, *indparams)`)."""
         P = torch.as_tensor(np.atleast_2d(np.asarray(fpar, dtype=np.double)), device=self.dev)
         out = torch.empty((1, self.ndata), dtype=torch.float64, device=self.dev)
-        _lib.call('mc3b_model_eval', self.func.model_id, P.data_ptr(), P.shape[1], 1,
-                  self.nmodel, self.d_x.data_ptr(), self.ndata, out.data_ptr(),
-                  _lib.stream_ptr())
+        if self.kind == 'cuda':
+            _lib.call('mc3b_user_model_eval', self.jit_eval, P.data_ptr(), P.shape[1], 1,
+                      self.d_x.data_ptr(), self.ndata, out.data_ptr(), _lib.stream_ptr())
+        else:
+            _lib.call('mc3b_model_eval', self.func.model_id, P.data_ptr(), P.shape[1], 1,
+                      self.nmodel, self.d_x.data_ptr(), self.ndata, out.data_ptr(),
+                      _lib.stream_ptr())
         self.launches += 1
         return to_host(out[0])
 
@@ -756,7 +781,7 @@ class Population:
             # (single device only: an eager NCCL all-gather per generation costs the
             # host more than the generation itself, 0.69 vs 0.24 ms at 8 GPUs)
             heavy = float(self.nlocal)*self.ndata > 2e8 and not self.small and self.world == 1
-            use_graph = self.kind == 'builtin' and not heavy and not \
+            use_graph = self.kind in ('builtin', 'cuda') and not heavy and not \
                 (self.world > 1 and self.shard == 'chains' and self.sampler == 'snooker'
                  and self.p2p is None)
         if use_graph and self.small:

@@ -9,11 +9,11 @@ from . import stats as ms
 
 
 def _model(func, params, indparams, indparams_dict, nfunc):
-    """Built-in models take exactly their own parameters: with the wavelet
+    """Built-in and CUDA models take exactly their own parameters: with the wavelet
     likelihood the three noise parameters at the end are not theirs
     (chain.py:317).  User callables get the full vector, as in the reference."""
-    from .models import BuiltinModel
-    if nfunc is not None and isinstance(func, BuiltinModel):
+    from .models import BuiltinModel, CudaModel
+    if nfunc is not None and isinstance(func, (BuiltinModel, CudaModel)):
         return func(params[:nfunc], *indparams, **indparams_dict)
     return func(params, *indparams, **indparams_dict)
 

@@ -31,7 +31,7 @@ def eval_model(pop, params, ret='model'):
     if ret == 'chisq':
         return chisq
     fpar = np.asarray(params, float)[:pop.nfunc]
-    if pop.kind == 'builtin' and pop.shard != 'data':
+    if pop.kind in ('builtin', 'cuda') and pop.shard != 'data':
         model = pop.model_eval(fpar)          # abscissa already on the device
     else:
         model = pop.func(fpar, *pop.indparams, **pop.indparams_dict)

@@ -9,11 +9,29 @@ The reference's `func` is any Python callable `func(params, *indparams,
 * a TorchModel: a user torch callable evaluated ONCE per generation over the
   whole population, `fn(P[nchains, npars], *indparams) -> model[nchains, N]`
   on the device;
+* a CudaModel: the user's own formula as a CUDA device function, compiled at run
+  time (NVRTC, mc3_b200/jit.py) into the same fused kernel as the built-in models --
+  the fast path for any model of one abscissa:
+
+      transit = CudaModel('''
+          __device__ real model(real x, const real* p) {      // p[0..nparams)
+              real z = fabs(x - p[1]) / p[2];                  // helpers above `model` are allowed
+              return p[3] - p[0] * (z < 1 ? (real)1 : (z < p[4] ? (p[4] - z)/(p[4] - 1) : (real)0));
+          }''', nparams=5, name='trapezoid')
+
+  `real` is double (float with dtype='f32'); models.cuh is included, so fast_sin and
+  fast_sincos_core are available.  nparams counts the parameters the model itself
+  consumes (with wlike=True it gets params[0:-3]), at most 32.  The source compiles on
+  first use; a compile error raises ValueError with the NVRTC log;
+* a TorchModel: a user torch callable evaluated ONCE per generation over the
+  whole population, `fn(P[nchains, npars], *indparams) -> model[nchains, N]`
+  on the device;
 * any other callable: the reference's own convention, evaluated per chain on
   the host (compatibility path; the chi-squared still runs on the GPU).
 
-BuiltinModel objects are also plain callables with the reference signature
-`model(params, x)`; the evaluation runs on the GPU (mc3b_model_eval).
+BuiltinModel and CudaModel objects are also plain callables with the reference
+signature `model(params, x)`; the evaluation runs on the GPU (mc3b_model_eval,
+mc3b_user_model_eval).
 """
 import numpy as np
 
@@ -63,6 +81,67 @@ class BuiltinModel:
 
     def __repr__(self):
         return f'<mc3_b200 built-in model {self.name}>'
+
+
+def _eval_rows(params, x, launch):
+    """model(params, x) on the current GPU: [nrows, N] (or [N] for one row)."""
+    import torch
+    params = np.atleast_2d(np.asarray(params, dtype=np.double))
+    x = np.ascontiguousarray(x, dtype=np.double)
+    dev = torch.device('cuda')
+    dp = torch.from_numpy(np.ascontiguousarray(params)).to(dev)
+    dx = torch.from_numpy(x).to(dev)
+    out = torch.empty((params.shape[0], x.size), dtype=torch.float64, device=dev)
+    launch(dp, dx, out)
+    res = out.cpu().numpy()
+    return res[0] if res.shape[0] == 1 else res
+
+
+class CudaModel:
+    """A user model written as a CUDA device function (see the module docstring):
+    `__device__ real model(real x, const real* p)` in `source`, taking `nparams`
+    parameters.  Compiled lazily, once per process and dtype; pickles as its source
+    (one process per GPU receives it and compiles its own copy)."""
+
+    def __init__(self, source, nparams, name='cuda_model'):
+        nparams = int(nparams)
+        if not 1 <= nparams <= _lib.MAX_PARS:
+            raise ValueError(f'a CudaModel takes 1 to {_lib.MAX_PARS} parameters, got {nparams}')
+        self.source, self.nparams, self.name = str(source), nparams, str(name)
+
+    def __getstate__(self):
+        return {'source': self.source, 'nparams': self.nparams, 'name': self.name}
+
+    def __setstate__(self, state):
+        self.__init__(state['source'], state['nparams'], state['name'])
+
+    def nmodel(self, nfunc_params):
+        """Number of leading parameters the model consumes."""
+        if nfunc_params != self.nparams:
+            raise ValueError(
+                f'{self.name} takes {self.nparams} parameters, got {nfunc_params}')
+        return self.nparams
+
+    def cache_key(self, dtype=_lib.F64):
+        from . import jit
+        return jit.cache_key(self.source, self.nparams, dtype)
+
+    def handle(self, dtype=_lib.F64, stats=None):
+        """mc3b_user_model_t* of this model for dtype (_lib.F64 / _lib.F32)."""
+        from . import jit
+        return jit.handle(self.source, self.nparams, dtype, self.name, stats)
+
+    def __call__(self, params, x):
+        self.nmodel(np.shape(np.atleast_2d(params))[1])
+        h = self.handle(_lib.F64)
+
+        def launch(dp, dx, out):
+            _lib.call('mc3b_user_model_eval', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
+                      dx.data_ptr(), dx.numel(), out.data_ptr(), _lib.stream_ptr())
+        return _eval_rows(params, x, launch)
+
+    def __repr__(self):
+        return f'<mc3_b200 CUDA model {self.name} ({self.nparams} parameters)>'
 
 
 class TorchModel:
