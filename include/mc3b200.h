@@ -70,10 +70,12 @@ int mc3b_device_sms(void);
 int mc3b_model_chisq_plan(int64_t nchains, int64_t n, int dtype, int* nsplit);
 
 /* The same for a given kernel family: launches with opts.moment (the
- * sufficient-statistics kernel) are planned with MC3B_PLAN_MOMENT, everything else
+ * sufficient-statistics kernel) are planned with MC3B_PLAN_MOMENT (MC3B_PLAN_SPECTRAL when
+ * opts.moment->spectral is set), everything else
  * with MC3B_PLAN_GENERAL (= mc3b_model_chisq_plan). */
 #define MC3B_PLAN_GENERAL 0
 #define MC3B_PLAN_MOMENT 1
+#define MC3B_PLAN_SPECTRAL 2    /* the spectral form of mc3b_moment_t: always one split */
 int mc3b_model_chisq_plan_kind(int kind, int64_t nchains, int64_t n, int dtype, int* nsplit);
 
 /* The split boundaries behind that plan, in data points: split s sums the points
@@ -180,7 +182,11 @@ typedef struct mc3b_chisq_opts {
  *   layout  of `folded`: 0 = pairs interleaved as in mc3b_fold_data (Pe, Po by FMAs),
  *           1 = the four B fragments of mma.m8n8k4 per tile (Pe, Po as FP64 tensor-core
  *           products: fewer operand reads, instructions and shared-memory loads)
- *   guard_hits  device int32 counter or NULL */
+ *   guard_hits  device int32 counter or NULL
+ *   spectral  [host] NULL: the tile kernels above.  Otherwise the spectral form below replaces
+ *           them (folded, tiles and opts.work are then not read); its launches are planned
+ *           with MC3B_PLAN_SPECTRAL (one split) and its rows are unguarded in the same way. */
+struct mc3b_spectral;
 typedef struct mc3b_moment {
     const double* folded;
     const double* tiles;
@@ -188,7 +194,45 @@ typedef struct mc3b_moment {
     double xlo, xhi;
     int32_t* guard_hits;
     int32_t layout;     /* as given to mc3b_moment_prepare */
+    const struct mc3b_spectral* spectral;
 } mc3b_moment_t;
+
+/* Spectral form of the same chi-squared: O(1) per chain instead of O(n).  With
+ * t = x - xc, d' = d - (c0ref + slref x), L' = a + b t the line relative to the reference
+ * line (a = c0 - c0ref + (sl - slref) xc, b = sl - slref), w = 2 pi / P and
+ * S_g(w) = sum_i g_i e^{i w x_i},
+ *   sigma^2 chisq = A^2 [n/2 - Re(e^{2 i ph} S_1(2w))/2]
+ *                 + 2 A Im(e^{i ph} [a S_1(w) + b S_t(w) - S_d'(w)])
+ *                 + n a^2 + 2 a b St + b^2 St2 - 2 a Sd - 2 b Std + D2
+ * (St = sum t, St2 = sum t^2, Sd = sum d', Std = sum t d', D2 = sum d'^2).  The data enter
+ * only through S at the chain's own frequency.  Per node w_j = w1 + j delta (j < n1) of the
+ * band and w2 + j delta (j < n2) of the doubled band, the table holds Taylor coefficients
+ *   T_g[j][k] = sum_i g_i t_i^k e^{i w_j x_i} / k!,  S_g(w_j + dw) = e^{i dw xc} sum_k (i dw)^k T_g[j][k]
+ * to order K = `order` (9 or 15); truncation error <= (|dw| R)^{K+1} / (K+1)! sum |g_i|,
+ * R = max |t_i|, |dw| <= delta/2 (mc3_b200/spectral.py plans delta and K for 1e-18).
+ * Like the tile form, the result is what is left after terms of size (|s| + |L'| + |d'|)^2
+ * cancel: relative error eps_eff * amp, eps_eff < 3e-15 (profiles/spectral_error.py); the
+ * same guard (amp_max of mc3b_moment_t) applies, and a chain whose w or 2w has no node
+ * within delta/2 also takes the point-by-point evaluation and counts in guard_hits.
+ *   table  device, mc3b_spectral_size() doubles, written by mc3b_spectral_prepare:
+ *          MC3B_SPECTRAL_HEAD sums {n, St, St2, Sd, Std, D2, 0, 0}, then per node of the band
+ *          K + 2 complex T_1 and K + 1 complex T_d' (T_t[k] = (k + 1) T_1[k + 1]), then per
+ *          node of the doubled band K + 1 complex T_1 (complex = re, im). */
+#define MC3B_SPECTRAL_HEAD 8
+typedef struct mc3b_spectral {
+    double* table;
+    double w1, w2, delta, xc;   /* first node of the band and of the doubled band, spacing, centre */
+    int32_t n1, n2, order;      /* nodes of the band, of the doubled band; K */
+} mc3b_spectral_t;
+
+/* Doubles of the table of mc3b_spectral_t for n1, n2 nodes and order K (9 or 15). */
+int mc3b_spectral_size(int n1, int n2, int order, int64_t* ndoubles /*[host]*/);
+
+/* Writes s->table from the n points x, data (device, fp64, any order: for a piecewise-
+ * uniform abscissa the reordered arrays) about the reference line c0ref + slref x.  One
+ * CTA per node, fixed-order sums: the same bits on every device.  Done once per data set. */
+int mc3b_spectral_prepare(const double* x, const double* data, int64_t n, double c0ref,
+                          double slref, const mc3b_spectral_t* s, void* stream);
 
 /* mc3b_chisq_finish for rows written by the moment form WITHOUT `fuse`: adds the
  * nsplit rows of every chain in split order, applies the guard of mc3b_moment_t

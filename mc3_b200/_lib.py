@@ -42,11 +42,17 @@ class SamplerStruct(ctypes.Structure):
     ]
 
 
+class SpectralStruct(ctypes.Structure):
+    """mc3b_spectral_t."""
+    _fields_ = [('table', c_vp), ('w1', c_dbl), ('w2', c_dbl), ('delta', c_dbl), ('xc', c_dbl),
+                ('n1', c_i32), ('n2', c_i32), ('order', c_i32)]
+
+
 class MomentStruct(ctypes.Structure):
     """mc3b_moment_t."""
     _fields_ = [('folded', c_vp), ('tiles', c_vp), ('c0ref', c_dbl), ('slref', c_dbl),
                 ('d2tot', c_dbl), ('amp_max', c_dbl), ('xlo', c_dbl), ('xhi', c_dbl),
-                ('guard_hits', c_vp), ('layout', c_i32)]
+                ('guard_hits', c_vp), ('layout', c_i32), ('spectral', ctypes.POINTER(SpectralStruct))]
 
 
 class ChisqOpts(ctypes.Structure):
@@ -85,6 +91,8 @@ _SIGS = {
     'mc3b_moment_finish': (c_int, [ctypes.POINTER(MomentStruct), c_vp, c_i64, c_int, c_i64, c_vp, c_i64, c_int,
                                    c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mc3b_moment_prepare': (c_int, [c_vp, c_i64, c_dbl, c_dbl, c_vp, c_dbl, c_dbl, c_int, c_vp, c_vp, c_vp]),
+    'mc3b_spectral_size': (c_int, [c_int, c_int, c_int, ctypes.POINTER(c_i64)]),
+    'mc3b_spectral_prepare': (c_int, [c_vp, c_vp, c_i64, c_dbl, c_dbl, ctypes.POINTER(SpectralStruct), c_vp]),
     'mc3b_model_eval': (c_int, [c_int, c_vp, c_i64, c_i64, c_int, c_vp, c_i64,
                                 c_vp, c_vp]),
     'mc3b_user_model_compile': (c_int, [ctypes.c_char_p, ctypes.c_char_p, c_int, c_int, c_vp, c_i64,

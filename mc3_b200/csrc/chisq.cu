@@ -23,8 +23,13 @@ namespace {
 // CTAs per SM and its CTAs are short, so its waves are planned for 4 and its splits shrink
 // more slowly and stop at 8 tiles (measured at config 2: 0.0954 against 0.0985 ms; the same plan
 // costs the other kernels 3-16 %, profiles/r2_plan_ab.txt).
+// MC3B_PLAN_SPECTRAL: one thread per chain and no data stream, so one split.
 Shape plan_shape(int64_t nchains, int64_t n, int dtype, int sms, int kind = MC3B_PLAN_GENERAL) {
     Shape s;
+    if (kind == MC3B_PLAN_SPECTRAL) {
+        s.lc = 32; s.nsplit = 1; s.nsched = 0;
+        return s;
+    }
     int RESIDENT = kind == MC3B_PLAN_MOMENT ? 4 : mc3b_chisq::RESIDENT;    // MC3B_PLAN_RESIDENT: experiments
     if (const char* e = getenv("MC3B_PLAN_RESIDENT")) RESIDENT = atoi(e) > 0 ? atoi(e) : RESIDENT;
     s.lc = nchains >= 96 ? 32 : (nchains >= 12 ? 8 : 1);
@@ -99,6 +104,18 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
                 if (o.tile_x != nullptr) {
                     MC3B_CHECK_ARG(o.dx != 0.0 && o.ntiles >= 0 && o.ntiles * 128 <= n, "tile_x needs dx and ntiles <= n/128");
                     A.xt = o.tile_x; A.dxg = o.dx; A.ntiles = o.ntiles;
+                }
+                if (usig && o.moment != nullptr && o.moment->spectral != nullptr) {
+                    const mc3b_spectral_t& s = *o.moment->spectral;
+                    MC3B_CHECK_ARG(s.table && (((uintptr_t)s.table) & 15) == 0 && s.n1 > 0 && s.n2 > 0 &&
+                                   (s.order == 9 || s.order == 15) && s.delta > 0.0 && o.moment->amp_max > 0.0,
+                                   "bad spectral table");
+                    A.m.c0ref = o.moment->c0ref; A.m.slref = o.moment->slref; A.m.d2tot = o.moment->d2tot;
+                    A.m.amp_max = o.moment->amp_max; A.m.guard_hits = o.moment->guard_hits;
+                    A.m.xlo = o.moment->xlo; A.m.xhi = o.moment->xhi;
+                    A.m.spec = s.table; A.m.sw1 = s.w1; A.m.sw2 = s.w2; A.m.sdelta = s.delta; A.m.sxc = s.xc;
+                    A.m.sn1 = s.n1; A.m.sn2 = s.n2; A.m.sorder = s.order;
+                    return mc3b_launch_spectral_chisq(A, (unsigned)groups, st);
                 }
                 if (usig && o.moment != nullptr) {
                     MC3B_CHECK_ARG(o.work, "the moment form needs the constants workspace (work)");
@@ -202,7 +219,8 @@ int mc3b_chisq_setup(const double* params, int64_t ldp, int64_t nchains, const v
     MC3B_CHECK_ARG(plan_chains >= nchains, "plan_chains (%lld) is smaller than the launch (%lld chains)",
                    (long long)plan_chains, (long long)nchains);
     sh = plan_shape(plan_chains, n, dtype, mc3b_sm_count(),
-                    o.moment != nullptr && usig ? MC3B_PLAN_MOMENT : MC3B_PLAN_GENERAL);
+                    o.moment != nullptr && usig ? (o.moment->spectral ? MC3B_PLAN_SPECTRAL : MC3B_PLAN_MOMENT)
+                                                : MC3B_PLAN_GENERAL);
     A.nsched = sh.nsched;
     if (sh.nsched > 0) memcpy(A.tstart, sh.tstart, sizeof(int32_t) * (sh.nsched + 1));
     MC3B_CHECK_ARG(nsplit == sh.nsplit, "nsplit %d does not match the plan (%d)", nsplit, sh.nsplit);
@@ -232,7 +250,8 @@ template int mc3b_chisq_setup<float>(const double*, int64_t, int64_t, const void
 extern "C" int mc3b_model_chisq_plan_kind(int kind, int64_t nchains, int64_t n, int dtype, int* nsplit) {
     MC3B_CHECK_ARG(nchains > 0 && n > 0 && nsplit != nullptr, "bad plan arguments");
     MC3B_CHECK_ARG(dtype == MC3B_F64 || dtype == MC3B_F32, "bad dtype %d", dtype);
-    MC3B_CHECK_ARG(kind == MC3B_PLAN_GENERAL || kind == MC3B_PLAN_MOMENT, "bad plan kind %d", kind);
+    MC3B_CHECK_ARG(kind == MC3B_PLAN_GENERAL || kind == MC3B_PLAN_MOMENT || kind == MC3B_PLAN_SPECTRAL,
+                   "bad plan kind %d", kind);
     int sms = mc3b_sm_count();
     if (sms <= 0) sms = 148;        // planning without a device (CPU-side sizing)
     *nsplit = plan_shape(nchains, n, dtype, sms, kind).nsplit;
@@ -309,6 +328,20 @@ extern "C" int mc3b_moment_prepare(const double* data, int64_t ntiles, double x0
     MC3B_CHECK_ARG(layout == 0 || layout == 1, "bad moment layout %d", layout);
     MC3B_CHECK_ARG((((uintptr_t)tiles) & 31) == 0, "tiles must be 32-byte aligned");
     return mc3b_launch_moment_prepare(data, ntiles, x0, dx, tile_x, c0ref, slref, folded, tiles, layout, (cudaStream_t)stream);
+}
+
+extern "C" int mc3b_spectral_size(int n1, int n2, int order, int64_t* ndoubles) {
+    MC3B_CHECK_ARG(n1 > 0 && n2 > 0 && (order == 9 || order == 15) && ndoubles, "bad spectral_size arguments");
+    *ndoubles = MC3B_SPECTRAL_HEAD + 2 * ((int64_t)n1 * (2 * order + 3) + (int64_t)n2 * (order + 1));
+    return MC3B_OK;
+}
+
+extern "C" int mc3b_spectral_prepare(const double* x, const double* data, int64_t n, double c0ref, double slref,
+                                     const mc3b_spectral_t* s, void* stream) {
+    MC3B_CHECK_ARG(x && data && s && s->table && n > 0, "bad spectral_prepare arguments");
+    MC3B_CHECK_ARG(s->n1 > 0 && s->n2 > 0 && (int64_t)s->n1 + s->n2 < 0x7fffffff && (s->order == 9 || s->order == 15) &&
+                   s->delta > 0.0, "bad spectral table description");
+    return mc3b_launch_spectral_prepare(x, data, n, c0ref, slref, *s, (cudaStream_t)stream);
 }
 
 extern "C" int mc3b_model_chisq(int model_id, int dtype, const double* params, int64_t ldp, int64_t nchains,

@@ -53,6 +53,10 @@ struct MomentArgs {
     double xlo, xhi;                // range of the abscissa (bound of the line term of the guard)
     int32_t* guard_hits;
     int layout;                     // of `folded`: 0 pairs interleaved (k_sinefold<MOM>), 1 mma fragments (k_sinemma)
+    // spectral form (k_spectral_chisq, include/mc3b200.h mc3b_spectral_t): nullptr = the tile kernels
+    const double* spec;             // sums, then the Taylor tables of both bands (mc3b_spectral_prepare)
+    double sw1, sw2, sdelta, sxc;   // first node of the band and of the doubled band, node spacing, centre of x
+    int sn1, sn2, sorder;           // nodes per band, Taylor order K
 };
 
 template <typename T> struct ChisqArgs {
@@ -201,4 +205,7 @@ int mc3b_launch_moment_finish(const ChisqArgs<double>& a, int nsplit, int npars,
                               const double* pup, double* chisq, cudaStream_t st);
 int mc3b_launch_moment_prepare(const double* d, int64_t ntiles, double x0, double dx, const double* tile_x,
                                double c0ref, double slref, double* folded, double* tiles, int layout, cudaStream_t st);
+int mc3b_launch_spectral_chisq(const ChisqArgs<double>& a, unsigned groups, cudaStream_t st);
+int mc3b_launch_spectral_prepare(const double* x, const double* d, int64_t n, double c0ref, double slref,
+                                 const mc3b_spectral_t& s, cudaStream_t st);
 #endif

@@ -860,7 +860,160 @@ __global__ void __launch_bounds__(128) k_moment_prepare(const double* __restrict
     }
 }
 
+// ---- spectral form: the whole chi-squared from a precomputed spectrum of the data ----------
+// With t = x - xc, d' = d - (c0ref + slref x), the line relative to the reference line written
+// about the centre, L' = a + b t, and S_g(w) = sum_n g_n e^{i w x_n},
+//   sigma^2 chisq = A^2 [n/2 - Re(e^{2 i ph} S_1(2w))/2] + 2 A Im(e^{i ph} [a S_1(w) + b S_t(w) - S_d'(w)])
+//                 + n a^2 + 2 a b St + b^2 St2 - 2 a Sd - 2 b Std + D2
+// (St = sum t, St2 = sum t^2, Sd = sum d', Std = sum t d', D2 = sum d'^2, all measured).  The data
+// enter only through S at the chain's own frequency; per node w_j of a grid Delta apart the table
+// holds T_g[j][k] = sum_n g_n t_n^k e^{i w_j x_n} / k!, and
+//   S_g(w_j + delta) = e^{i delta xc} sum_k (i delta)^k T_g[j][k]          (complex Horner)
+// with truncation error <= (|delta| R)^{K+1} / (K+1)! sum |g|, R = max |t|.  S_t needs no table of
+// its own: T_t[j][k] = (k + 1) T_1[j][k + 1], so the band's nodes hold T_1 to order K + 1.
+// Layout (doubles): spec::HEAD sums {n, St, St2, Sd, Std, D2, 0, 0}; per node of the band,
+// K + 2 complex T_1 then K + 1 complex T_d'; per node of the doubled band, K + 1 complex T_1.
+namespace spec {
+constexpr int HEAD = MC3B_SPECTRAL_HEAD;
+}
+
+// One CTA per node (the band's, then the doubled band's) plus one for the sums; every thread
+// adds the points i = tid mod 256 in order, then lanes (xor tree) and warps (in order): the
+// bits depend on neither the SM count nor the device.
+template <int K>
+__global__ void __launch_bounds__(256) k_spectral_table(const double* __restrict__ x, const double* __restrict__ d,
+                                                        int64_t n, double c0ref, double slref, double xc, double w1,
+                                                        double w2, double delta, int n1, int n2,
+                                                        double* __restrict__ out) {
+    constexpr int NV = 4 * K + 6;
+    __shared__ double red[8][NV];
+    const int j = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const bool band1 = j < n1, sums = j == n1 + n2;
+    const double om = band1 ? fma((double)j, delta, w1) : fma((double)(j - n1), delta, w2);
+    double v[NV];                   // re T_1[0..K+1], im T_1[0..K+1], re T_d'[0..K], im T_d'[0..K]
+#pragma unroll
+    for (int k = 0; k < NV; k++) v[k] = 0.0;
+    if (sums) {
+        for (int64_t i = threadIdx.x; i < n; i += 256) {
+            const double xv = x[i], t = xv - xc, dp = d[i] - fma(slref, xv, c0ref);
+            v[1] += t; v[2] = fma(t, t, v[2]); v[3] += dp; v[4] = fma(t, dp, v[4]); v[5] = fma(dp, dp, v[5]);
+        }
+    } else {
+        for (int64_t i = threadIdx.x; i < n; i += 256) {
+            const double xv = x[i], t = xv - xc;
+            double pr, pi;
+            sincos(om * xv, &pi, &pr);
+            const double dp = band1 ? d[i] - fma(slref, xv, c0ref) : 0.0;
+#pragma unroll
+            for (int k = 0; k < K + 2; k++) {
+                v[k] += pr; v[K + 2 + k] += pi;
+                if (band1 && k <= K) { v[2 * K + 4 + k] = fma(dp, pr, v[2 * K + 4 + k]); v[3 * K + 5 + k] = fma(dp, pi, v[3 * K + 5 + k]); }
+                pr *= t; pi *= t;
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < NV; k++) {
+        double s = v[k];
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (lane == 0) red[warp][k] = s;
+    }
+    __syncthreads();
+    const int k = threadIdx.x;
+    if (k >= NV) return;
+    double s = 0.0;
+    for (int w = 0; w < 8; w++) s += red[w][k];
+    if (sums) {
+        if (k < spec::HEAD) out[k] = k == 0 ? (double)n : (k < 6 ? s : 0.0);
+        return;
+    }
+    const int kk = k < 2 * K + 4 ? k % (K + 2) : (k - 2 * K - 4) % (K + 1);
+    const int im = k < 2 * K + 4 ? k / (K + 2) : (k - 2 * K - 4) / (K + 1);
+    double fact = 1.0;
+    for (int i = 2; i <= kk; i++) fact *= (double)i;
+    double* tab = out + spec::HEAD;
+    if (band1) {
+        const int64_t e = (int64_t)j * (2 * K + 3) + (k < 2 * K + 4 ? kk : K + 2 + kk);
+        tab[2 * e + im] = s / fact;
+    } else if (k < 2 * K + 4 && kk <= K) {
+        const int64_t e = (int64_t)n1 * (2 * K + 3) + (int64_t)(j - n1) * (K + 1) + kk;
+        tab[2 * e + im] = s / fact;
+    }
+}
+
+// One thread per chain, no data stream: three complex Horner sums of K + 1 terms and three
+// sincos, whatever n is.  The row is that of a one-split launch of the tile kernels, and as
+// unguarded: a chain whose frequency (or twice it) falls outside the table gets NaN, which
+// MomentFix (fused epilogue or mc3b_moment_finish) sends to the point-by-point evaluation
+// together with the chains whose amplification is too large.
+__global__ void __launch_bounds__(WARPS * 32) k_spectral_chisq(ChisqArgs<double> a) {
+    asm volatile("griddepcontrol.launch_dependents;");   // the next proposal kernel may start its draws
+    int64_t c = (int64_t)blockIdx.x * (WARPS * 32) + threadIdx.x;
+    const bool live = c < a.nchains;
+    if (!live) c = a.nchains - 1;
+    const MomentArgs& m = a.m;
+    const double* p = a.params + c * a.ldp;
+    const double amp = p[0], om = 6.283185307179586476925287 / p[1], ph = p[2];
+    const double b = p[4] - m.slref;
+    const double ac = fma(b, m.sxc, p[3] - m.c0ref);           // L' at the centre
+    const double j1 = rint((om - m.sw1) / m.sdelta), j2 = rint((2.0 * om - m.sw2) / m.sdelta);
+    double q = __longlong_as_double(0x7ff8000000000000LL);
+    if (j1 >= 0.0 && j1 < (double)m.sn1 && j2 >= 0.0 && j2 < (double)m.sn2) {
+        const int K = m.sorder;
+        const double d1 = om - fma(j1, m.sdelta, m.sw1), d2 = fma(2.0, om, -fma(j2, m.sdelta, m.sw2));
+        const double2* tab = reinterpret_cast<const double2*>(m.spec + spec::HEAD);
+        const double2* T = tab + (int64_t)j1 * (2 * K + 3);
+        const double2* U = tab + (int64_t)m.sn1 * (2 * K + 3) + (int64_t)j2 * (K + 1);
+        // H = sum_k (i d1)^k [a T_1[k] + b (k+1) T_1[k+1] - T_d'[k]],  G = sum_k (i d2)^k U[k]
+        double hr = 0.0, hi = 0.0, gr = 0.0, gi = 0.0;
+        for (int k = K; k >= 0; k--) {
+            const double2 t0 = T[k], t1 = T[k + 1], td = T[K + 2 + k], u = U[k];
+            const double bk = b * (double)(k + 1);
+            const double cr = fma(ac, t0.x, fma(bk, t1.x, -td.x));
+            const double ci = fma(ac, t0.y, fma(bk, t1.y, -td.y));
+            const double nr = fma(-d1, hi, cr);
+            hi = fma(d1, hr, ci); hr = nr;
+            const double mr = fma(-d2, gi, u.x);
+            gi = fma(d2, gr, u.y); gr = mr;
+        }
+        double sp, cp, s1, c1, s2, c2;
+        sincos(ph, &sp, &cp);
+        sincos(d1 * m.sxc, &s1, &c1);
+        sincos(d2 * m.sxc, &s2, &c2);
+        const double er = fma(cp, c1, -sp * s1), ei = fma(sp, c1, cp * s1);      // e^{i ph} e^{i d1 xc}
+        const double im1 = fma(er, hi, ei * hr);
+        const double pr = (cp - sp) * (cp + sp), pi = 2.0 * sp * cp;              // e^{2 i ph}
+        const double fr = fma(pr, c2, -pi * s2), fi = fma(pr, s2, pi * c2);      // ... e^{i d2 xc}
+        const double re2 = fma(fr, gr, -fi * gi);
+        const double* h = m.spec;                   // n, St, St2, Sd, Std, D2
+        const double line = fma(ac, fma(h[0], ac, 2.0 * fma(b, h[1], -h[3])), fma(b, fma(b, h[2], -2.0 * h[4]), h[5]));
+        const double w0 = a.w[0];
+        q = fma(amp * amp, 0.5 * (h[0] - re2), fma(2.0 * amp, im1, line)) * (w0 * w0);
+    }
+    if (live) a.partial[c] = q;
+#ifndef MC3B_NO_FUSE_CODE
+    if (a.f.on) fused_metropolis(a.f, a.partial, a.ldpartial, a.nchains, WARPS * 32, MomentFix{a});
+#endif
+}
+
 }  // namespace
+
+int mc3b_launch_spectral_chisq(const ChisqArgs<double>& a, unsigned groups, cudaStream_t st) {
+    k_spectral_chisq<<<groups, WARPS * 32, 0, st>>>(a);
+    MC3B_CHECK_LAUNCH("k_spectral_chisq");
+    return MC3B_OK;
+}
+
+int mc3b_launch_spectral_prepare(const double* x, const double* d, int64_t n, double c0ref, double slref,
+                                 const mc3b_spectral_t& s, cudaStream_t st) {
+    const unsigned nb = (unsigned)(s.n1 + s.n2 + 1);
+    if (s.order == 9)
+        k_spectral_table<9><<<nb, 256, 0, st>>>(x, d, n, c0ref, slref, s.xc, s.w1, s.w2, s.delta, s.n1, s.n2, s.table);
+    else
+        k_spectral_table<15><<<nb, 256, 0, st>>>(x, d, n, c0ref, slref, s.xc, s.w1, s.w2, s.delta, s.n1, s.n2, s.table);
+    MC3B_CHECK_LAUNCH("k_spectral_table");
+    return MC3B_OK;
+}
 
 int mc3b_launch_sinefold(const ChisqArgs<double>& a0, double* work, unsigned groups, unsigned nsplit, cudaStream_t st) {
     const bool mom = a0.m.folded != nullptr;

@@ -36,7 +36,7 @@ import torch
 
 from . import _lib
 from .models import BuiltinModel, CudaModel, TorchModel, SINUSOID, SINUSOID_GRID
-from . import gridseg
+from . import gridseg, spectral
 from .parallel import chain_slice, allgather_rows, gather_history, sum_owned
 
 
@@ -230,6 +230,7 @@ class Population:
             # MC3B_NO_MOMENT=1 disables.
             self.moment = None
             self.use_moment = False
+            self.spectral = None
             if self.d_fold is not None and nfold >= 256 \
                     and not os.environ.get('MC3B_NO_MOMENT') and not os.environ.get('MC3B_NO_FUSE'):
                 with torch.cuda.device(self.dev):
@@ -258,6 +259,29 @@ class Population:
                 M.xlo, M.xhi = float(x.min()), float(x.max())
                 M.guard_hits = self.guard_hits.data_ptr()
                 M.layout = layout
+                # ... and, where it applies, the spectral form of the same sum (k_spectral_chisq,
+                # include/mc3b200.h mc3b_spectral_t): chi-squared from a precomputed spectrum of the
+                # data, O(1) per chain instead of O(n).  Not with a period band that reaches 0,
+                # beyond the table's caps (spectral.plan), with the k_sinemma layout or with
+                # MC3B_NO_SPECTRAL=1: k_sinefold<MOM> as above.
+                self.spectral = None
+                wband = spectral.band(self.params, self.pstep, self.pmin, self.pmax)
+                plan = spectral.plan(float(x.min()), float(x.max()), *wband, x.size) \
+                    if wband is not None and layout == 0 and not os.environ.get('MC3B_NO_SPECTRAL') else None
+                if plan is not None:
+                    S = _lib.SpectralStruct()
+                    S.w1, S.w2, S.delta, S.xc = plan['w1'], plan['w2'], plan['delta'], plan['xc']
+                    S.n1, S.n2, S.order = plan['n1'], plan['n2'], plan['order']
+                    size = ctypes.c_int64(0)
+                    _lib.call('mc3b_spectral_size', S.n1, S.n2, S.order, ctypes.byref(size))
+                    with torch.cuda.device(self.dev):
+                        self.d_spectral = torch.zeros(size.value, **f64)
+                        S.table = self.d_spectral.data_ptr()
+                        _lib.call('mc3b_spectral_prepare', kx.data_ptr(), kd.data_ptr(), x.size, c0r, slr,
+                                  ctypes.byref(S), _lib.stream_ptr())
+                    self.spectral = S
+                    self.spectral_plan = plan
+                    M.spectral = ctypes.pointer(S)
                 self.moment = M
                 self.use_moment = True
                 self._guard_log = []          # (generation, ring slot) per run() call, oldest first
@@ -435,11 +459,12 @@ class Population:
             return nb
         return max(self.plan_chains, getattr(self, '_plan_rows', 0), nb)
 
-    def _plan(self, nb, moment=False):
-        key = (self._plan_chains(nb), bool(moment))
+    def _plan(self, nb, kind=0):
+        """kind: 0 general, 1 moment form, 2 its spectral form (MC3B_PLAN_*)."""
+        key = (self._plan_chains(nb), int(kind))
         if key not in self._plans:
             ns = ctypes.c_int(0)
-            _lib.call('mc3b_model_chisq_plan_kind', 1 if moment else 0, key[0], self.ndata, self.dtype,
+            _lib.call('mc3b_model_chisq_plan_kind', key[1], key[0], self.ndata, self.dtype,
                       ctypes.byref(ns))
             self._plans[key] = ns.value
         return self._plans[key]
@@ -535,7 +560,8 @@ class Population:
         if self.kind in ('builtin', 'cuda'):
             moment = bool(getattr(self, 'use_moment', False)) and self.d_fold is not None \
                 and (fuse is not None or moment_ok)
-            ns = self._plan(nb, moment)
+            spec = moment and self.moment.spectral
+            ns = self._plan(nb, 2 if spec else 1 if moment else 0)
             part = self._workspace(('part', nb, ns), (ns, nb))
             self._last_part = part
             o = _lib.ChisqOpts()
@@ -546,7 +572,7 @@ class Population:
                 o.ntiles = self.seg['starts'].size
             if self.d_fold is not None:
                 o.folded = self.d_fold.data_ptr()
-                if not os.environ.get('MC3B_NO_FOLD_CONSTS') or moment:
+                if (not os.environ.get('MC3B_NO_FOLD_CONSTS') or moment) and not spec:
                     o.work = self._workspace(('foldk', nb), (_lib.FOLD_WORK, nb)).data_ptr()
                     self.launches += 1
                 if moment:
