@@ -54,6 +54,7 @@ enum { MC3B_MRW = 0, MC3B_DEMC = 1, MC3B_SNOOKER = 2 };
 
 #define MC3B_MAX_PARS 32            /* parameters per model vector          */
 #define MC3B_MAX_SPLIT 4096         /* data splits of one chi-squared launch */
+#define MC3B_MAX_INPUTS 4           /* per-point inputs of a user model      */
 
 int mc3b_version(void);
 const char* mc3b_last_error(void);
@@ -285,6 +286,11 @@ int mc3b_model_eval(int model_id, const double* params, int64_t ldp,
  * models.cuh (fast_sin, fast_sincos_core, ...) is included.  NVRTC compiles it into
  * the kernels of the built-in models (csrc/chisq_kernel.cuh), so the model runs on the
  * same fused, TMA-staged, graph-capturable path.
+ *
+ * A model of several per-point inputs (ninputs = k, 1 <= k <= MC3B_MAX_INPUTS) takes k
+ * reals before the parameters:  __device__ real model(real t, real xc, real yc, const
+ * real* p)  for k = 3.  It is compiled with the _ex entry points and launched with the
+ * _inputs ones; the plain entry points are those of k = 1.
  * ---------------------------------------------------------------------- */
 typedef struct mc3b_user_model mc3b_user_model_t;          /* opaque */
 
@@ -320,6 +326,32 @@ int mc3b_user_model_chisq_ex(const mc3b_user_model_t* m, const double* params,
 int mc3b_user_model_eval(const mc3b_user_model_t* m, const double* params,
                          int64_t ldp, int64_t nchains, const double* x, int64_t n,
                          double* out, void* stream);
+
+/* mc3b_user_model_compile / _load for a model of `ninputs` per-point inputs
+ * (1..MC3B_MAX_INPUTS); ninputs = 1 is exactly the plain entry point.  A source whose
+ * `model` takes another number of inputs fails to compile (MC3B_ERR_ARG, see the log). */
+int mc3b_user_model_compile_ex(const char* nvrtc_path, const char* source, int nmodel,
+                               int ninputs, int dtype, void* cubin /*[host]*/,
+                               int64_t cap, int64_t* size /*[host]*/,
+                               char* log /*[host]*/, int64_t logcap);
+int mc3b_user_model_load_ex(const void* cubin /*[host]*/, int64_t size, int nmodel,
+                            int ninputs, int dtype, mc3b_user_model_t** out /*[host]*/);
+
+/* mc3b_user_model_chisq_ex and _eval with the inputs as an array xs [host] of nx
+ * device pointers (nx must equal the handle's ninputs), each n values of the
+ * handle's dtype (_chisq_inputs) or fp64 (_eval_inputs).  The plain entry points
+ * refuse a handle of more than one input (MC3B_ERR_ARG).  A launch whose inputs
+ * are not all 16-byte aligned reads them without TMA, as for an unaligned x. */
+int mc3b_user_model_chisq_inputs(const mc3b_user_model_t* m, const double* params,
+                                 int64_t ldp, int64_t nchains,
+                                 const void* const* xs /*[host] nx device pointers*/,
+                                 int nx, const void* data, const void* invsig, int64_t n,
+                                 double* partial, int64_t ldpartial, int nsplit,
+                                 const mc3b_chisq_opts_t* opts, void* stream);
+int mc3b_user_model_eval_inputs(const mc3b_user_model_t* m, const double* params,
+                                int64_t ldp, int64_t nchains,
+                                const double* const* xs /*[host] nx device pointers*/,
+                                int nx, int64_t n, double* out, void* stream);
 
 /* chisq[c] = sum_s partial[s*ldpartial + c] (fixed order s = 0..nsplit-1)
  *          + sum over j with priorlow_j > 0 and priorup_j > 0 of

@@ -14,6 +14,7 @@ F64, F32 = 0, 1
 MRW, DEMC, SNOOKER = 0, 1, 2
 SAMPLERS = {'mrw': MRW, 'demc': DEMC, 'snooker': SNOOKER}
 MAX_PARS = 32
+MAX_INPUTS = 4                    # MC3B_MAX_INPUTS: per-point inputs of a user model
 
 c_i64, c_i32, c_int = ctypes.c_int64, ctypes.c_int32, ctypes.c_int
 c_vp, c_dbl = ctypes.c_void_p, ctypes.c_double
@@ -102,6 +103,13 @@ _SIGS = {
     'mc3b_user_model_chisq_ex': (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64,
                                          c_int, ctypes.POINTER(ChisqOpts), c_vp]),
     'mc3b_user_model_eval': (c_int, [c_vp, c_vp, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp]),
+    'mc3b_user_model_compile_ex': (c_int, [ctypes.c_char_p, ctypes.c_char_p, c_int, c_int, c_int, c_vp, c_i64,
+                                           ctypes.POINTER(c_i64), ctypes.c_char_p, c_i64]),
+    'mc3b_user_model_load_ex': (c_int, [ctypes.c_char_p, c_i64, c_int, c_int, c_int, ctypes.POINTER(c_vp)]),
+    'mc3b_user_model_chisq_inputs': (c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.POINTER(c_vp), c_int, c_vp, c_vp,
+                                             c_i64, c_vp, c_i64, c_int, ctypes.POINTER(ChisqOpts), c_vp]),
+    'mc3b_user_model_eval_inputs': (c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.POINTER(c_vp), c_int, c_i64, c_vp,
+                                            c_vp]),
     'mc3b_chisq_finish': (c_int, [c_vp, c_i64, c_int, c_i64, c_vp, c_i64, c_int,
                                   c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mc3b_chisq_batch': (c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp]),
@@ -173,6 +181,12 @@ def call(name, *args):
         msg = lib.mc3b_last_error().decode('utf-8', 'replace')
         raise Mc3bError(f'{name} failed (status {rc}): {msg}')
     return rc
+
+
+def ptrs(ts):
+    """Host array of the device pointers of torch tensors (the `xs` of the
+    mc3b_user_model_*_inputs entry points)."""
+    return (c_vp*len(ts))(*[t.data_ptr() for t in ts])
 
 
 def ptr(t):

@@ -81,7 +81,14 @@ template <typename T> struct ChisqArgs {
     int64_t ldpartial;
     int use_tma;
     FuseArgs f;
+    // the inputs of a user model of NX per-point inputs (xs[0] = x).  After every other
+    // field, so that the built-in kernels read the same offsets; 32 bytes, so that the
+    // parameters after this block keep their 16-byte alignment (wide constant loads)
+    const T* xs[MC3B_MAX_INPUTS];
 };
+
+// Inputs of the model-value kernel of a user model of several inputs (k_model_eval_x).
+struct EvalInputs { const double* x[MC3B_MAX_INPUTS]; };
 
 // The Metropolis step itself, compiled once per translation unit: S points to the
 // CTA's shared-memory copy of the sampler description.

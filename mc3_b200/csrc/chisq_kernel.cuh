@@ -10,7 +10,8 @@
 //   warp  = LC chains x LP = 32/LC point lanes.  LC = 32: one chain per lane,
 //           every lane walks all points of a tile (shared-memory broadcast);
 //           LC = 8 / 1: fewer chains, lanes share the points of the tile.
-//   data  = x, data, 1/sigma tiles of TILE points, staged into shared memory
+//   data  = x, data, 1/sigma tiles of TILE points (and the tiles of inputs 2..NX
+//           of a user model of several inputs), staged into shared memory
 //           by 1-D TMA bulk copies (cp.async.bulk + mbarrier, 3 stages), so a
 //           tile is fetched once per CTA and serves all its chains; the
 //           per-chain constants live in registers for the whole launch.
@@ -39,11 +40,16 @@ template <class M, typename T, int LC, int CPT, bool USIG>
 __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESIDENT)) k_model_chisq(ChisqArgs<T> a) {
     constexpr int TILE = tilecfg<T>::TILE;
     constexpr int LP = 32 / LC;
+    constexpr int NX = ninputs_of<M>::value;
+    static_assert(NX >= 1 && NX <= MC3B_MAX_INPUTS && (NX == 1 || (!M::GUARD && !M::TILE_STATE)),
+                  "models of several inputs have neither guard nor tile state");
     asm volatile("griddepcontrol.launch_dependents;");   // the next proposal kernel may start its draws
     __shared__ __align__(128) T sx[STAGES][TILE];
     __shared__ __align__(128) T sd[STAGES][TILE];
     __shared__ __align__(128) T sw[STAGES][TILE];
     __shared__ __align__(8) uint64_t bar[STAGES];
+    // inputs 2..NX: declared only for a model of several inputs (as sdw for PM below)
+    __shared__ __align__(128) T sxe[NX > 1 ? STAGES : 1][NX > 1 ? NX - 1 : 1][NX > 1 ? TILE : 2];
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int lc = lane % LC, lp = lane / LC;
@@ -81,10 +87,14 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
         __syncthreads();
         auto issue = [&](int64_t t, int s) {
             const int64_t off = t * TILE;
-            mbar_expect_tx(&bar[s], (USIG ? 2u : 3u) * TILE * sizeof(T));
+            mbar_expect_tx(&bar[s], ((USIG ? 2u : 3u) + (unsigned)(NX - 1)) * TILE * sizeof(T));
             bulk_g2s(sx[s], a.x + off, TILE * sizeof(T), &bar[s]);
             bulk_g2s(sd[s], a.d + off, TILE * sizeof(T), &bar[s]);
             if constexpr (!USIG) bulk_g2s(sw[s], a.w + off, TILE * sizeof(T), &bar[s]);
+            if constexpr (NX > 1) {
+#pragma unroll
+                for (int j = 0; j < NX - 1; j++) bulk_g2s(sxe[s][j], a.xs[j + 1] + off, TILE * sizeof(T), &bar[s]);
+            }
         };
         if (threadIdx.x == 0)
             for (int s = 0; s < STAGES && s < nt; s++) issue(tb + s, s);
@@ -124,9 +134,19 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
                 T x[U], y[U];
 #pragma unroll
                 for (int u = 0; u < U; u++) x[u] = sx[s][i + u * LP];
+                T xv[NX][U];                    // NX > 1: every input of the U points
+                if constexpr (NX > 1) {
+#pragma unroll
+                    for (int u = 0; u < U; u++) {
+                        xv[0][u] = x[u];
+#pragma unroll
+                        for (int j = 1; j < NX; j++) xv[j][u] = sxe[s][j - 1][i + u * LP];
+                    }
+                }
 #pragma unroll
                 for (int k = 0; k < CPT; k++) {
-                    eval_points<M, T, U>(mdl[k], x, y, 0);
+                    if constexpr (NX == 1) eval_points<M, T, U>(mdl[k], x, y, 0);
+                    else eval_points<M, T, NX, U>(mdl[k], xv, y);
 #pragma unroll
                     for (int u = 0; u < U; u++) {
                         const T r = USIG ? y[u] - sd[s][i + u * LP]
@@ -138,7 +158,7 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
             }
 #pragma unroll
             for (int k = 0; k < CPT; k++) tacc[k] = (uacc[k][0] + uacc[k][1]) + (uacc[k][2] + uacc[k][3]);
-            if (M::GUARD) {                     // extreme model arguments: redo the tile safely
+            if constexpr (M::GUARD) {           // extreme model arguments: redo the tile safely
 #pragma unroll
                 for (int k = 0; k < CPT; k++) {
                     if (mdl[k].flagged()) {
@@ -167,6 +187,10 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
             __syncthreads();
             for (int i = threadIdx.x; i < TILE; i += WARPS * 32) {
                 sx[0][i] = a.x[off + i]; sd[0][i] = a.d[off + i]; sw[0][i] = USIG ? (T)1 : a.w[off + i];
+                if constexpr (NX > 1) {
+#pragma unroll
+                    for (int j = 0; j < NX - 1; j++) sxe[0][j][i] = a.xs[j + 1][off + i];
+                }
             }
             __syncthreads();
             T tacc[CPT];
@@ -174,9 +198,13 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
             for (int k = 0; k < CPT; k++) tacc[k] = (T)0;
             for (int i = lp; i < TILE; i += LP) {
                 const T x = sx[0][i], d = sd[0][i], w = sw[0][i];
+                T v[NX];
+                v[0] = x;
+#pragma unroll
+                for (int j = 1; j < NX; j++) v[j] = sxe[0][j - 1][i];
 #pragma unroll
                 for (int k = 0; k < CPT; k++) {
-                    const T r = (mdl[k].eval_safe(x) - d) * w;
+                    const T r = (eval_safe_at(mdl[k], v) - d) * w;
                     tacc[k] = fma(r, r, tacc[k]);
                 }
             }
@@ -192,9 +220,13 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
         for (int k = 0; k < CPT; k++) tacc[k] = (T)0;
         for (int64_t i = nfull * TILE + lp; i < a.n; i += LP) {
             const T x = a.x[i], d = a.d[i], w = USIG ? (T)1 : a.w[i];
+            T v[NX];
+            v[0] = x;
+#pragma unroll
+            for (int j = 1; j < NX; j++) v[j] = a.xs[j][i];
 #pragma unroll
             for (int k = 0; k < CPT; k++) {
-                const T r = (mdl[k].eval_safe(x) - d) * w;
+                const T r = (eval_safe_at(mdl[k], v) - d) * w;
                 tacc[k] = fma(r, r, tacc[k]);
             }
         }
@@ -223,6 +255,21 @@ __global__ void k_model_eval(const double* params, int64_t ldp, const double* x,
     m.load(params + (int64_t)blockIdx.y * ldp);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         out[(int64_t)blockIdx.y * n + i] = m.eval_safe(x[i]);
+}
+
+// ... of a model of NX > 1 inputs: input j of point i is xs.x[j][i]
+template <class M>
+__global__ void k_model_eval_x(const double* params, int64_t ldp, EvalInputs xs, int64_t n, double* out) {
+    constexpr int NX = ninputs_of<M>::value;
+    using T = typename M::real;
+    M m;
+    m.load(params + (int64_t)blockIdx.y * ldp);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        T v[NX];
+#pragma unroll
+        for (int j = 0; j < NX; j++) v[j] = (T)xs.x[j][i];
+        out[(int64_t)blockIdx.y * n + i] = m.eval_safe(v);
+    }
 }
 
 }  // namespace

@@ -318,6 +318,10 @@ template <typename T> struct BoxModel {
 
 template <class M, typename = void> struct premul_of { static constexpr bool value = false; };
 template <class M> struct premul_of<M, decltype((void)M::PREMUL)> { static constexpr bool value = M::PREMUL; };
+// Per-point inputs a model reads (M::NX; 1 unless the model says otherwise): a model of
+// NX > 1 inputs has eval(const T (&v)[NX]) and eval_safe likewise.
+template <class M, typename = void> struct ninputs_of { static constexpr int value = 1; };
+template <class M> struct ninputs_of<M, decltype((void)M::NX)> { static constexpr int value = M::NX; };
 
 // y[u] = model(x[u]) for U points at once.  Models may provide their own evalN
 // (stage-by-stage over the U points, so that in-order issue sees U independent
@@ -330,6 +334,23 @@ template <class M, typename T, int U>
 __device__ __forceinline__ void eval_points(M& m, const T (&x)[U], T (&y)[U], long) {
 #pragma unroll
     for (int u = 0; u < U; u++) y[u] = m.eval(x[u]);
+}
+// ... and for a model of NX > 1 inputs: x[j][u] is input j of point u.
+template <class M, typename T, int NX, int U>
+__device__ __forceinline__ void eval_points(M& m, const T (&x)[NX][U], T (&y)[U]) {
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+        T v[NX];
+#pragma unroll
+        for (int j = 0; j < NX; j++) v[j] = x[j][u];
+        y[u] = m.eval(v);
+    }
+}
+// m.eval_safe at one point, v[j] = input j (the plain call for a model of one input).
+template <class M, typename T, int NX>
+__device__ __forceinline__ T eval_safe_at(const M& m, const T (&v)[NX]) {
+    if constexpr (NX == 1) return m.eval_safe(v[0]);
+    else return m.eval_safe(v);
 }
 
 // Dispatch a generic lambda-like functor F<Model> over (model_id, nmodel).

@@ -11,7 +11,7 @@ The reference's `func` is any Python callable `func(params, *indparams,
   on the device;
 * a CudaModel: the user's own formula as a CUDA device function, compiled at run
   time (NVRTC, mc3_b200/jit.py) into the same fused kernel as the built-in models --
-  the fast path for any model of one abscissa:
+  the fast path for any model of up to MAX_INPUTS (4) per-point inputs:
 
       transit = CudaModel('''
           __device__ real model(real x, const real* p) {      // p[0..nparams)
@@ -21,8 +21,11 @@ The reference's `func` is any Python callable `func(params, *indparams,
 
   `real` is double (float with dtype='f32'); models.cuh is included, so fast_sin and
   fast_sincos_core are available.  nparams counts the parameters the model itself
-  consumes (with wlike=True it gets params[0:-3]), at most 32.  The source compiles on
-  first use; a compile error raises ValueError with the NVRTC log;
+  consumes (with wlike=True it gets params[0:-3]), at most 32.  With ninputs=k the
+  model takes k reals before the parameters, `model(real t, real xc, real yc, const
+  real* p)` for k = 3, and the fit passes k arrays of the data's shape as indparams,
+  in the same order.  The source compiles on first use; a compile error raises
+  ValueError with the NVRTC log;
 * a TorchModel: a user torch callable evaluated ONCE per generation over the
   whole population, `fn(P[nchains, npars], *indparams) -> model[nchains, N]`
   on the device;
@@ -83,16 +86,18 @@ class BuiltinModel:
         return f'<mc3_b200 built-in model {self.name}>'
 
 
-def _eval_rows(params, x, launch):
-    """model(params, x) on the current GPU: [nrows, N] (or [N] for one row)."""
+def _eval_rows(params, xs, launch):
+    """model(params, *xs) on the current GPU: [nrows, N] (or [N] for one row)."""
     import torch
     params = np.atleast_2d(np.asarray(params, dtype=np.double))
-    x = np.ascontiguousarray(x, dtype=np.double)
+    xs = [np.ascontiguousarray(x, dtype=np.double) for x in xs]
+    if any(x.shape != xs[0].shape for x in xs):
+        raise ValueError('the input arrays of a model must have one shape')
     dev = torch.device('cuda')
     dp = torch.from_numpy(np.ascontiguousarray(params)).to(dev)
-    dx = torch.from_numpy(x).to(dev)
-    out = torch.empty((params.shape[0], x.size), dtype=torch.float64, device=dev)
-    launch(dp, dx, out)
+    dxs = [torch.from_numpy(x).to(dev) for x in xs]
+    out = torch.empty((params.shape[0], xs[0].size), dtype=torch.float64, device=dev)
+    launch(dp, dxs, out)
     res = out.cpu().numpy()
     return res[0] if res.shape[0] == 1 else res
 
@@ -100,20 +105,31 @@ def _eval_rows(params, x, launch):
 class CudaModel:
     """A user model written as a CUDA device function (see the module docstring):
     `__device__ real model(real x, const real* p)` in `source`, taking `nparams`
-    parameters.  Compiled lazily, once per process and dtype; pickles as its source
+    parameters, or with ninputs = k > 1 inputs `model(real x1, ..., real xk, const
+    real* p)`.  Compiled lazily, once per process and dtype; pickles as its source
     (one process per GPU receives it and compiles its own copy)."""
 
-    def __init__(self, source, nparams, name='cuda_model'):
+    ninputs = 1            # stored on the instance only when it is not 1
+
+    def __init__(self, source, nparams, name='cuda_model', ninputs=1):
         nparams = int(nparams)
         if not 1 <= nparams <= _lib.MAX_PARS:
             raise ValueError(f'a CudaModel takes 1 to {_lib.MAX_PARS} parameters, got {nparams}')
+        ninputs = int(ninputs)
+        if not 1 <= ninputs <= _lib.MAX_INPUTS:
+            raise ValueError(f'a CudaModel takes 1 to {_lib.MAX_INPUTS} inputs, got {ninputs}')
         self.source, self.nparams, self.name = str(source), nparams, str(name)
+        if ninputs != 1:
+            self.ninputs = ninputs
 
     def __getstate__(self):
-        return {'source': self.source, 'nparams': self.nparams, 'name': self.name}
+        state = {'source': self.source, 'nparams': self.nparams, 'name': self.name}
+        if self.ninputs != 1:
+            state['ninputs'] = self.ninputs
+        return state
 
     def __setstate__(self, state):
-        self.__init__(state['source'], state['nparams'], state['name'])
+        self.__init__(state['source'], state['nparams'], state['name'], state.get('ninputs', 1))
 
     def nmodel(self, nfunc_params):
         """Number of leading parameters the model consumes."""
@@ -124,24 +140,31 @@ class CudaModel:
 
     def cache_key(self, dtype=_lib.F64):
         from . import jit
-        return jit.cache_key(self.source, self.nparams, dtype)
+        return jit.cache_key(self.source, self.nparams, dtype, self.ninputs)
 
     def handle(self, dtype=_lib.F64, stats=None):
         """mc3b_user_model_t* of this model for dtype (_lib.F64 / _lib.F32)."""
         from . import jit
-        return jit.handle(self.source, self.nparams, dtype, self.name, stats)
+        return jit.handle(self.source, self.nparams, dtype, self.name, stats, self.ninputs)
 
-    def __call__(self, params, x):
+    def __call__(self, params, *xs):
+        if len(xs) != self.ninputs:
+            raise ValueError(f'{self.name} takes {self.ninputs} input array(s), got {len(xs)}')
         self.nmodel(np.shape(np.atleast_2d(params))[1])
         h = self.handle(_lib.F64)
 
-        def launch(dp, dx, out):
-            _lib.call('mc3b_user_model_eval', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
-                      dx.data_ptr(), dx.numel(), out.data_ptr(), _lib.stream_ptr())
-        return _eval_rows(params, x, launch)
+        def launch(dp, dxs, out):
+            if self.ninputs == 1:
+                _lib.call('mc3b_user_model_eval', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
+                          dxs[0].data_ptr(), dxs[0].numel(), out.data_ptr(), _lib.stream_ptr())
+            else:
+                _lib.call('mc3b_user_model_eval_inputs', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
+                          _lib.ptrs(dxs), len(dxs), dxs[0].numel(), out.data_ptr(), _lib.stream_ptr())
+        return _eval_rows(params, xs, launch)
 
     def __repr__(self):
-        return f'<mc3_b200 CUDA model {self.name} ({self.nparams} parameters)>'
+        inputs = f', {self.ninputs} inputs' if self.ninputs != 1 else ''
+        return f'<mc3_b200 CUDA model {self.name} ({self.nparams} parameters{inputs})>'
 
 
 class TorchModel:
