@@ -353,6 +353,48 @@ int mc3b_user_model_eval_inputs(const mc3b_user_model_t* m, const double* params
                                 const double* const* xs /*[host] nx device pointers*/,
                                 int nx, int64_t n, double* out, void* stream);
 
+/* A model of run-time constants and a per-chain prepare step.  The array p that
+ * `model` sees has nmodel + nconst + nwork slots (at most MC3B_MAX_PARS):
+ * [parameters | constants | work].  The constants come with each launch, so their
+ * values are not compiled into the module.  The source may define
+ *     __device__ void prepare(real* p)
+ * which runs once per chain wherever the parameters are loaded (once per chain and
+ * CTA), after the constants, and may write any slot of that private copy: the place to
+ * hoist what depends on the chain alone (1/sigma, 2 pi/P) into the work slots.  It is
+ * found by name lookup, so a comment that mentions it does not count; a `prepare` that
+ * cannot be called with a real* fails to compile at its own line, and nwork > 0 without
+ * one is refused (MC3B_ERR_ARG).  nconst = nwork = 0 with no prepare is exactly
+ * mc3b_user_model_compile_ex / _load_ex. */
+typedef struct {
+    int nmodel, ninputs, nconst, nwork, dtype;
+} mc3b_user_model_desc_t;
+
+int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* source,
+                                 const mc3b_user_model_desc_t* desc /*[host]*/,
+                                 void* cubin /*[host]*/, int64_t cap,
+                                 int64_t* size /*[host]*/, char* log /*[host]*/,
+                                 int64_t logcap);
+int mc3b_user_model_load_desc(const void* cubin /*[host]*/, int64_t size,
+                              const mc3b_user_model_desc_t* desc /*[host]*/,
+                              mc3b_user_model_t** out /*[host]*/);
+
+/* _chisq_inputs and _eval_inputs with the nk constants at `consts` [device], in the
+ * handle's dtype (_chisq_consts) or fp64 (_eval_consts); nk must equal the handle's
+ * nconst, and consts may be NULL when it is 0.  They take every handle; the entry points
+ * above refuse one of nconst > 0 (MC3B_ERR_ARG). */
+int mc3b_user_model_chisq_consts(const mc3b_user_model_t* m, const double* params,
+                                 int64_t ldp, int64_t nchains,
+                                 const void* const* xs /*[host] nx device pointers*/,
+                                 int nx, const void* consts, int nk, const void* data,
+                                 const void* invsig, int64_t n, double* partial,
+                                 int64_t ldpartial, int nsplit,
+                                 const mc3b_chisq_opts_t* opts, void* stream);
+int mc3b_user_model_eval_consts(const mc3b_user_model_t* m, const double* params,
+                                int64_t ldp, int64_t nchains,
+                                const double* const* xs /*[host] nx device pointers*/,
+                                int nx, const double* consts, int nk, int64_t n,
+                                double* out, void* stream);
+
 /* chisq[c] = sum_s partial[s*ldpartial + c] (fixed order s = 0..nsplit-1)
  *          + sum over j with priorlow_j > 0 and priorup_j > 0 of
  *            ((p_cj - prior_j) / (p_cj > prior_j ? priorup_j : priorlow_j))^2

@@ -65,6 +65,11 @@ class ChisqOpts(ctypes.Structure):
                 ('ntiles', c_i64)]
 
 
+class UserModelDesc(ctypes.Structure):
+    """mc3b_user_model_desc_t."""
+    _fields_ = [('nmodel', c_int), ('ninputs', c_int), ('nconst', c_int), ('nwork', c_int), ('dtype', c_int)]
+
+
 FOLD_WORK = 27                    # MC3B_FOLD_WORK
 
 
@@ -110,6 +115,14 @@ _SIGS = {
                                              c_i64, c_vp, c_i64, c_int, ctypes.POINTER(ChisqOpts), c_vp]),
     'mc3b_user_model_eval_inputs': (c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.POINTER(c_vp), c_int, c_i64, c_vp,
                                             c_vp]),
+    'mc3b_user_model_compile_desc': (c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.POINTER(UserModelDesc), c_vp,
+                                             c_i64, ctypes.POINTER(c_i64), ctypes.c_char_p, c_i64]),
+    'mc3b_user_model_load_desc': (c_int, [ctypes.c_char_p, c_i64, ctypes.POINTER(UserModelDesc),
+                                          ctypes.POINTER(c_vp)]),
+    'mc3b_user_model_chisq_consts': (c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.POINTER(c_vp), c_int, c_vp, c_int,
+                                             c_vp, c_vp, c_i64, c_vp, c_i64, c_int, ctypes.POINTER(ChisqOpts), c_vp]),
+    'mc3b_user_model_eval_consts': (c_int, [c_vp, c_vp, c_i64, c_i64, ctypes.POINTER(c_vp), c_int, c_vp, c_int,
+                                            c_i64, c_vp, c_vp]),
     'mc3b_chisq_finish': (c_int, [c_vp, c_i64, c_int, c_i64, c_vp, c_i64, c_int,
                                   c_vp, c_vp, c_vp, c_vp, c_vp]),
     'mc3b_chisq_batch': (c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp]),

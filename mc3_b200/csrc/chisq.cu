@@ -215,6 +215,7 @@ int mc3b_chisq_setup(const double* params, int64_t ldp, int64_t nchains, const v
     A.xt = nullptr; A.dxg = 0.0; A.ntiles = 0; A.partial = partial; A.ldpartial = ldpartial;
     A.xs[0] = (const T*)x;
     for (int j = 1; j < MC3B_MAX_INPUTS; j++) A.xs[j] = nullptr;
+    A.uconst = nullptr; A.uconst_pad = nullptr;
     const bool usig = o.uniform_sigma != 0;
     A.use_tma = ((((uintptr_t)x | (uintptr_t)d | (usig ? 0 : (uintptr_t)w)) & 15) == 0) ? 1 : 0;
     const int64_t plan_chains = o.plan_chains > 0 ? o.plan_chains : nchains;

@@ -85,9 +85,14 @@ template <typename T> struct ChisqArgs {
     // field, so that the built-in kernels read the same offsets; 32 bytes, so that the
     // parameters after this block keep their 16-byte alignment (wide constant loads)
     const T* xs[MC3B_MAX_INPUTS];
+    // the run-time constants of a user model (mc3b_user_model_chisq_consts), nullptr when it
+    // has none; padded to 16 bytes for the same reason as xs
+    const T* uconst;
+    const void* uconst_pad;
 };
 
-// Inputs of the model-value kernel of a user model of several inputs (k_model_eval_x).
+// Inputs of the model-value kernels of a user model of several inputs or of constants
+// (k_model_eval_x, k_model_eval_k).
 struct EvalInputs { const double* x[MC3B_MAX_INPUTS]; };
 
 // The Metropolis step itself, compiled once per translation unit: S points to the

@@ -63,6 +63,8 @@ __global__ void __launch_bounds__(WARPS * 32, (CPT == 2 ? MC3B_RESIDENT2 : RESID
         if constexpr (M::TILE_STATE) {
             const double dx = ((double)a.x[a.n - 1] - (double)a.x[0]) / (double)(a.n - 1);
             mdl[k].load(a.params + c * a.ldp, dx, TILE);
+        } else if constexpr (takes_consts<M>::value) {
+            mdl[k].load(a.params + c * a.ldp, a.uconst);
         } else {
             mdl[k].load(a.params + c * a.ldp);
         }
@@ -269,6 +271,23 @@ __global__ void k_model_eval_x(const double* params, int64_t ldp, EvalInputs xs,
 #pragma unroll
         for (int j = 0; j < NX; j++) v[j] = (T)xs.x[j][i];
         out[(int64_t)blockIdx.y * n + i] = m.eval_safe(v);
+    }
+}
+
+// ... of a model of run-time constants or a prepare step (takes_consts), any NX: the
+// constants k are fp64 here whatever the model's type
+template <class M>
+__global__ void k_model_eval_k(const double* params, int64_t ldp, EvalInputs xs, const double* k, int64_t n,
+                               double* out) {
+    constexpr int NX = ninputs_of<M>::value;
+    using T = typename M::real;
+    M m;
+    m.load(params + (int64_t)blockIdx.y * ldp, k);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        T v[NX];
+#pragma unroll
+        for (int j = 0; j < NX; j++) v[j] = (T)xs.x[j][i];
+        out[(int64_t)blockIdx.y * n + i] = eval_safe_at(m, v);
     }
 }
 

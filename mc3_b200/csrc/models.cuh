@@ -322,6 +322,10 @@ template <class M> struct premul_of<M, decltype((void)M::PREMUL)> { static const
 // NX > 1 inputs has eval(const T (&v)[NX]) and eval_safe likewise.
 template <class M, typename = void> struct ninputs_of { static constexpr int value = 1; };
 template <class M> struct ninputs_of<M, decltype((void)M::NX)> { static constexpr int value = M::NX; };
+// A model that declares M::NC (a user model of run-time constants, or of a prepare step) is
+// loaded with load(p, k): its parameters, then the NC constants k[0..NC).  Others: load(p).
+template <class M, typename = void> struct takes_consts { static constexpr bool value = false; };
+template <class M> struct takes_consts<M, decltype((void)M::NC)> { static constexpr bool value = true; };
 
 // y[u] = model(x[u]) for U points at once.  Models may provide their own evalN
 // (stage-by-stage over the U points, so that in-order issue sees U independent

@@ -7,7 +7,7 @@ launches through the C ABI (include/mc3b200.h):
 
     mc3b_propose      draws, jump, bounds, shared fill        chain.py:185-247
     mc3b_model_chisq  built-in model + chi-squared, all chains  chain.py:249, 302-340
-                      (mc3b_user_model_chisq_inputs for a CudaModel: the same kernel)
+                      (mc3b_user_model_chisq_consts for a CudaModel: the same kernel)
     mc3b_metropolis   partial sums + priors, accept, write    chain.py:251-289
 
 advancing every chain in lock-step (SURVEY.md finding 6: within one generation
@@ -174,10 +174,13 @@ class Population:
             # model values are fp64 whatever the dtype, as mc3b_model_eval's
             self.jit_eval = func.handle(_lib.F64) if user else None
             nin = func.ninputs if user else 1
+            # a CudaModel of run-time constants: the indparams after its inputs, flattened
+            # (CudaModel.split_args); every rank builds its own copy
+            xargs, kc = func.split_args(self.indparams) if user else (self.indparams, None)
             if nin > 1:
                 # a CudaModel of several inputs: one 1-D array per input, in the order of
                 # the arguments of its `model`
-                xin = [np.ascontiguousarray(a, dtype=np.double) for a in self.indparams]
+                xin = [np.ascontiguousarray(a, dtype=np.double) for a in xargs]
                 if len(xin) != nin or any(a.ndim != 1 or a.size != self.ndata_total for a in xin):
                     raise ValueError(f'CudaModel {func.name!r} takes {nin} inputs: it needs indparams=[x1, ..., '
                                      f'x{nin}], {nin} 1-D arrays with the same shape as data (got '
@@ -189,10 +192,13 @@ class Population:
             x = x[lo:hi]
             self.d_x = torch.from_numpy(x).to(self.dev)
             # every input of the model on the device (d_xs[0] is d_x); their host array of
-            # pointers is what mc3b_user_model_eval_inputs takes
+            # pointers is what mc3b_user_model_eval_consts takes
             self.d_xs = [self.d_x] + [torch.from_numpy(a[lo:hi]).to(self.dev) for a in xin[1:]] \
                 if nin > 1 else [self.d_x]
             self.d_xptrs = _lib.ptrs(self.d_xs)
+            # ... and its constants, fp64 (model values) and in the kernel's dtype; None: none
+            self.d_kc = torch.from_numpy(kc).to(self.dev) if kc is not None and kc.size else None
+            self.nconst = func.nconst if user else 0
             self.d_invsig = 1.0/self.d_uncert
             # one uncertainty for all points: no weight stream, residuals are plain
             # differences (mc3b_chisq_opts_t.uniform_sigma); MC3B_NO_USIG=1 disables
@@ -311,6 +317,7 @@ class Population:
                 self.k_x, self.k_d, self.k_w = kx, kd, kw
                 self.k_xs = [self.k_x] + self.d_xs[1:]
             self.k_xptrs = _lib.ptrs(self.k_xs)
+            self.k_kc = self.d_kc.float() if self.d_kc is not None and self.dtype == _lib.F32 else self.d_kc
         elif self.shard == 'data':
             raise ValueError("shard='data' needs a built-in model")
         elif isinstance(func, TorchModel):
@@ -497,8 +504,9 @@ class Population:
         """Model values [nb, N] on the device for non-built-in models."""
         if self.kind == 'cuda':
             rows = self._workspace(('mrows', P.shape[0]), (P.shape[0], self.ndata))
-            _lib.call('mc3b_user_model_eval_inputs', self.jit_eval, P.data_ptr(), _lib.ld(P), P.shape[0],
-                      self.d_xptrs, len(self.d_xs), self.ndata, rows.data_ptr(), _lib.stream_ptr())
+            _lib.call('mc3b_user_model_eval_consts', self.jit_eval, P.data_ptr(), _lib.ld(P), P.shape[0],
+                      self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst, self.ndata,
+                      rows.data_ptr(), _lib.stream_ptr())
             self.launches += 1
             return rows
         if self.kind == 'torch':
@@ -601,8 +609,9 @@ class Population:
                 o.fuse = ctypes.pointer(self.S)
                 o.fuse_done = self.fuse_done.data_ptr()
             if self.kind == 'cuda':
-                _lib.call('mc3b_user_model_chisq_inputs', self.jit, P.data_ptr(), _lib.ld(P), nb,
-                          self.k_xptrs, len(self.k_xs), self.k_d.data_ptr(), self.k_w.data_ptr(),
+                _lib.call('mc3b_user_model_chisq_consts', self.jit, P.data_ptr(), _lib.ld(P), nb,
+                          self.k_xptrs, len(self.k_xs), _lib.ptr(self.k_kc), self.nconst,
+                          self.k_d.data_ptr(), self.k_w.data_ptr(),
                           self.ndata, part.data_ptr(), nb, ns, ctypes.byref(o), st)
             else:
                 _lib.call('mc3b_model_chisq_ex', self.chisq_model_id, self.dtype,
@@ -627,8 +636,9 @@ class Population:
         P = torch.as_tensor(np.atleast_2d(np.asarray(fpar, dtype=np.double)), device=self.dev)
         out = torch.empty((1, self.ndata), dtype=torch.float64, device=self.dev)
         if self.kind == 'cuda':
-            _lib.call('mc3b_user_model_eval_inputs', self.jit_eval, P.data_ptr(), P.shape[1], 1,
-                      self.d_xptrs, len(self.d_xs), self.ndata, out.data_ptr(), _lib.stream_ptr())
+            _lib.call('mc3b_user_model_eval_consts', self.jit_eval, P.data_ptr(), P.shape[1], 1,
+                      self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst, self.ndata,
+                      out.data_ptr(), _lib.stream_ptr())
         else:
             _lib.call('mc3b_model_eval', self.func.model_id, P.data_ptr(), P.shape[1], 1,
                       self.nmodel, self.d_x.data_ptr(), self.ndata, out.data_ptr(),

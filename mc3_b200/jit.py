@@ -11,7 +11,8 @@ is used; the library dlopen's the same path.
 
 Compiled CUBINs are kept in memory per process, and on disk in the directory named
 by MC3B_JIT_CACHE when it is set.  The key covers the source, the parameter count,
-the number of inputs, the dtype, MC3B_VERSION, the NVRTC version and the embedded kernel headers; the
+the number of inputs, constants and work slots, the dtype, MC3B_VERSION, the NVRTC version and the
+embedded kernel headers (not the values of the constants: they are run-time data); the
 loader also checks the module's own ABI record, so a stale file is compiled again
 rather than launched.
 """
@@ -89,21 +90,30 @@ def _headers_digest():
     return _HEADERS
 
 
-def cache_key(source, nmodel, dtype, ninputs=1):
+def cache_key(source, nmodel, dtype, ninputs=1, nconst=0, nwork=0):
     """Hex key of one compiled model (dtype: _lib.F64 or _lib.F32).  A model of one
-    input keeps the key it had before models took several inputs."""
+    input and no constants or work slots keeps the key it had before models took
+    several inputs."""
     _, ver = find_nvrtc()
     h = hashlib.sha256()
     parts = [source, str(int(nmodel)), str(int(dtype)), str(_lib.load().mc3b_version()),
              f'{ver[0]}.{ver[1]}', _headers_digest()]
     if int(ninputs) != 1:
         parts.append(f'ninputs={int(ninputs)}')
+    if int(nconst) != 0:
+        parts.append(f'nconst={int(nconst)}')
+    if int(nwork) != 0:
+        parts.append(f'nwork={int(nwork)}')
     for part in parts:
         h.update(part.encode() + b'\0')
     return h.hexdigest()
 
 
-def compile_cubin(source, nmodel, dtype, name='model', ninputs=1):
+def _desc(nmodel, dtype, ninputs, nconst, nwork):
+    return ctypes.byref(_lib.UserModelDesc(int(nmodel), int(ninputs), int(nconst), int(nwork), int(dtype)))
+
+
+def compile_cubin(source, nmodel, dtype, name='model', ninputs=1, nconst=0, nwork=0):
     """NVRTC: source -> sm_100a CUBIN bytes.  ValueError with the log when the source
     does not compile."""
     path, _ = find_nvrtc()
@@ -113,8 +123,8 @@ def compile_cubin(source, nmodel, dtype, name='model', ninputs=1):
     lib = _lib.load()
     while True:
         buf = ctypes.create_string_buffer(cap)
-        rc = lib.mc3b_user_model_compile_ex(path.encode(), source.encode(), int(nmodel), int(ninputs), int(dtype),
-                                            buf, cap, ctypes.byref(size), log, len(log))
+        rc = lib.mc3b_user_model_compile_desc(path.encode(), source.encode(), _desc(nmodel, dtype, ninputs, nconst, nwork),
+                                              buf, cap, ctypes.byref(size), log, len(log))
         if rc == _lib.ERR_ARG and size.value > cap:
             cap = size.value
             continue
@@ -128,18 +138,18 @@ def compile_cubin(source, nmodel, dtype, name='model', ninputs=1):
     return buf.raw[:size.value]
 
 
-def _load(cubin, nmodel, dtype, ninputs=1):
+def _load(cubin, nmodel, dtype, ninputs=1, nconst=0, nwork=0):
     h = ctypes.c_void_p()
-    rc = _lib.load().mc3b_user_model_load_ex(cubin, len(cubin), int(nmodel), int(ninputs), int(dtype),
-                                             ctypes.byref(h))
+    rc = _lib.load().mc3b_user_model_load_desc(cubin, len(cubin), _desc(nmodel, dtype, ninputs, nconst, nwork),
+                                               ctypes.byref(h))
     return h if rc == _lib.OK else rc
 
 
-def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1):
-    """Loaded module of (source, nmodel, dtype, ninputs): compiled once per process
+def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1, nconst=0, nwork=0):
+    """Loaded module of (source, nmodel, dtype, ninputs, nconst, nwork): compiled once per process
     (and taken from MC3B_JIT_CACHE when it is there).  stats, a dict, receives where
     the CUBIN came from ('memory', 'disk', 'nvrtc') and the seconds it took."""
-    key = cache_key(source, nmodel, dtype, ninputs)
+    key = cache_key(source, nmodel, dtype, ninputs, nconst, nwork)
     with _LOCK:
         h = _HANDLES.get(key)
         if h is not None:
@@ -155,10 +165,10 @@ def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1):
             with open(fpath, 'rb') as f:
                 cubin = f.read()
             origin = 'disk'
-        h = _load(cubin, nmodel, dtype, ninputs) if cubin is not None else None
+        h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork) if cubin is not None else None
         if not isinstance(h, ctypes.c_void_p):
             # not compiled yet, or a stale file that the loader refused: compile
-            cubin = compile_cubin(source, nmodel, dtype, name, ninputs)
+            cubin = compile_cubin(source, nmodel, dtype, name, ninputs, nconst, nwork)
             origin = 'nvrtc'
             if fpath:
                 os.makedirs(cdir, exist_ok=True)
@@ -166,7 +176,7 @@ def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1):
                 with open(tmp, 'wb') as f:
                     f.write(cubin)
                 os.replace(tmp, fpath)
-            h = _load(cubin, nmodel, dtype, ninputs)
+            h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork)
             if not isinstance(h, ctypes.c_void_p):
                 raise _lib.Mc3bError('mc3b_user_model_load failed: '
                                      + _lib.load().mc3b_last_error().decode('utf-8', 'replace'))

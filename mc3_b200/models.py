@@ -24,8 +24,13 @@ The reference's `func` is any Python callable `func(params, *indparams,
   consumes (with wlike=True it gets params[0:-3]), at most 32.  With ninputs=k the
   model takes k reals before the parameters, `model(real t, real xc, real yc, const
   real* p)` for k = 3, and the fit passes k arrays of the data's shape as indparams,
-  in the same order.  The source compiles on first use; a compile error raises
-  ValueError with the NVRTC log;
+  in the same order.  With nconst=m, the indparams after those arrays (numbers, 0-d
+  or 1-D arrays) are flattened in order into m run-time constants, p[nparams:nparams+m]
+  (their values are launch data, never part of the compiled module); nwork=w adds w
+  slots after them for an optional `__device__ void prepare(real* p)`, run once per
+  chain wherever the parameters are loaded, to hoist what depends on the chain alone
+  (1/sigma, 2 pi/P).  p holds [parameters | constants | work], at most 32 slots.  The
+  source compiles on first use; a compile error raises ValueError with the NVRTC log;
 * a TorchModel: a user torch callable evaluated ONCE per generation over the
   whole population, `fn(P[nchains, npars], *indparams) -> model[nchains, N]`
   on the device;
@@ -106,30 +111,46 @@ class CudaModel:
     """A user model written as a CUDA device function (see the module docstring):
     `__device__ real model(real x, const real* p)` in `source`, taking `nparams`
     parameters, or with ninputs = k > 1 inputs `model(real x1, ..., real xk, const
-    real* p)`.  Compiled lazily, once per process and dtype; pickles as its source
+    real* p)`.  With nconst = m, p[nparams:nparams+m] holds m run-time constants, and
+    nwork more slots follow for an optional `__device__ void prepare(real* p)` to fill
+    once per chain.  Compiled lazily, once per process and dtype; pickles as its source
     (one process per GPU receives it and compiles its own copy)."""
 
     ninputs = 1            # stored on the instance only when it is not 1
+    nconst = 0             # ... only when it is not 0
+    nwork = 0              # ... only when it is not 0
 
-    def __init__(self, source, nparams, name='cuda_model', ninputs=1):
+    def __init__(self, source, nparams, name='cuda_model', ninputs=1, nconst=0, nwork=0):
         nparams = int(nparams)
         if not 1 <= nparams <= _lib.MAX_PARS:
             raise ValueError(f'a CudaModel takes 1 to {_lib.MAX_PARS} parameters, got {nparams}')
         ninputs = int(ninputs)
         if not 1 <= ninputs <= _lib.MAX_INPUTS:
             raise ValueError(f'a CudaModel takes 1 to {_lib.MAX_INPUTS} inputs, got {ninputs}')
+        nconst, nwork = int(nconst), int(nwork)
+        if nconst < 0 or nwork < 0:
+            raise ValueError(f'nconst and nwork must not be negative, got {nconst} and {nwork}')
+        if nparams + nconst + nwork > _lib.MAX_PARS:
+            raise ValueError(f'nparams + nconst + nwork = {nparams} + {nconst} + {nwork} exceeds the '
+                             f'{_lib.MAX_PARS} slots of a model')
         self.source, self.nparams, self.name = str(source), nparams, str(name)
         if ninputs != 1:
             self.ninputs = ninputs
+        if nconst != 0:
+            self.nconst = nconst
+        if nwork != 0:
+            self.nwork = nwork
 
     def __getstate__(self):
         state = {'source': self.source, 'nparams': self.nparams, 'name': self.name}
-        if self.ninputs != 1:
-            state['ninputs'] = self.ninputs
+        for key in ('ninputs', 'nconst', 'nwork'):
+            if key in vars(self):
+                state[key] = vars(self)[key]
         return state
 
     def __setstate__(self, state):
-        self.__init__(state['source'], state['nparams'], state['name'], state.get('ninputs', 1))
+        self.__init__(state['source'], state['nparams'], state['name'], state.get('ninputs', 1),
+                      state.get('nconst', 0), state.get('nwork', 0))
 
     def nmodel(self, nfunc_params):
         """Number of leading parameters the model consumes."""
@@ -138,32 +159,53 @@ class CudaModel:
                 f'{self.name} takes {self.nparams} parameters, got {nfunc_params}')
         return self.nparams
 
+    def split_args(self, args):
+        """(per-point arrays, constants) of the arguments after the parameters: the first
+        ninputs are the arrays; with nconst or nwork set, the rest (numbers, 0-d and 1-D
+        arrays) are flattened in order into the constants, which must come to nconst
+        values.  A model of neither takes its arrays only (constants None)."""
+        if not (self.nconst or self.nwork):
+            return list(args), None
+        xs, rest = list(args[:self.ninputs]), args[self.ninputs:]
+        vals = [np.asarray(a, dtype=np.double) for a in rest]
+        if any(v.ndim > 1 for v in vals):
+            raise ValueError(f'{self.name}: constants are numbers or 1-D arrays, got shapes '
+                             f'{[v.shape for v in vals]}')
+        k = np.concatenate([v.ravel() for v in vals]) if vals else np.zeros(0)
+        if k.size != self.nconst:
+            raise ValueError(f'{self.name} takes {self.nconst} constant(s) after its {self.ninputs} input '
+                             f'array(s), got {k.size}')
+        return xs, k
+
     def cache_key(self, dtype=_lib.F64):
         from . import jit
-        return jit.cache_key(self.source, self.nparams, dtype, self.ninputs)
+        return jit.cache_key(self.source, self.nparams, dtype, self.ninputs, self.nconst, self.nwork)
 
     def handle(self, dtype=_lib.F64, stats=None):
         """mc3b_user_model_t* of this model for dtype (_lib.F64 / _lib.F32)."""
         from . import jit
-        return jit.handle(self.source, self.nparams, dtype, self.name, stats, self.ninputs)
+        return jit.handle(self.source, self.nparams, dtype, self.name, stats, self.ninputs, self.nconst,
+                          self.nwork)
 
-    def __call__(self, params, *xs):
+    def __call__(self, params, *args):
+        import torch
+        xs, k = self.split_args(args)
         if len(xs) != self.ninputs:
             raise ValueError(f'{self.name} takes {self.ninputs} input array(s), got {len(xs)}')
         self.nmodel(np.shape(np.atleast_2d(params))[1])
         h = self.handle(_lib.F64)
 
         def launch(dp, dxs, out):
-            if self.ninputs == 1:
-                _lib.call('mc3b_user_model_eval', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
-                          dxs[0].data_ptr(), dxs[0].numel(), out.data_ptr(), _lib.stream_ptr())
-            else:
-                _lib.call('mc3b_user_model_eval_inputs', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
-                          _lib.ptrs(dxs), len(dxs), dxs[0].numel(), out.data_ptr(), _lib.stream_ptr())
+            dk = None if k is None or k.size == 0 else torch.from_numpy(k).to(out.device)
+            _lib.call('mc3b_user_model_eval_consts', h, dp.data_ptr(), dp.shape[1], dp.shape[0],
+                      _lib.ptrs(dxs), len(dxs), _lib.ptr(dk), self.nconst, dxs[0].numel(), out.data_ptr(),
+                      _lib.stream_ptr())
         return _eval_rows(params, xs, launch)
 
     def __repr__(self):
         inputs = f', {self.ninputs} inputs' if self.ninputs != 1 else ''
+        inputs += f', {self.nconst} constants' if self.nconst else ''
+        inputs += f', {self.nwork} work slots' if self.nwork else ''
         return f'<mc3_b200 CUDA model {self.name} ({self.nparams} parameters{inputs})>'
 
 
