@@ -115,10 +115,13 @@ struct NoFix { __device__ __forceinline__ void operator()(bool, int64_t, double&
 // and with the decreasing split schedule it is also the shortest.  The other CTAs
 // publish their row with one fire-and-forget reduction (no round trip: an atomic
 // whose result every CTA waited for cost ~10 us per launch over the six waves) and
-// leave; the reducer spins until all nsplit-1 arrivals are in.
+// leave; the reducer spins until all nsplit-1 arrivals are in.  A one-split launch has no
+// arrivals to wait for.  own_row: the thread that owns a chain wrote that chain's only row,
+// and `row` is the value it wrote -- added from the register instead of read back.
 template <class Fix = NoFix>
 __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double* partial, int64_t ldpartial,
-                                                 int64_t nchains, int chains_per_cta, Fix fix = Fix()) {
+                                                 int64_t nchains, int chains_per_cta, Fix fix = Fix(),
+                                                 bool own_row = false, double row = 0.0) {
     __shared__ __align__(16) mc3b_sampler_t sS;
     __shared__ double vbuf[STAGE_DOUBLES];
     __syncthreads();                               // the CTA's partial row is written
@@ -132,11 +135,13 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
     }
     if (threadIdx.x == 0) {
         sS = f.S;                                  // constant bank -> shared, static offsets only
-        int seen;
-        do {
-            asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(f.done + blockIdx.x) : "memory");
-        } while (seen < others);
-        f.done[blockIdx.x] = 0;                    // every arrival is in: ready for the next launch
+        if (others > 0) {
+            int seen;
+            do {
+                asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(f.done + blockIdx.x) : "memory");
+            } while (seen < others);
+            f.done[blockIdx.x] = 0;                // every arrival is in: ready for the next launch
+        }
     }
     __syncthreads();
     if (threadIdx.x < 32) {                        // one warp stages the per-parameter vectors
@@ -170,7 +175,7 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
     bool inb = false;
     if (mine) {
         inb = sS.inb[f.c_off + cl] != 0;
-        if (inb) nxt = sum_partials<true>(partial, ldpartial, (int)gridDim.y, cl);
+        if (inb) nxt = own_row ? 0.0 + row : sum_partials<true>(partial, ldpartial, (int)gridDim.y, cl);
     }
     fix(inb, cl, nxt);
     if (mine) fused_metropolis_step(&sS, nxt, f.c_off + cl, gen, zrow0);

@@ -946,12 +946,28 @@ __global__ void __launch_bounds__(256) k_spectral_table(const double* __restrict
 // unguarded: a chain whose frequency (or twice it) falls outside the table gets NaN, which
 // MomentFix (fused epilogue or mc3b_moment_finish) sends to the point-by-point evaluation
 // together with the chains whose amplification is too large.
-__global__ void __launch_bounds__(WARPS * 32) k_spectral_chisq(ChisqArgs<double> a) {
+// What is constant during a run (the table's sums, the weight) is requested at entry, before the
+// chain's parameters arrive, together with an L2 prefetch of one 128-byte line of the table per
+// launched thread (the whole table at config 2's 4096 chains; only its first lines for small
+// populations).  The Horner sums are unrolled and the table loads written ahead of the first FMA.
+// Launched with WARPS * 32 threads.  The register cap (without it ptxas settles on 72 registers
+// and spills) holds the whole table row of a chain at K = 9 (31 complex values, 124 registers);
+// at K = 15 the row (49 complex values) does not fit and ptxas issues it in more than one batch.
+template <int K>
+__global__ void __maxnreg__(168) k_spectral_chisq(ChisqArgs<double> a) {
     asm volatile("griddepcontrol.launch_dependents;");   // the next proposal kernel may start its draws
+    const MomentArgs& m = a.m;
+    const double* h = m.spec;                       // n, St, St2, Sd, Std, D2
+    const double h0 = h[0], h1 = h[1], h2 = h[2], h3 = h[3], h4 = h[4], h5 = h[5];
+    const double w0 = a.w[0];
+    {
+        const int64_t bytes = 8 * (spec::HEAD + 2 * ((int64_t)m.sn1 * (2 * K + 3) + (int64_t)m.sn2 * (K + 1)));
+        const int64_t at = ((int64_t)blockIdx.x * (WARPS * 32) + threadIdx.x) * 128;
+        if (at < bytes) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(m.spec) + at));
+    }
     int64_t c = (int64_t)blockIdx.x * (WARPS * 32) + threadIdx.x;
     const bool live = c < a.nchains;
     if (!live) c = a.nchains - 1;
-    const MomentArgs& m = a.m;
     const double* p = a.params + c * a.ldp;
     const double amp = p[0], om = 6.283185307179586476925287 / p[1], ph = p[2];
     const double b = p[4] - m.slref;
@@ -959,22 +975,26 @@ __global__ void __launch_bounds__(WARPS * 32) k_spectral_chisq(ChisqArgs<double>
     const double j1 = rint((om - m.sw1) / m.sdelta), j2 = rint((2.0 * om - m.sw2) / m.sdelta);
     double q = __longlong_as_double(0x7ff8000000000000LL);
     if (j1 >= 0.0 && j1 < (double)m.sn1 && j2 >= 0.0 && j2 < (double)m.sn2) {
-        const int K = m.sorder;
         const double d1 = om - fma(j1, m.sdelta, m.sw1), d2 = fma(2.0, om, -fma(j2, m.sdelta, m.sw2));
         const double2* tab = reinterpret_cast<const double2*>(m.spec + spec::HEAD);
         const double2* T = tab + (int64_t)j1 * (2 * K + 3);
         const double2* U = tab + (int64_t)m.sn1 * (2 * K + 3) + (int64_t)j2 * (K + 1);
+        double2 t[K + 2], td[K + 1], u[K + 1];
+#pragma unroll
+        for (int k = 0; k < K + 2; k++) t[k] = T[k];
+#pragma unroll
+        for (int k = 0; k <= K; k++) { td[k] = T[K + 2 + k]; u[k] = U[k]; }
         // H = sum_k (i d1)^k [a T_1[k] + b (k+1) T_1[k+1] - T_d'[k]],  G = sum_k (i d2)^k U[k]
         double hr = 0.0, hi = 0.0, gr = 0.0, gi = 0.0;
+#pragma unroll
         for (int k = K; k >= 0; k--) {
-            const double2 t0 = T[k], t1 = T[k + 1], td = T[K + 2 + k], u = U[k];
             const double bk = b * (double)(k + 1);
-            const double cr = fma(ac, t0.x, fma(bk, t1.x, -td.x));
-            const double ci = fma(ac, t0.y, fma(bk, t1.y, -td.y));
+            const double cr = fma(ac, t[k].x, fma(bk, t[k + 1].x, -td[k].x));
+            const double ci = fma(ac, t[k].y, fma(bk, t[k + 1].y, -td[k].y));
             const double nr = fma(-d1, hi, cr);
             hi = fma(d1, hr, ci); hr = nr;
-            const double mr = fma(-d2, gi, u.x);
-            gi = fma(d2, gr, u.y); gr = mr;
+            const double mr = fma(-d2, gi, u[k].x);
+            gi = fma(d2, gr, u[k].y); gr = mr;
         }
         double sp, cp, s1, c1, s2, c2;
         sincos(ph, &sp, &cp);
@@ -985,21 +1005,20 @@ __global__ void __launch_bounds__(WARPS * 32) k_spectral_chisq(ChisqArgs<double>
         const double pr = (cp - sp) * (cp + sp), pi = 2.0 * sp * cp;              // e^{2 i ph}
         const double fr = fma(pr, c2, -pi * s2), fi = fma(pr, s2, pi * c2);      // ... e^{i d2 xc}
         const double re2 = fma(fr, gr, -fi * gi);
-        const double* h = m.spec;                   // n, St, St2, Sd, Std, D2
-        const double line = fma(ac, fma(h[0], ac, 2.0 * fma(b, h[1], -h[3])), fma(b, fma(b, h[2], -2.0 * h[4]), h[5]));
-        const double w0 = a.w[0];
-        q = fma(amp * amp, 0.5 * (h[0] - re2), fma(2.0 * amp, im1, line)) * (w0 * w0);
+        const double line = fma(ac, fma(h0, ac, 2.0 * fma(b, h1, -h3)), fma(b, fma(b, h2, -2.0 * h4), h5));
+        q = fma(amp * amp, 0.5 * (h0 - re2), fma(2.0 * amp, im1, line)) * (w0 * w0);
     }
     if (live) a.partial[c] = q;
 #ifndef MC3B_NO_FUSE_CODE
-    if (a.f.on) fused_metropolis(a.f, a.partial, a.ldpartial, a.nchains, WARPS * 32, MomentFix{a});
+    if (a.f.on) fused_metropolis(a.f, a.partial, a.ldpartial, a.nchains, WARPS * 32, MomentFix{a}, true, q);
 #endif
 }
 
 }  // namespace
 
 int mc3b_launch_spectral_chisq(const ChisqArgs<double>& a, unsigned groups, cudaStream_t st) {
-    k_spectral_chisq<<<groups, WARPS * 32, 0, st>>>(a);
+    if (a.m.sorder == 9) k_spectral_chisq<9><<<groups, WARPS * 32, 0, st>>>(a);
+    else k_spectral_chisq<15><<<groups, WARPS * 32, 0, st>>>(a);
     MC3B_CHECK_LAUNCH("k_spectral_chisq");
     return MC3B_OK;
 }

@@ -30,27 +30,31 @@ __global__ void __launch_bounds__(128) k_propose(mc3b_sampler_t S, mc3b_draws_t 
     const bool live = c < c_end;
     const bool devgen = gen < 0;                     // device-driven generation (graph mode)
     __shared__ double vbuf[STAGE_DOUBLES];
-    stage_vectors(S, vbuf);                          // constant during a run: safe before the wait
+    stage_vectors<128>(S, vbuf);                     // constant during a run: safe before the wait
     Draws dr;
-    double nrm[MAXP];
+    double nrm[PCHUNK];                              // support draws of the first chunk of free parameters
     int64_t gspec = gen;
     if (!REPLAY) {
         if (devgen) {
             gspec = *reinterpret_cast<volatile int64_t*>(S.gen_dev) + (pdl ? 1 : 0);
             zsize = S.M0 + (gspec / S.thinning) * S.nchains;
         }
-        if (live) chain_draws<false>(S, D, gspec, zsize, c, dr, nrm);
+        if (live) { chain_draws<false>(S, D, gspec, zsize, c, dr); chain_normals<false>(S, D, gspec, c, 0, nrm); }
     }
     if (pdl) asm volatile("griddepcontrol.wait;" ::: "memory");
     if (devgen) {
         gen = *reinterpret_cast<volatile int64_t*>(S.gen_dev);
         zsize = S.M0 + (gen / S.thinning) * S.nchains;
     }
-    if (REPLAY) { if (live) chain_draws<true>(S, D, gen, zsize, c, dr, nrm); }
-    else if (gen != gspec && live) chain_draws<false>(S, D, gen, zsize, c, dr, nrm);
+    if (REPLAY) {
+        if (live) { chain_draws<true>(S, D, gen, zsize, c, dr); chain_normals<true>(S, D, gen, c, 0, nrm); }
+    } else if (gen != gspec && live) {
+        chain_draws<false>(S, D, gen, zsize, c, dr);
+        chain_normals<false>(S, D, gen, c, 0, nrm);
+    }
     if (!REPLAY && S.F_peers) flags_wait(S, gen);    // every device has finished generation gen-1
     if (!live) return;
-    propose_apply(S, dr, nrm, gen, c);
+    propose_apply<REPLAY>(S, D, dr, nrm, gen, c);
 }
 
 __global__ void __launch_bounds__(128) k_metropolis(mc3b_sampler_t S, const double* partial, int64_t ldpartial, int nsplit,
@@ -58,7 +62,7 @@ __global__ void __launch_bounds__(128) k_metropolis(mc3b_sampler_t S, const doub
                                                     int64_t c_end) {
     const int64_t c = c_begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     __shared__ double vbuf[STAGE_DOUBLES];
-    stage_vectors(S, vbuf);
+    stage_vectors<128>(S, vbuf);
     if (c >= c_end) return;
     if (gen < 0) {                                   // device-driven generation (graph mode)
         gen = *S.gen_dev;

@@ -73,35 +73,67 @@ __device__ __forceinline__ void stage_peers_point(mc3b_sampler_t& S, double* buf
     if (S.Z_peers) S.Z_peers = reinterpret_cast<double* const*>(slot + MAXW);
     if (S.F_peers) S.F_peers = reinterpret_cast<int64_t* const*>(slot + 2 * MAXW);
 }
-__device__ __forceinline__ void stage_vectors(mc3b_sampler_t& S, double* buf) {
-    const int np = S.npars, nf = S.nfree;
-    const double* src[7] = {S.pstep, S.pmin, S.pmax, S.params0, S.prior, S.priorlow, S.priorup};
-    for (int i = threadIdx.x; i < 7 * np; i += blockDim.x) {
-        const int v = i / np, k = i - v * np;
-        if (src[v]) buf[v * MAXP + k] = src[v][k];
+// The CTA's share of the per-parameter vectors and of the free indices, NT threads: every
+// load is issued before the first shared-memory store (a store between two loads would hold
+// the second behind it, since the source is a generic pointer that may alias shared memory).
+__device__ __forceinline__ const double* stage_src(const mc3b_sampler_t& T, int v) {
+    return v == 0 ? T.pstep : v == 1 ? T.pmin : v == 2 ? T.pmax : v == 3 ? T.params0
+         : v == 4 ? T.prior : v == 5 ? T.priorlow : T.priorup;
+}
+template <int NT>
+__device__ __forceinline__ void stage_vectors_load(const mc3b_sampler_t& T, double* buf, int tid) {
+    constexpr int NV = (7 * MAXP + NT - 1) / NT, NI = (MAXP + NT - 1) / NT;
+    const int np = T.npars, nf = T.nfree;
+    double val[NV];
+    int32_t fr[NI];
+#pragma unroll
+    for (int r = 0; r < NV; r++) {
+        const int i = tid + r * NT, v = i / np, k = i - v * np;
+        const double* src = stage_src(T, v);
+        val[r] = i < 7 * np && src ? src[k] : 0.0;
+    }
+#pragma unroll
+    for (int r = 0; r < NI; r++) fr[r] = tid + r * NT < nf ? T.ifree[tid + r * NT] : 0;
+#pragma unroll
+    for (int r = 0; r < NV; r++) {
+        const int i = tid + r * NT, v = i / np, k = i - v * np;
+        if (i < 7 * np && stage_src(T, v)) buf[v * MAXP + k] = val[r];
     }
     int32_t* ifr = reinterpret_cast<int32_t*>(buf + 7 * MAXP);
-    for (int i = threadIdx.x; i < nf; i += blockDim.x) ifr[i] = S.ifree[i];
-    stage_peers_load(S, buf, threadIdx.x, blockDim.x);
+#pragma unroll
+    for (int r = 0; r < NI; r++)
+        if (tid + r * NT < nf) ifr[tid + r * NT] = fr[r];
+}
+// the whole CTA of NT = blockDim.x threads
+template <int NT>
+__device__ __forceinline__ void stage_vectors(mc3b_sampler_t& S, double* buf) {
+    stage_vectors_load<NT>(S, buf, threadIdx.x);
+    stage_peers_load(S, buf, threadIdx.x, NT);
     __syncthreads();
     S.pstep = buf; S.pmin = buf + MAXP; S.pmax = buf + 2 * MAXP; S.params0 = buf + 3 * MAXP;
     if (S.prior) { S.prior = buf + 4 * MAXP; S.priorlow = buf + 5 * MAXP; S.priorup = buf + 6 * MAXP; }
-    S.ifree = ifr;
+    S.ifree = reinterpret_cast<int32_t*>(buf + 7 * MAXP);
     stage_peers_point(S, buf);
 }
+
+// The proposal works on the free parameters in chunks of PCHUNK held in registers: the loads
+// of a chunk (the chain's row, the partner or snooker rows) are issued together, before any
+// store to nextp, and nothing of a chain's proposal lives in local memory.
+constexpr int PCHUNK = 2;
+static_assert(MAXP % PCHUNK == 0, "the parameter vectors are whole chunks");
 
 // The random numbers chain c consumes in generation gen (chain.py:185, 197-203,
 // 223-229, 257): a function of (seed, chain, generation) only -- not of the chains'
 // states, so a proposal kernel launched as a programmatic dependent of the previous
 // generation's model kernel draws them while that kernel is still running.
+// chain_draws: partner indices, snooker draws and u; chain_normals: the support draws of
+// the free parameters j0 .. j0 + PCHUNK - 1 (j0 a multiple of PCHUNK), scaled by pstep.
 template <bool REPLAY>
 __device__ __forceinline__ void chain_draws(const mc3b_sampler_t& S, const mc3b_draws_t& D, int64_t gen,
-                                            int64_t zsize, int64_t c, Draws& dr, double* nrm) {
-    const int nfree = S.nfree;
+                                            int64_t zsize, int64_t c, Draws& dr) {
     dr.iz = -1; dr.usj = 1.0; dr.gs = 0.0;
 
     if (REPLAY) {
-        for (int j = 0; j < nfree; j++) nrm[j] = D.normal[j];
         dr.a = dr.b = 0;
         if (S.sampler != MC3B_MRW) { dr.a = D.a[c]; dr.b = D.b[c]; }
         if (S.sampler == MC3B_SNOOKER) { dr.iz = D.iz[c]; dr.usj = D.usj[c]; dr.gs = D.gs[c]; }
@@ -128,83 +160,127 @@ __device__ __forceinline__ void chain_draws(const mc3b_sampler_t& S, const mc3b_
             dr.a = dr.b = 0;
         }
         dr.u = u01(w2.z, w2.w);
-        for (int j = 0; j < nfree; j += 2) {        // per-chain support draw
-            const uint4 w = ph(cid, 3u + (uint32_t)(j >> 1), g0, g1);
-            double n0, n1;
-            box_muller(u01(w.x, w.y), u01(w.z, w.w), n0, n1);
-            nrm[j] = n0 * S.pstep[S.ifree[j]];
-            if (j + 1 < nfree) nrm[j + 1] = n1 * S.pstep[S.ifree[j + 1]];
+    }
+}
+template <bool REPLAY>
+__device__ __forceinline__ void chain_normals(const mc3b_sampler_t& S, const mc3b_draws_t& D, int64_t gen, int64_t c,
+                                              int j0, double (&nrm)[PCHUNK]) {
+    const int nfree = S.nfree;
+    if (REPLAY) {
+#pragma unroll
+        for (int q = 0; q < PCHUNK; q++) nrm[q] = j0 + q < nfree ? D.normal[j0 + q] : 0.0;
+    } else {
+        const Philox ph(S.seed);
+        const uint32_t cid = (uint32_t)c, g0 = (uint32_t)gen, g1 = (uint32_t)((uint64_t)gen >> 32);
+#pragma unroll
+        for (int q = 0; q < PCHUNK; q += 2) {       // per-chain support draw
+            const int j = j0 + q;
+            nrm[q] = nrm[q + 1] = 0.0;
+            if (j < nfree) {
+                const uint4 w = ph(cid, 3u + (uint32_t)(j >> 1), g0, g1);
+                double n0, n1;
+                box_muller(u01(w.x, w.y), u01(w.z, w.w), n0, n1);
+                nrm[q] = n0 * S.pstep[S.ifree[j]];
+                if (j + 1 < nfree) nrm[q + 1] = n1 * S.pstep[S.ifree[j + 1]];
+            }
         }
     }
 }
 
 // Jump, bounds, shared parameters and the snooker factor from the draws and the
-// population as of the start of generation gen (chain.py:195-255).
-__device__ __forceinline__ void propose_apply(const mc3b_sampler_t& S, const Draws& dr, const double* nrm,
-                                              int64_t gen, int64_t c) {
+// population as of the start of generation gen (chain.py:195-255).  nrm0: the support
+// draws of the first chunk (chain_normals, j0 = 0); the later chunks draw their own.
+template <bool REPLAY>
+__device__ __forceinline__ void propose_apply(const mc3b_sampler_t& S, const mc3b_draws_t& D, const Draws& dr,
+                                              const double (&nrm0)[PCHUNK], int64_t gen, int64_t c) {
     const int nfree = S.nfree, npars = S.npars;
     // population as of the start of this generation (peer mode: half gen & 1)
     const double* Xg = S.X_peers ? S.X_peers[S.rank] + (gen & 1) * S.nchains * nfree : S.X;
     const double* x = Xg + c * nfree;
-    double jump[MAXP];
+    const bool snooker = S.sampler == MC3B_SNOOKER, demc = S.sampler == MC3B_DEMC;
+    // rows the jump takes its difference from: z1 - z2 (snooker), x1 - x2 (demc)
+    const double* r1 = snooker ? S.Z + dr.a * nfree : Xg + dr.a * nfree;
+    const double* r2 = snooker ? S.Z + dr.b * nfree : Xg + dr.b * nfree;
+    const bool sjump = snooker && dr.usj < 0.1;
+    const double* zrow = sjump ? S.Z + dr.iz * nfree : x;
 
-    double mrfactor = 1.0;
-    bool sjump = false;
-    const double* zrow = nullptr;
-    if (S.sampler == MC3B_SNOOKER) {
-        const double* z1 = S.Z + dr.a * nfree;
-        const double* z2 = S.Z + dr.b * nfree;
-        sjump = dr.usj < 0.1;
-        if (sjump) {                                 // chain.py:202-213
-            zrow = S.Z + dr.iz * nfree;
-            bool same = true;
-            for (int j = 0; j < nfree; j++) same = same && (zrow[j] == x[j]);
-            if (same) {
-                for (int j = 0; j < nfree; j++) jump[j] = __dmul_rn(dr.gs, __dsub_rn(z2[j], z1[j]));
-            } else {
-                double zp1 = 0.0, zp2 = 0.0, dd = 0.0;
-                for (int j = 0; j < nfree; j++) {
-                    const double dz = __dsub_rn(x[j], zrow[j]);
-                    zp1 = __dadd_rn(zp1, __dmul_rn(z1[j], dz));
-                    zp2 = __dadd_rn(zp2, __dmul_rn(z2[j], dz));
+    // snooker jump (chain.py:202-213): sums over every free parameter before the first jump
+    bool same = true;
+    double zp1 = 0.0, zp2 = 0.0, dd = 0.0;
+    if (sjump) {
+#pragma unroll 1
+        for (int j0 = 0; j0 < nfree; j0 += PCHUNK) {
+            double xv[PCHUNK], zv[PCHUNK], av[PCHUNK], bv[PCHUNK];
+#pragma unroll
+            for (int q = 0; q < PCHUNK; q++) {
+                const bool in = j0 + q < nfree;
+                xv[q] = in ? x[j0 + q] : 0.0; zv[q] = in ? zrow[j0 + q] : 0.0;
+                av[q] = in ? r1[j0 + q] : 0.0; bv[q] = in ? r2[j0 + q] : 0.0;
+            }
+#pragma unroll
+            for (int q = 0; q < PCHUNK; q++) {
+                if (j0 + q < nfree) {
+                    same = same && (zv[q] == xv[q]);
+                    const double dz = __dsub_rn(xv[q], zv[q]);
+                    zp1 = __dadd_rn(zp1, __dmul_rn(av[q], dz));
+                    zp2 = __dadd_rn(zp2, __dmul_rn(bv[q], dz));
                     dd = __dadd_rn(dd, __dmul_rn(dz, dz));
                 }
-                const double f = __dmul_rn(dr.gs, __dsub_rn(zp1, zp2));
-                for (int j = 0; j < nfree; j++)
-                    jump[j] = __ddiv_rn(__dmul_rn(f, __dsub_rn(x[j], zrow[j])), dd);
             }
-        } else {                                     // chain.py:214-217
-            for (int j = 0; j < nfree; j++)
-                jump[j] = __dadd_rn(__dmul_rn(S.gamma, __dsub_rn(z1[j], z2[j])), __dmul_rn(S.fepsilon, nrm[j]));
         }
-    } else if (S.sampler == MC3B_DEMC) {             // chain.py:230-232
-        const double* x1 = Xg + dr.a * nfree;
-        const double* x2 = Xg + dr.b * nfree;
-        for (int j = 0; j < nfree; j++)
-            jump[j] = __dadd_rn(__dmul_rn(S.gamma, __dsub_rn(x1[j], x2[j])), __dmul_rn(S.fepsilon, nrm[j]));
-    } else {                                         // mrw, chain.py:219-220
-        for (int j = 0; j < nfree; j++) jump[j] = nrm[j];
     }
+    const double f = __dmul_rn(dr.gs, __dsub_rn(zp1, zp2));
 
     // chain.py:235-247 -- propose, bounds, shared parameters
     double* np_ = S.nextp + c * npars;
-    for (int k = 0; k < npars; k++) np_[k] = S.params0[k];
     int inb = 1;
-    for (int j = 0; j < nfree; j++) {
-        const int k = S.ifree[j];
-        double v = __dadd_rn(x[j], jump[j]);
-        if (S.reflect) {                             // opt-in, non-reference behaviour
-            const double lo = S.pmin[k], hi = S.pmax[k];
-            for (int it = 0; it < 8 && (v < lo || v > hi); it++) v = v < lo ? 2.0 * lo - v : 2.0 * hi - v;
+#pragma unroll 1
+    for (int j0 = 0; j0 < nfree; j0 += PCHUNK) {
+        double xv[PCHUNK], av[PCHUNK], bv[PCHUNK], zv[PCHUNK], nrm[PCHUNK];
+#pragma unroll
+        for (int q = 0; q < PCHUNK; q++) {          // one batch of loads per chunk
+            const bool in = j0 + q < nfree;
+            xv[q] = in ? x[j0 + q] : 0.0;
+            av[q] = in && (snooker || demc) ? r1[j0 + q] : 0.0;
+            bv[q] = in && (snooker || demc) ? r2[j0 + q] : 0.0;
+            zv[q] = in && sjump ? zrow[j0 + q] : 0.0;
         }
-        np_[k] = v;
-        if (v < S.pmin[k] || v > S.pmax[k]) {
-            inb = 0;
-            atomicAdd(&S.outbounds[j], 1);
+        if (j0 == 0) {
+#pragma unroll
+            for (int q = 0; q < PCHUNK; q++) nrm[q] = nrm0[q];
+            for (int k = 0; k < npars; k++) np_[k] = S.params0[k];
+        } else {
+            chain_normals<REPLAY>(S, D, gen, c, j0, nrm);
+        }
+#pragma unroll
+        for (int q = 0; q < PCHUNK; q++) {
+            const int j = j0 + q;
+            if (j >= nfree) break;
+            double jump;
+            if (sjump) {
+                jump = same ? __dmul_rn(dr.gs, __dsub_rn(bv[q], av[q]))
+                            : __ddiv_rn(__dmul_rn(f, __dsub_rn(xv[q], zv[q])), dd);
+            } else if (snooker || demc) {           // chain.py:214-217, 230-232
+                jump = __dadd_rn(__dmul_rn(S.gamma, __dsub_rn(av[q], bv[q])), __dmul_rn(S.fepsilon, nrm[q]));
+            } else {                                // mrw, chain.py:219-220
+                jump = nrm[q];
+            }
+            const int k = S.ifree[j];
+            double v = __dadd_rn(xv[q], jump);
+            if (S.reflect) {                        // opt-in, non-reference behaviour
+                const double lo = S.pmin[k], hi = S.pmax[k];
+                for (int it = 0; it < 8 && (v < lo || v > hi); it++) v = v < lo ? 2.0 * lo - v : 2.0 * hi - v;
+            }
+            np_[k] = v;
+            if (v < S.pmin[k] || v > S.pmax[k]) {
+                inb = 0;
+                atomicAdd(&S.outbounds[j], 1);
+            }
         }
     }
     for (int k = 0; k < npars; k++)
         if (S.pstep[k] < 0.0) np_[k] = np_[-(int)S.pstep[k] - 1];
+    double mrfactor = 1.0;
     if (sjump && inb) {                              // chain.py:251-255
         double cn = 0.0, nn = 0.0;
         for (int j = 0; j < nfree; j++) {
@@ -224,9 +300,10 @@ template <bool REPLAY>
 __device__ __forceinline__ void propose_chain(const mc3b_sampler_t& S, const mc3b_draws_t& D, int64_t gen,
                                               int64_t zsize, int64_t c) {
     Draws dr;
-    double nrm[MAXP];
-    chain_draws<REPLAY>(S, D, gen, zsize, c, dr, nrm);
-    propose_apply(S, dr, nrm, gen, c);
+    double nrm[PCHUNK];
+    chain_draws<REPLAY>(S, D, gen, zsize, c, dr);
+    chain_normals<REPLAY>(S, D, gen, c, 0, nrm);
+    propose_apply<REPLAY>(S, D, dr, nrm, gen, c);
 }
 
 // Data chi-squared of a proposal: the partial rows of the model kernel added in
@@ -263,10 +340,20 @@ __device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double
     const bool peer = S.X_peers != nullptr;
     const int64_t half = S.nchains * nfree;
     double* x = peer ? S.X_peers[S.rank] + (gen & 1) * half + c * nfree : S.X + c * nfree;
-    double cur = S.chisq_cur[c];
-    bool accept = false;
     const double* np_ = S.nextp + c * npars;
-    if (S.inb[c]) {
+    // every per-chain value the step may need, loaded up front as one batch (behind the branches
+    // each was a round trip); the two rows go to L1 meanwhile without holding registers across the
+    // step (generic prefetch: no operation on a row in shared memory)
+    const int inb = S.inb[c];
+    double cur = S.chisq_cur[c];
+    const double mrf = S.mrfactor[c], u = S.u[c], best = S.best_chisq[c];
+    const int32_t nacc = S.naccept[c];
+    asm volatile("prefetch.L1 [%0];" ::"l"(np_));
+    asm volatile("prefetch.L1 [%0];" ::"l"(np_ + npars - 1));
+    asm volatile("prefetch.L1 [%0];" ::"l"(x));
+    asm volatile("prefetch.L1 [%0];" ::"l"(x + nfree - 1));
+    bool accept = false;
+    if (inb) {
         double nxt = nxt_data;
         if (S.prior != nullptr) {                    // stats.py:208-216 + stats.h:90-109
             double pr = 0.0;
@@ -280,13 +367,13 @@ __device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double
             }
             nxt += pr;
         }
-        const double ratio = exp(0.5 * (cur - nxt)) * S.mrfactor[c];
-        if (ratio > S.u[c]) {                        // chain.py:257-274 (NaN rejects)
+        const double ratio = exp(0.5 * (cur - nxt)) * mrf;
+        if (ratio > u) {                        // chain.py:257-274 (NaN rejects)
             accept = true;
             cur = nxt;
             S.chisq_cur[c] = nxt;
-            S.naccept[c] += 1;
-            if (nxt < S.best_chisq[c]) {
+            S.naccept[c] = nacc + 1;
+            if (nxt < best) {
                 S.best_chisq[c] = nxt;
                 S.best_gen[c] = gen;
                 for (int j = 0; j < nfree; j++) S.best_x[c * nfree + j] = np_[S.ifree[j]];
