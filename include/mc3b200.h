@@ -186,7 +186,19 @@ typedef struct mc3b_chisq_opts {
  *   guard_hits  device int32 counter or NULL
  *   spectral  [host] NULL: the tile kernels above.  Otherwise the spectral form below replaces
  *           them (folded, tiles and opts.work are then not read); its launches are planned
- *           with MC3B_PLAN_SPECTRAL (one split) and its rows are unguarded in the same way. */
+ *           with MC3B_PLAN_SPECTRAL (one split) and its rows are unguarded in the same way.
+ *   record  NULL, or (with guard_hits) the device address of MC3B_GUARD_RECORDS int64 slots of
+ *           page-locked, device-mapped host memory (mc3b_host_device_pointer).  A launch with
+ *           `fuse` then stores, from the thread that finishes last, after every hit of the
+ *           launch is counted, one aligned 64-bit record into slot g % MC3B_GUARD_RECORDS:
+ *           (g mod 2^32) << 32 | *guard_hits, g = the generations completed with this launch
+ *           (opts.gen + 1, or *fuse->gen_dev + 1 before its increment when opts.gen < 0).  The
+ *           host polls the slot until its high word is g mod 2^32 and reads the cumulative count
+ *           of generation g with no copy on the stream.  Fill the slots with a stamp no
+ *           generation of that slot has, e.g. slot s with stamp s + 1; a record stays until
+ *           generation g + MC3B_GUARD_RECORDS overwrites it.  Launches without `fuse` (and
+ *           mc3b_moment_finish) write none. */
+#define MC3B_GUARD_RECORDS 64
 struct mc3b_spectral;
 typedef struct mc3b_moment {
     const double* folded;
@@ -196,6 +208,7 @@ typedef struct mc3b_moment {
     int32_t* guard_hits;
     int32_t layout;     /* as given to mc3b_moment_prepare */
     const struct mc3b_spectral* spectral;
+    int64_t* record;
 } mc3b_moment_t;
 
 /* Spectral form of the same chi-squared: O(1) per chain instead of O(n).  With
@@ -529,6 +542,11 @@ int mc3b_peer_alloc(int64_t nbytes, void** ptr, unsigned char* handle64);
 int mc3b_peer_open(const unsigned char* handle64, void** ptr);
 int mc3b_peer_close(void* ptr);
 int mc3b_peer_free(void* ptr);
+
+/* Device address of page-locked host memory mapped into the current device's address
+ * space (cudaHostGetDevicePointer), e.g. for mc3b_moment_t.record; fails when `host` is
+ * not such memory.  *dev [host]. */
+int mc3b_host_device_pointer(void* host, void** dev);
 
 /* Report-point counters of this device's chains, packed for one D2H copy
  * (replaces the hub's reads of the shared numaccept / outbounds / bestp arrays,

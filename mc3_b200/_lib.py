@@ -15,6 +15,7 @@ MRW, DEMC, SNOOKER = 0, 1, 2
 SAMPLERS = {'mrw': MRW, 'demc': DEMC, 'snooker': SNOOKER}
 MAX_PARS = 32
 MAX_INPUTS = 4                    # MC3B_MAX_INPUTS: per-point inputs of a user model
+GUARD_RECORDS = 64                # MC3B_GUARD_RECORDS: slots of the moment form's guard record ring
 
 c_i64, c_i32, c_int = ctypes.c_int64, ctypes.c_int32, ctypes.c_int
 c_vp, c_dbl = ctypes.c_void_p, ctypes.c_double
@@ -53,7 +54,8 @@ class MomentStruct(ctypes.Structure):
     """mc3b_moment_t."""
     _fields_ = [('folded', c_vp), ('tiles', c_vp), ('c0ref', c_dbl), ('slref', c_dbl),
                 ('d2tot', c_dbl), ('amp_max', c_dbl), ('xlo', c_dbl), ('xhi', c_dbl),
-                ('guard_hits', c_vp), ('layout', c_i32), ('spectral', ctypes.POINTER(SpectralStruct))]
+                ('guard_hits', c_vp), ('layout', c_i32), ('spectral', ctypes.POINTER(SpectralStruct)),
+                ('record', c_vp)]
 
 
 class ChisqOpts(ctypes.Structure):
@@ -138,6 +140,7 @@ _SIGS = {
     'mc3b_peer_open': (c_int, [ctypes.c_char_p, ctypes.POINTER(c_vp)]),
     'mc3b_peer_close': (c_int, [c_vp]),
     'mc3b_peer_free': (c_int, [c_vp]),
+    'mc3b_host_device_pointer': (c_int, [c_vp, ctypes.POINTER(c_vp)]),
     'mc3b_pack_counters': (c_int, [ctypes.POINTER(SamplerStruct), c_vp, c_vp]),
     'mc3b_advance': (c_int, [ctypes.POINTER(SamplerStruct), c_vp]),
     'mc3b_run_small': (c_int, [ctypes.POINTER(SamplerStruct), c_int, c_int, c_vp, c_vp, c_vp,

@@ -105,6 +105,8 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
                     MC3B_CHECK_ARG(o.dx != 0.0 && o.ntiles >= 0 && o.ntiles * 128 <= n, "tile_x needs dx and ntiles <= n/128");
                     A.xt = o.tile_x; A.dxg = o.dx; A.ntiles = o.ntiles;
                 }
+                MC3B_CHECK_ARG(o.moment == nullptr || !o.moment->record || o.moment->guard_hits,
+                               "a guard record ring needs guard_hits");
                 if (usig && o.moment != nullptr && o.moment->spectral != nullptr) {
                     const mc3b_spectral_t& s = *o.moment->spectral;
                     MC3B_CHECK_ARG(s.table && (((uintptr_t)s.table) & 15) == 0 && s.n1 > 0 && s.n2 > 0 &&
@@ -112,7 +114,7 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
                                    "bad spectral table");
                     A.m.c0ref = o.moment->c0ref; A.m.slref = o.moment->slref; A.m.d2tot = o.moment->d2tot;
                     A.m.amp_max = o.moment->amp_max; A.m.guard_hits = o.moment->guard_hits;
-                    A.m.xlo = o.moment->xlo; A.m.xhi = o.moment->xhi;
+                    A.m.xlo = o.moment->xlo; A.m.xhi = o.moment->xhi; A.m.record = o.moment->record;
                     A.m.spec = s.table; A.m.sw1 = s.w1; A.m.sw2 = s.w2; A.m.sdelta = s.delta; A.m.sxc = s.xc;
                     A.m.sn1 = s.n1; A.m.sn2 = s.n2; A.m.sorder = s.order;
                     return mc3b_launch_spectral_chisq(A, (unsigned)groups, st);
@@ -126,6 +128,7 @@ int model_chisq_t(int model_id, const double* params, int64_t ldp, int64_t nchai
                     A.m.c0ref = o.moment->c0ref; A.m.slref = o.moment->slref; A.m.d2tot = o.moment->d2tot;
                     A.m.amp_max = o.moment->amp_max; A.m.guard_hits = o.moment->guard_hits;
                     A.m.xlo = o.moment->xlo; A.m.xhi = o.moment->xhi; A.m.layout = o.moment->layout;
+                    A.m.record = o.moment->record;
                     MC3B_CHECK_ARG(A.m.layout == 0 || A.m.layout == 1, "bad moment layout %d", A.m.layout);
                     return mc3b_launch_sinefold(A, (double*)o.work, (unsigned)groups, (unsigned)nsplit, st);
                 }

@@ -52,11 +52,14 @@ struct MomentArgs {
     double c0ref, slref, d2tot, amp_max;
     double xlo, xhi;                // range of the abscissa (bound of the line term of the guard)
     int32_t* guard_hits;
-    int layout;                     // of `folded`: 0 pairs interleaved (k_sinefold<MOM>), 1 mma fragments (k_sinemma)
     // spectral form (k_spectral_chisq, include/mc3b200.h mc3b_spectral_t): nullptr = the tile kernels
     const double* spec;             // sums, then the Taylor tables of both bands (mc3b_spectral_prepare)
     double sw1, sw2, sdelta, sxc;   // first node of the band and of the doubled band, node spacing, centre of x
     int sn1, sn2, sorder;           // nodes per band, Taylor order K
+    int layout;                     // of `folded`: 0 pairs interleaved (k_sinefold<MOM>), 1 mma fragments (k_sinemma)
+    int64_t* record;                // guard record ring (mc3b_moment_t.record) or nullptr
+    // (layout packed with the ints above: the record adds no bytes, so that every field after
+    // this block keeps its offset and the kernels without the moment form are unchanged)
 };
 
 template <typename T> struct ChisqArgs {
@@ -103,8 +106,14 @@ static __device__ __noinline__ void fused_metropolis_step(const mc3b_sampler_t* 
 }
 
 // Hook between the sum of a chain's partial rows and its Metropolis step; called by
-// every thread of the reducer CTA (it may use CTA barriers).
-struct NoFix { __device__ __forceinline__ void operator()(bool, int64_t, double&) const {} };
+// every thread of the reducer CTA (it may use CTA barriers).  recording(): the thread
+// whose arrival completes the launch calls record(g), g = generations completed, after
+// every group's hook has run.
+struct NoFix {
+    __device__ __forceinline__ void operator()(bool, int64_t, double&) const {}
+    __device__ __forceinline__ bool recording() const { return false; }
+    __device__ __forceinline__ void record(int64_t) const {}
+};
 
 // chains_per_cta: chains a CTA covers (its thread t < chains_per_cta owns chain
 // blockIdx.x * chains_per_cta + t of the launch).  `f` must be the kernel
@@ -180,16 +189,20 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
     fix(inb, cl, nxt);
     if (mine) fused_metropolis_step(&sS, nxt, f.c_off + cl, gen, zrow0);
     __syncthreads();
-    if (threadIdx.x == 0 && f.advance) {
+    const bool rec = fix.recording();              // false for NoFix: its code is unchanged
+    if (threadIdx.x == 0 && (f.advance || rec)) {
         // one fence for the CTA's stores (cumulative over the barrier): system scope when they
         // went to peer devices, so that the flag below needs no fence of its own
         if (sS.X_peers) __threadfence_system(); else __threadfence();
         if (atomicAdd(&f.done[gridDim.x], 1) == (int)gridDim.x - 1) {
             f.done[gridDim.x] = 0;
             __threadfence();
-            const int64_t g = *sS.gen_dev + 1;
-            *sS.gen_dev = g;
-            if (sS.F_peers) flags_publish(sS, g);    // every group's peer stores are performed
+            if (rec) fix.record(gen + 1);          // gen: read before any bump of gen_dev
+            if (!rec || f.advance) {
+                const int64_t g = *sS.gen_dev + 1;
+                *sS.gen_dev = g;
+                if (sS.F_peers) flags_publish(sS, g);    // every group's peer stores are performed
+            }
         }
     }
 }

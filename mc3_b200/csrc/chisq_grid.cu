@@ -376,6 +376,18 @@ struct MomentFix {
             }
         }
     }
+    // Guard record of the fused epilogue (include/mc3b200.h mc3b_moment_t.record): the host reads
+    // the count of generation g without a copy on the stream.  Called after the fence that
+    // follows every group's arrival, so every hit of the launch (each counted before its CTA's
+    // barrier and fence) is in; one aligned 64-bit store, stamp in the high word.
+    __device__ __forceinline__ bool recording() const { return a.m.record != nullptr; }
+    __device__ __forceinline__ void record(int64_t g) const {
+        int hits;
+        asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(hits) : "l"(a.m.guard_hits) : "memory");
+        const unsigned long long v = ((unsigned long long)(uint32_t)g << 32) | (uint32_t)hits;
+        asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(a.m.record + (g & (MC3B_GUARD_RECORDS - 1))), "l"(v)
+                     : "memory");
+    }
 };
 
 #ifndef MC3B_FOLD_MINB

@@ -65,6 +65,12 @@ extern "C" int mc3b_peer_free(void* ptr) {
     return MC3B_OK;
 }
 
+extern "C" int mc3b_host_device_pointer(void* host, void** dev) {
+    MC3B_CHECK_ARG(host && dev, "bad arguments");
+    MC3B_CUDA(cudaHostGetDevicePointer(dev, host, 0));
+    return MC3B_OK;
+}
+
 // Roofline denominator: 8 independent accumulators per thread, each a chain of
 // dependent FMAs; 256 threads x 8 CTAs per SM keeps the pipe full.
 namespace {

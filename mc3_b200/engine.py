@@ -72,6 +72,67 @@ def on_device(fn):
 _DT = {'f64': _lib.F64, 'f32': _lib.F32, np.float64: _lib.F64, np.float32: _lib.F32}
 
 
+class GuardRecords:
+    """Host side of the moment form's guard records (include/mc3b200.h mc3b_moment_t.record).
+    `ring` is the int64 view of R page-locked slots the fused epilogue writes: slot g % R holds
+    (g mod 2^32) << 32 | guard hits counted up to the end of generation g.  Hits counted outside
+    generations (mc3b_moment_finish in chisq() and init_population) enter the next record.
+
+    The rule (step) is a function of generation boundaries only: at the start of a run() call,
+    the record of G* = the generation count at the start of the call before the previous one is
+    read, G* clamped to >= gen - R + 1 so that its slot cannot have been overwritten (the device
+    is never ahead of what the host has enqueued).  The form is left when the hits since the last
+    record read exceed 1e-3 per chain-step.  The record has normally long arrived; until it has,
+    the host polls its slot."""
+    R = _lib.GUARD_RECORDS
+
+    def __init__(self, ring):
+        self.ring = ring
+        # slot s only ever holds generations g = s (mod R), and R divides 2^32: stamp s + 1 is none of them
+        ring[:] = ((np.arange(self.R, dtype=np.int64) + 1) % self.R) << 32
+        self.starts = []        # generation counts at the start of the last calls whose record exists
+        self.seen = (0, 0)      # (generation, hits) of the last record read
+        self.end = None         # generation count at the end of the last recording call
+
+    def read(self, g):
+        """Hits of record g, or None while slot g % R holds another generation's stamp."""
+        v = int(self.ring[g % self.R])
+        return v & 0xffffffff if (v >> 32) & 0xffffffff == g & 0xffffffff else None
+
+    def wait(self, g, idle):
+        """Poll record g; idle() tells whether the stream has finished all enqueued work."""
+        while True:
+            h = self.read(g)
+            if h is not None:
+                return h
+            if idle():
+                h = self.read(g)
+                if h is None:
+                    raise _lib.Mc3bError(f'guard record of generation {g} missing with the stream idle '
+                                         f'(slot holds {int(self.ring[g % self.R]):#x})')
+                return h
+
+    def step(self, gen, ngen, nlocal, recording, idle):
+        """At the start of a run() call from generation count `gen` over `ngen` generations;
+        recording: they run the fused moment kernel.  True: leave the moment form."""
+        if not recording:
+            self.starts = []        # the generations of this call leave no records
+            return False
+        while len(self.starts) >= 2:
+            g = max(self.starts.pop(0), gen - self.R + 1)
+            g0, h0 = self.seen
+            if g <= g0:
+                continue
+            hits = self.wait(g, idle)
+            if (hits - h0) & 0xffffffff > 1e-3*nlocal*(g - g0):
+                return True
+            self.seen = (g, hits)
+        if self.end == gen:         # the record of generation `gen` exists
+            self.starts.append(gen)
+        self.end = gen + ngen
+        return False
+
+
 class Population:
     def __init__(self, data, uncert, func, params, indparams=(), indparams_dict=None,
                  pstep=None, pmin=None, pmax=None, prior=None, priorlow=None,
@@ -302,13 +363,16 @@ class Population:
                     self.spectral = S
                     self.spectral_plan = plan
                     M.spectral = ctypes.pointer(S)
+                # the guard count of every generation, written by the fused epilogue into
+                # page-locked host memory (include/mc3b200.h mc3b_moment_t.record)
+                with torch.cuda.device(self.dev):
+                    self._guard_ring = torch.empty(_lib.GUARD_RECORDS, dtype=torch.int64).pin_memory()
+                    dptr = ctypes.c_void_p()
+                    _lib.call('mc3b_host_device_pointer', self._guard_ring.data_ptr(), ctypes.byref(dptr))
+                M.record = dptr.value
+                self._guard = GuardRecords(self._guard_ring.numpy())
                 self.moment = M
                 self.use_moment = True
-                self._guard_log = []          # (generation, ring slot) per run() call, oldest first
-                self._guard_seen = (0, 0)     # (generation, hits) of the last record evaluated
-                self._guard_pin = torch.zeros(4, dtype=torch.int32).pin_memory()
-                self._guard_ev = [torch.cuda.Event() for _ in range(4)]
-                self._guard_n = 0
             if self.dtype == _lib.F32:
                 self.k_x, self.k_d, self.k_w = (t.float().contiguous() for t in
                                                 (self.d_x, self.d_data, self.d_invsig))
@@ -826,8 +890,6 @@ class Population:
         block of generations."""
         if ngen <= 0:
             return
-        if getattr(self, 'use_moment', False):
-            self._moment_policy()
         if use_graph is None:
             # A generation with >= ~0.3 ms of device work hides its three host
             # launches completely: skip the capture (10-15 ms) and run eagerly.
@@ -837,6 +899,10 @@ class Population:
             use_graph = self.kind in ('builtin', 'cuda') and not heavy and not \
                 (self.world > 1 and self.shard == 'chains' and self.sampler == 'snooker'
                  and self.p2p is None)
+        if getattr(self, 'use_moment', False):
+            # the persistent small-population kernel never runs the moment form, and
+            # unfused generations write no guard records
+            self._moment_policy(ngen, self.fused and not (use_graph and self.small))
         if use_graph and self.small:
             # launch-latency-bound population: all generations inside one resident CTA
             done = 0
@@ -885,38 +951,26 @@ class Population:
         self.launches += ngen*self._graph_launches
         self.gen += ngen
 
-    def _moment_policy(self):
-        """Decide, at the start of a run() call, whether the generation loop keeps the
-        sufficient-statistics kernel.  Deterministic: the decision at this call uses the
-        guard count recorded at the end of the call before the previous one (its copy has
-        long landed, so the host does not stall), i.e. it depends on generation
-        boundaries, not on timing.  Before the first generation the amplification is
-        estimated from the best chi-squared of the initial population."""
+    def _moment_policy(self, ngen, recording):
+        """Decide, at the start of a run() call of `ngen` generations, whether the
+        generation loop keeps the sufficient-statistics kernel.  Before the first
+        generation the amplification is estimated from the best chi-squared of the
+        initial population; after that the guard records decide (GuardRecords.step).
+        recording: this call's generations run the fused moment kernel."""
         M = self.moment
-        if self.gen == 0 and not self._guard_log and np.isfinite(self.best_log_post0):
+        if self.gen == 0 and np.isfinite(self.best_log_post0):
             n, w0 = self.ndata, 1.0/float(self.host_uncert0)
             mag = abs(float(self.bestp0[0]))*np.sqrt(n) + np.sqrt(M.d2tot)
             if mag*mag*w0*w0 > 0.5*M.amp_max*max(-2.0*self.best_log_post0, 1e-300):
                 self._moment_off()
                 return
-        while len(self._guard_log) >= 2:
-            gen, slot = self._guard_log.pop(0)
-            self._guard_ev[slot].synchronize()
-            g0, h0 = self._guard_seen
-            hits = int(self._guard_pin[slot])
-            if gen > g0 and (hits - h0) > 1e-3*self.nlocal*(gen - g0):
-                self._moment_off()
-                return
-            self._guard_seen = (gen, hits)
-        slot = self._guard_n % 4
-        self._guard_n += 1
-        self._guard_pin[slot:slot + 1].copy_(self.guard_hits, non_blocking=True)
-        self._guard_ev[slot].record()
-        self._guard_log.append((self.gen, slot))
+        idle = torch.cuda.current_stream(self.dev).query
+        if self._guard.step(self.gen, ngen, self.nlocal, recording, idle):
+            self._moment_off()
 
     def _moment_off(self):
         self.use_moment = False
-        self._guard_log = []
+        self._guard.starts = []
         self._graph = None
         self._block_graph = None
 

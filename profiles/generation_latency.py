@@ -9,7 +9,9 @@ launch overhead is not charged to the device time):
   graph_replay      pop._graph.replay(): one captured generation
   propose           mc3b_propose alone, device-driven as in the graph
   chisq_fused       pop.data_chisq(P, fuse=...): the chi-squared kernel + fused Metropolis epilogue
-  guard_snapshot    the 4-byte device-to-host copy _moment_policy puts in every run() call
+  graph_replay_no_record   graph_replay of a generation captured without the guard record ring
+                    (mc3b_moment_t.record = NULL): the cost of the record's store.  Timed in the
+                    order with, without, without, with (the _2 entries)
 
     python profiles/generation_latency.py [--out FILE] [--label NAME]
 
@@ -68,7 +70,7 @@ def main():
     pop = Population(w['data'], w['uncert'], mc3.models.BUILTIN[w['model']], w['params'], [w['x']], {},
                      w['pstep'], w['pmin'], w['pmax'], w['prior'], w['priorlow'], w['priorup'],
                      nchains=4096, sampler=w['sampler'], fepsilon=w['fepsilon'], thinning=1,
-                     nzchain=4*K + 64, seed=1234)
+                     nzchain=10*K + 64, seed=1234)
     pop.init_population('normal')
     pop.run(3, use_graph=True)                   # warm-up (captures the generation graph)
     torch.cuda.synchronize()
@@ -95,17 +97,22 @@ def main():
     def chisq_fused():
         pop.data_chisq(P, fuse=(c0, pop.gen, -1, False))
 
-    def guard_snapshot():
-        pop._guard_pin[0:1].copy_(pop.guard_hits, non_blocking=True)
-
     res = {'spectral': pop.spectral is not None, 'use_moment': bool(getattr(pop, 'use_moment', False))}
     res['step'] = measure(pop, step, flush, spin)
     pop.gen_dev.fill_(pop.gen)
+    ring = pop.moment.record
+    pop.moment.record = None
+    plain, _ = pop._capture(1)
+    pop.moment.record = ring
+    # A B B A: with and without the record store, alternated against drift
     res['graph_replay'] = measure(pop, replay, flush, spin)
+    res['graph_replay_no_record'] = measure(pop, plain.replay, flush, spin)
+    res['graph_replay_no_record_2'] = measure(pop, plain.replay, flush, spin)
+    res['graph_replay_2'] = measure(pop, replay, flush, spin)
+    del plain
     res['propose'] = measure(pop, propose, flush, spin)
     res['chisq_fused'] = measure(pop, chisq_fused, flush, spin)
-    res['guard_snapshot'] = measure(pop, guard_snapshot, flush, spin)
-    pop.gen += 2*K
+    pop.gen += 8*K                               # the four graph_replay items, flushed and warm
     pop.gen_dev.fill_(pop.gen)
     torch.cuda.synchronize()
     res['gpu'] = gpu_info()
