@@ -115,6 +115,31 @@ struct NoFix {
     __device__ __forceinline__ void record(int64_t) const {}
 };
 
+// After every thread's step: the CTA counts its arrival, and the thread whose arrival completes
+// the launch records and bumps the generation counter.  gdev: *S.gen_dev as read earlier in the
+// launch (whenever f.advance is set); nothing else writes it while the launch runs.
+template <class Fix>
+__device__ __forceinline__ void fused_metropolis_end(const FuseArgs& f, const mc3b_sampler_t& S, const Fix& fix,
+                                                     int64_t gen, int64_t gdev) {
+    __syncthreads();
+    const bool rec = fix.recording();              // false for NoFix: its code is unchanged
+    if (threadIdx.x == 0 && (f.advance || rec)) {
+        // one fence for the CTA's stores (cumulative over the barrier): system scope when they
+        // went to peer devices, so that the flag below needs no fence of its own
+        if (S.X_peers) __threadfence_system(); else __threadfence();
+        if (atomicAdd(&f.done[gridDim.x], 1) == (int)gridDim.x - 1) {
+            f.done[gridDim.x] = 0;
+            __threadfence();
+            if (rec) fix.record(gen + 1);
+            if (f.advance) {
+                const int64_t g = gdev + 1;
+                *S.gen_dev = g;
+                if (S.F_peers) flags_publish(S, g);      // every group's peer stores are performed
+            }
+        }
+    }
+}
+
 // chains_per_cta: chains a CTA covers (its thread t < chains_per_cta owns chain
 // blockIdx.x * chains_per_cta + t of the launch).  `f` must be the kernel
 // parameter itself (read from the constant bank, never copied to the stack).
@@ -125,12 +150,10 @@ struct NoFix {
 // publish their row with one fire-and-forget reduction (no round trip: an atomic
 // whose result every CTA waited for cost ~10 us per launch over the six waves) and
 // leave; the reducer spins until all nsplit-1 arrivals are in.  A one-split launch has no
-// arrivals to wait for.  own_row: the thread that owns a chain wrote that chain's only row,
-// and `row` is the value it wrote -- added from the register instead of read back.
+// arrivals to wait for.
 template <class Fix = NoFix>
 __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double* partial, int64_t ldpartial,
-                                                 int64_t nchains, int chains_per_cta, Fix fix = Fix(),
-                                                 bool own_row = false, double row = 0.0) {
+                                                 int64_t nchains, int chains_per_cta, Fix fix = Fix()) {
     __shared__ __align__(16) mc3b_sampler_t sS;
     __shared__ double vbuf[STAGE_DOUBLES];
     __syncthreads();                               // the CTA's partial row is written
@@ -175,36 +198,60 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
     __syncthreads();
     const int64_t cl = (int64_t)blockIdx.x * chains_per_cta + threadIdx.x;
     const bool mine = (int)threadIdx.x < chains_per_cta && cl < nchains;
+    const int64_t gdev = f.gen < 0 || f.advance ? *sS.gen_dev : 0;
     int64_t gen = f.gen, zrow0 = f.zrow0;
     if (gen < 0) {
-        gen = *sS.gen_dev;
+        gen = gdev;
         zrow0 = ((gen + 1) % sS.thinning == 0) ? sS.M0 + ((gen + 1) / sS.thinning - 1) * sS.nchains : -1;
     }
     double nxt = 0.0;
     bool inb = false;
     if (mine) {
         inb = sS.inb[f.c_off + cl] != 0;
-        if (inb) nxt = own_row ? 0.0 + row : sum_partials<true>(partial, ldpartial, (int)gridDim.y, cl);
+        if (inb) nxt = sum_partials<true>(partial, ldpartial, (int)gridDim.y, cl);
     }
     fix(inb, cl, nxt);
     if (mine) fused_metropolis_step(&sS, nxt, f.c_off + cl, gen, zrow0);
-    __syncthreads();
-    const bool rec = fix.recording();              // false for NoFix: its code is unchanged
-    if (threadIdx.x == 0 && (f.advance || rec)) {
-        // one fence for the CTA's stores (cumulative over the barrier): system scope when they
-        // went to peer devices, so that the flag below needs no fence of its own
-        if (sS.X_peers) __threadfence_system(); else __threadfence();
-        if (atomicAdd(&f.done[gridDim.x], 1) == (int)gridDim.x - 1) {
-            f.done[gridDim.x] = 0;
-            __threadfence();
-            if (rec) fix.record(gen + 1);          // gen: read before any bump of gen_dev
-            if (!rec || f.advance) {
-                const int64_t g = *sS.gen_dev + 1;
-                *sS.gen_dev = g;
-                if (sS.F_peers) flags_publish(sS, g);    // every group's peer stores are performed
-            }
-        }
-    }
+    fused_metropolis_end(f, sS, fix, gen, gdev);
+}
+
+// The one-split launch of k_spectral_chisq, whose thread t of CTA b owns chain b * WARPS * 32 + t,
+// in two parts.  fused_metropolis_load runs at kernel entry: each thread reads the generation
+// counter and its chain's state (metropolis_load), and the CTA stages the per-parameter vectors,
+// every load issued before the first shared-memory store.  None of it depends on the chain's
+// chi-squared and no other thread writes it during the launch, so these loads overlap the
+// chi-squared instead of following it one round trip after another.
+struct FusedEntry {
+    int64_t gen;                    // generation of the step (f.gen, or *gen_dev when device-driven)
+    int64_t gdev;                   // *gen_dev when the launch bumps it or is device-driven
+    ChainState st;
+};
+__device__ __forceinline__ FusedEntry fused_metropolis_load(const FuseArgs& f, double* vbuf, int64_t cl) {
+    FusedEntry e;
+    e.gdev = f.gen < 0 || f.advance ? *f.S.gen_dev : 0;
+    e.gen = f.gen < 0 ? e.gdev : f.gen;
+    e.st = metropolis_load(f.S, e.gen, f.c_off + cl);
+    stage_vectors_load<WARPS * 32>(f.S, vbuf, threadIdx.x);
+    stage_peers_load(f.S, vbuf, threadIdx.x, WARPS * 32);
+    return e;
+}
+// Every thread of the CTA, after its partial row is written: guard(act, nxt) is the Fix hook
+// (a CTA-wide call) with the chain's inputs already in registers; mine: the thread owns a chain,
+// whose only row is `row`, added from the register (0.0 + row: the bits of the split-order sum).
+template <class Fix, class Guard>
+__device__ __forceinline__ void fused_metropolis_apply(const FuseArgs& f, const FusedEntry& e, double* vbuf, int64_t cl,
+                                                       bool mine, double row, const Fix& fix, Guard guard) {
+    __syncthreads();                               // the staged vectors are in
+    mc3b_sampler_t S = f.S;
+    stage_point(S, vbuf);
+    const int64_t gen = e.gen;
+    int64_t zrow0 = f.zrow0;
+    if (f.gen < 0) zrow0 = ((gen + 1) % S.thinning == 0) ? S.M0 + ((gen + 1) / S.thinning - 1) * S.nchains : -1;
+    const bool inb = mine && e.st.inb != 0;
+    double nxt = inb ? 0.0 + row : 0.0;
+    guard(inb, nxt);
+    if (mine) metropolis_apply(S, e.st, nxt, gen, zrow0, f.c_off + cl);
+    fused_metropolis_end(f, S, fix, gen, e.gdev);
 }
 
 #ifndef __CUDACC_RTC__

@@ -328,16 +328,23 @@ struct MomentFix {
     const ChisqArgs<double>& a;
     // `act`: this thread owns a chain whose proposal is inside the bounds; nxt = its data chi-squared
     __device__ __forceinline__ void operator()(bool act, int64_t cl, double& nxt) const {
-        const MomentArgs& m = a.m;
-        const double w0 = a.w[0];
-        bool bad = false;
         const double* p = a.params + cl * a.ldp;
+        double pa = 0.0, pc = 0.0, ps = 0.0;
+        if (act) { pa = p[0]; pc = p[3]; ps = p[4]; }
+        guard(act, p, pa, pc, ps, a.w[0], nxt);
+    }
+    // the same with the chain's amplitude, intercept and slope (p[0], p[3], p[4]; read when act)
+    // and the weight w0 in registers
+    __device__ __forceinline__ void guard(bool act, const double* p, double pa, double pc, double ps, double w0,
+                                          double& nxt) const {
+        const MomentArgs& m = a.m;
+        bool bad = false;
         if (act) {
             // |L'| <= sqrt(n) max(|L'(xlo)|, |L'(xhi)|): a line is extremal at the ends of its range
             const double n = (double)a.n;
-            const double c0 = p[3] - m.c0ref, sl = p[4] - m.slref;
+            const double c0 = pc - m.c0ref, sl = ps - m.slref;
             const double lmax = fmax(fabs(fma(sl, m.xlo, c0)), fabs(fma(sl, m.xhi, c0)));
-            const double mag = (fabs(p[0]) + lmax) * sqrt(n) + sqrt(m.d2tot);
+            const double mag = (fabs(pa) + lmax) * sqrt(n) + sqrt(m.d2tot);
             bad = !(mag * mag * (w0 * w0) <= m.amp_max * nxt);        // NaN: exact path too
         }
         if (!__syncthreads_or(bad)) return;
@@ -981,9 +988,14 @@ __global__ void __maxnreg__(168) k_spectral_chisq(ChisqArgs<double> a) {
     const bool live = c < a.nchains;
     if (!live) c = a.nchains - 1;
     const double* p = a.params + c * a.ldp;
-    const double amp = p[0], om = 6.283185307179586476925287 / p[1], ph = p[2];
-    const double b = p[4] - m.slref;
-    const double ac = fma(b, m.sxc, p[3] - m.c0ref);           // L' at the centre
+    const double amp = p[0], om = 6.283185307179586476925287 / p[1], ph = p[2], p3 = p[3], p4 = p[4];
+#ifndef MC3B_NO_FUSE_CODE
+    __shared__ double vbuf[STAGE_DOUBLES];
+    FusedEntry fe;
+    if (a.f.on) fe = fused_metropolis_load(a.f, vbuf, c);
+#endif
+    const double b = p4 - m.slref;
+    const double ac = fma(b, m.sxc, p3 - m.c0ref);             // L' at the centre
     const double j1 = rint((om - m.sw1) / m.sdelta), j2 = rint((2.0 * om - m.sw2) / m.sdelta);
     double q = __longlong_as_double(0x7ff8000000000000LL);
     if (j1 >= 0.0 && j1 < (double)m.sn1 && j2 >= 0.0 && j2 < (double)m.sn2) {
@@ -1022,7 +1034,11 @@ __global__ void __maxnreg__(168) k_spectral_chisq(ChisqArgs<double> a) {
     }
     if (live) a.partial[c] = q;
 #ifndef MC3B_NO_FUSE_CODE
-    if (a.f.on) fused_metropolis(a.f, a.partial, a.ldpartial, a.nchains, WARPS * 32, MomentFix{a}, true, q);
+    if (a.f.on) {
+        const MomentFix fix{a};
+        fused_metropolis_apply(a.f, fe, vbuf, c, live, q, fix,
+                               [&](bool act, double& nxt) { fix.guard(act, p, amp, p3, p4, w0, nxt); });
+    }
 #endif
 }
 

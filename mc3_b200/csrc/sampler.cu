@@ -29,6 +29,21 @@ __global__ void __launch_bounds__(128) k_propose(mc3b_sampler_t S, mc3b_draws_t 
     const int64_t c = c_begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = c < c_end;
     const bool devgen = gen < 0;                     // device-driven generation (graph mode)
+    // the counter is requested with the staging loads, not one round trip after them
+    const int64_t g0 = devgen ? *reinterpret_cast<volatile int64_t*>(S.gen_dev) : gen;
+    // Without PDL or peers the population is final at entry: the chain's own row is requested now,
+    // and every thread sends one 128-byte line of the population to L2 (all of it at config 2's
+    // 4096 chains), where the partner rows, known only once the draws are taken, then hit.  (Not in
+    // replay mode, a check against the reference's draws: there it would spill.)
+    const bool early = !REPLAY && !pdl && S.X_peers == nullptr;
+    double xv0[PCHUNK];
+    if (early) {
+        const int64_t at = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 128;
+        if (at < S.nchains * S.nfree * 8)
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(S.X) + at));
+#pragma unroll
+        for (int q = 0; q < PCHUNK; q++) xv0[q] = live && q < S.nfree ? S.X[c * S.nfree + q] : 0.0;
+    }
     __shared__ double vbuf[STAGE_DOUBLES];
     stage_vectors<128>(S, vbuf);                     // constant during a run: safe before the wait
     Draws dr;
@@ -36,14 +51,14 @@ __global__ void __launch_bounds__(128) k_propose(mc3b_sampler_t S, mc3b_draws_t 
     int64_t gspec = gen;
     if (!REPLAY) {
         if (devgen) {
-            gspec = *reinterpret_cast<volatile int64_t*>(S.gen_dev) + (pdl ? 1 : 0);
+            gspec = g0 + (pdl ? 1 : 0);
             zsize = S.M0 + (gspec / S.thinning) * S.nchains;
         }
         if (live) { chain_draws<false>(S, D, gspec, zsize, c, dr); chain_normals<false>(S, D, gspec, c, 0, nrm); }
     }
     if (pdl) asm volatile("griddepcontrol.wait;" ::: "memory");
     if (devgen) {
-        gen = *reinterpret_cast<volatile int64_t*>(S.gen_dev);
+        gen = pdl ? *reinterpret_cast<volatile int64_t*>(S.gen_dev) : g0;
         zsize = S.M0 + (gen / S.thinning) * S.nchains;
     }
     if (REPLAY) {
@@ -54,7 +69,7 @@ __global__ void __launch_bounds__(128) k_propose(mc3b_sampler_t S, mc3b_draws_t 
     }
     if (!REPLAY && S.F_peers) flags_wait(S, gen);    // every device has finished generation gen-1
     if (!live) return;
-    propose_apply<REPLAY>(S, D, dr, nrm, gen, c);
+    propose_apply<REPLAY>(S, D, dr, nrm, gen, c, early, xv0);
 }
 
 __global__ void __launch_bounds__(128) k_metropolis(mc3b_sampler_t S, const double* partial, int64_t ldpartial, int nsplit,

@@ -104,16 +104,20 @@ __device__ __forceinline__ void stage_vectors_load(const mc3b_sampler_t& T, doub
     for (int r = 0; r < NI; r++)
         if (tid + r * NT < nf) ifr[tid + r * NT] = fr[r];
 }
+// S repointed to the staged copies (after a CTA barrier)
+__device__ __forceinline__ void stage_point(mc3b_sampler_t& S, double* buf) {
+    S.pstep = buf; S.pmin = buf + MAXP; S.pmax = buf + 2 * MAXP; S.params0 = buf + 3 * MAXP;
+    if (S.prior) { S.prior = buf + 4 * MAXP; S.priorlow = buf + 5 * MAXP; S.priorup = buf + 6 * MAXP; }
+    S.ifree = reinterpret_cast<int32_t*>(buf + 7 * MAXP);
+    stage_peers_point(S, buf);
+}
 // the whole CTA of NT = blockDim.x threads
 template <int NT>
 __device__ __forceinline__ void stage_vectors(mc3b_sampler_t& S, double* buf) {
     stage_vectors_load<NT>(S, buf, threadIdx.x);
     stage_peers_load(S, buf, threadIdx.x, NT);
     __syncthreads();
-    S.pstep = buf; S.pmin = buf + MAXP; S.pmax = buf + 2 * MAXP; S.params0 = buf + 3 * MAXP;
-    if (S.prior) { S.prior = buf + 4 * MAXP; S.priorlow = buf + 5 * MAXP; S.priorup = buf + 6 * MAXP; }
-    S.ifree = reinterpret_cast<int32_t*>(buf + 7 * MAXP);
-    stage_peers_point(S, buf);
+    stage_point(S, buf);
 }
 
 // The proposal works on the free parameters in chunks of PCHUNK held in registers: the loads
@@ -190,9 +194,11 @@ __device__ __forceinline__ void chain_normals(const mc3b_sampler_t& S, const mc3
 // Jump, bounds, shared parameters and the snooker factor from the draws and the
 // population as of the start of generation gen (chain.py:195-255).  nrm0: the support
 // draws of the first chunk (chain_normals, j0 = 0); the later chunks draw their own.
+// have_x0: xv0 holds the first chunk of the chain's row, already read.
 template <bool REPLAY>
 __device__ __forceinline__ void propose_apply(const mc3b_sampler_t& S, const mc3b_draws_t& D, const Draws& dr,
-                                              const double (&nrm0)[PCHUNK], int64_t gen, int64_t c) {
+                                              const double (&nrm0)[PCHUNK], int64_t gen, int64_t c,
+                                              bool have_x0 = false, const double (&xv0)[PCHUNK] = {}) {
     const int nfree = S.nfree, npars = S.npars;
     // population as of the start of this generation (peer mode: half gen & 1)
     const double* Xg = S.X_peers ? S.X_peers[S.rank] + (gen & 1) * S.nchains * nfree : S.X;
@@ -240,7 +246,7 @@ __device__ __forceinline__ void propose_apply(const mc3b_sampler_t& S, const mc3
 #pragma unroll
         for (int q = 0; q < PCHUNK; q++) {          // one batch of loads per chunk
             const bool in = j0 + q < nfree;
-            xv[q] = in ? x[j0 + q] : 0.0;
+            xv[q] = !in ? 0.0 : j0 == 0 && have_x0 ? xv0[q] : x[j0 + q];
             av[q] = in && (snooker || demc) ? r1[j0 + q] : 0.0;
             bv[q] = in && (snooker || demc) ? r2[j0 + q] : 0.0;
             zv[q] = in && sjump ? zrow[j0 + q] : 0.0;
@@ -332,28 +338,53 @@ __device__ __forceinline__ double sum_partials(const double* partial, int64_t ld
     return nxt;
 }
 
-// Metropolis step of chain c (chain.py:257-289); nxt_data = data chi-squared of its
-// proposal (unused when the proposal was out of bounds).
-__device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double nxt_data, int64_t gen, int64_t zrow0,
-                                                 int64_t c) {
+// The Metropolis step of chain c (chain.py:257-289) in two halves.  metropolis_load reads
+// what the step needs of the chain's state: none of it depends on the proposal's
+// chi-squared, and during a launch only the chain's own thread writes it (k_propose wrote
+// inb, mrfactor and u before), so a kernel may issue these loads at entry, in one batch, and
+// apply the step once the chi-squared is known.
+struct ChainState {
+    int inb;
+    int32_t nacc;
+    double cur, mrf, u, best;
+    double xv[PCHUNK];              // the chain's current row, first chunk
+};
+// x of chain c in generation gen (peer mode: half gen & 1 of this device)
+__device__ __forceinline__ double* chain_row(const mc3b_sampler_t& S, int64_t gen, int64_t c) {
+    if (S.X_peers) return S.X_peers[S.rank] + (gen & 1) * S.nchains * S.nfree + c * S.nfree;
+    return S.X + c * S.nfree;
+}
+__device__ __forceinline__ ChainState metropolis_load(const mc3b_sampler_t& S, int64_t gen, int64_t c) {
+    const int nfree = S.nfree;
+    const double* x = chain_row(S, gen, c);
+    const double* np_ = S.nextp + c * S.npars;
+    ChainState st;
+    st.inb = S.inb[c];
+    st.cur = S.chisq_cur[c];
+    st.mrf = S.mrfactor[c]; st.u = S.u[c]; st.best = S.best_chisq[c];
+    st.nacc = S.naccept[c];
+#pragma unroll
+    for (int q = 0; q < PCHUNK; q++) st.xv[q] = q < nfree ? x[q] : 0.0;
+    // the rest of both rows goes to L1 meanwhile, without holding registers across the step
+    // (generic prefetch: no operation on a row in shared memory)
+    asm volatile("prefetch.L1 [%0];" ::"l"(np_));
+    asm volatile("prefetch.L1 [%0];" ::"l"(np_ + S.npars - 1));
+    asm volatile("prefetch.L1 [%0];" ::"l"(x + nfree - 1));
+    return st;
+}
+
+// nxt_data = data chi-squared of the proposal (unused when the proposal was out of bounds)
+__device__ __forceinline__ void metropolis_apply(const mc3b_sampler_t& S, const ChainState& st, double nxt_data,
+                                                 int64_t gen, int64_t zrow0, int64_t c) {
     const int nfree = S.nfree, npars = S.npars;
     const bool peer = S.X_peers != nullptr;
-    const int64_t half = S.nchains * nfree;
-    double* x = peer ? S.X_peers[S.rank] + (gen & 1) * half + c * nfree : S.X + c * nfree;
+    double* x = chain_row(S, gen, c);
     const double* np_ = S.nextp + c * npars;
-    // every per-chain value the step may need, loaded up front as one batch (behind the branches
-    // each was a round trip); the two rows go to L1 meanwhile without holding registers across the
-    // step (generic prefetch: no operation on a row in shared memory)
-    const int inb = S.inb[c];
-    double cur = S.chisq_cur[c];
-    const double mrf = S.mrfactor[c], u = S.u[c], best = S.best_chisq[c];
-    const int32_t nacc = S.naccept[c];
-    asm volatile("prefetch.L1 [%0];" ::"l"(np_));
-    asm volatile("prefetch.L1 [%0];" ::"l"(np_ + npars - 1));
-    asm volatile("prefetch.L1 [%0];" ::"l"(x));
-    asm volatile("prefetch.L1 [%0];" ::"l"(x + nfree - 1));
-    bool accept = false;
-    if (inb) {
+    double cur = st.cur;
+    const double mrf = st.mrf, u = st.u, best = st.best;
+    const int32_t nacc = st.nacc;
+    bool accept = false, newbest = false;
+    if (st.inb) {
         double nxt = nxt_data;
         if (S.prior != nullptr) {                    // stats.py:208-216 + stats.h:90-109
             double pr = 0.0;
@@ -374,38 +405,57 @@ __device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double
             S.chisq_cur[c] = nxt;
             S.naccept[c] = nacc + 1;
             if (nxt < best) {
+                newbest = true;
                 S.best_chisq[c] = nxt;
                 S.best_gen[c] = gen;
-                for (int j = 0; j < nfree; j++) S.best_x[c * nfree + j] = np_[S.ifree[j]];
             }
         }
     }
     const bool write = zrow0 >= 0 && zrow0 + c < S.zlen;
     const int64_t row = zrow0 + c;
-    if (!peer) {
-        if (accept)
-            for (int j = 0; j < nfree; j++) x[j] = np_[S.ifree[j]];
-        if (write)
-            for (int j = 0; j < nfree; j++) S.Z[row * nfree + j] = x[j];      // chain.py:276-289
-    } else {
-        // next state of this chain into half (gen+1)&1 of EVERY device (NVLink
-        // peer stores); thinned rows likewise when the history is shared
-        const int64_t dst = ((gen + 1) & 1) * half + c * nfree;
-        for (int j = 0; j < nfree; j++) {
-            const double v = accept ? np_[S.ifree[j]] : x[j];
-            for (int p = 0; p < S.world; p++) S.X_peers[p][dst + j] = v;
-            if (write) {
-                if (S.Z_peers) { for (int p = 0; p < S.world; p++) S.Z_peers[p][row * nfree + j] = v; }
-                else S.Z[row * nfree + j] = v;
+    // the chain's next state v (chain.py:276-289) into best_x, x and the thinned history, or in peer
+    // mode into half (gen+1)&1 of EVERY device (NVLink peer stores; thinned rows likewise when the
+    // history is shared).  A chunk's loads are issued before its stores: the rows may alias as far
+    // as the compiler knows, and a store between two loads would hold the second behind it.
+    const int64_t dst = ((gen + 1) & 1) * S.nchains * nfree + c * nfree;
+    if (accept || write || peer) {
+#pragma unroll 1
+        for (int j0 = 0; j0 < nfree; j0 += PCHUNK) {
+            double v[PCHUNK];
+#pragma unroll
+            for (int q = 0; q < PCHUNK; q++) {
+                const int j = j0 + q;
+                v[q] = j >= nfree ? 0.0 : accept ? np_[S.ifree[j]] : j0 == 0 ? st.xv[q] : x[j];
+            }
+#pragma unroll
+            for (int q = 0; q < PCHUNK; q++) {
+                const int j = j0 + q;
+                if (j >= nfree) break;
+                if (newbest) S.best_x[c * nfree + j] = v[q];
+                if (!peer) {
+                    if (accept) x[j] = v[q];
+                    if (write) S.Z[row * nfree + j] = v[q];
+                } else {
+                    for (int p = 0; p < S.world; p++) S.X_peers[p][dst + j] = v[q];
+                    if (write) {
+                        if (S.Z_peers) { for (int p = 0; p < S.world; p++) S.Z_peers[p][row * nfree + j] = v[q]; }
+                        else S.Z[row * nfree + j] = v[q];
+                    }
+                }
             }
         }
-        // (no fence here: the caller orders the CTA's peer stores with ONE system fence after
-        // a CTA barrier, before it counts the group as done -- see fused_metropolis / k_metropolis)
     }
+    // (no fence for the peer stores: the caller orders the CTA's peer stores with ONE system fence
+    // after a CTA barrier, before it counts the group as done -- see fused_metropolis / k_metropolis)
     if (write) {
         S.log_post[row] = -0.5 * cur;
         S.zchain[row] = (int32_t)c;
     }
+}
+// both halves back to back
+__device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double nxt_data, int64_t gen, int64_t zrow0,
+                                                 int64_t c) {
+    metropolis_apply(S, metropolis_load(S, gen, c), nxt_data, gen, zrow0, c);
 }
 
 
