@@ -628,6 +628,20 @@ int mc3b_dwt_chisq(int model_id, const double* params, int64_t ldp,
                    const double* model, int64_t ldm, const double* data,
                    int64_t n, void* workspace, double* chisq, void* stream);
 
+/* mc3b_dwt_chisq for a user model (_dwt.c:71-118 with the model of chain.py:317
+ * evaluated on the device): the model reads params[c, 0..nmodel), its nx inputs xs
+ * [host] (nx device pointers of n points) and its nk constants (fp64, device; NULL
+ * when nk = 0), and its values go straight into the D4 pyramid, never to memory.
+ * Same workspace (mc3b_dwt_workspace), checks and results as a built-in model; nx
+ * and nk must equal the handle's, nmodel <= npars - 3.  The wavelet likelihood is
+ * fp64: the handle must be the model's fp64 module (MC3B_ERR_ARG otherwise). */
+int mc3b_user_model_dwt_chisq(const mc3b_user_model_t* m, const double* params,
+                              int64_t ldp, int64_t nchains, int npars,
+                              const double* const* xs /*[host] nx device pointers*/,
+                              int nx, const double* consts, int nk,
+                              const double* data, int64_t n, void* workspace,
+                              double* chisq, void* stream);
+
 /* _dwt.daub4: forward (isign >= 0) or inverse (isign < 0) D4 transform of a
  * length-n2 array, n2 = 2^k >= 4; workspace holds n2 doubles; in and out
  * must not alias.  Zero padding to 2^k is the caller's (stats.dwt_daub4 does it). */

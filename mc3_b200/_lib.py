@@ -157,6 +157,8 @@ _SIGS = {
     'mc3b_dwt_workspace': (c_i64, [c_i64, c_i64]),
     'mc3b_dwt_chisq': (c_int, [c_int, c_vp, c_i64, c_i64, c_int, c_int, c_vp, c_vp,
                                c_i64, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    'mc3b_user_model_dwt_chisq': (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, ctypes.POINTER(c_vp), c_int, c_vp,
+                                          c_int, c_vp, c_i64, c_vp, c_vp, c_vp]),
     'mc3b_daub4': (c_int, [c_vp, c_i64, c_int, c_vp, c_vp, c_vp]),
     'mc3b_binrms_workspace': (c_i64, [c_i64, c_i64, c_i64]),
     'mc3b_binrms': (c_int, [c_vp, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp,

@@ -4,159 +4,20 @@
 // pyramid (periodic at every level, wavelet.h:16-51, 109-117), and only what
 // _dwt.c:96-110 consumes: the sum of squared detail coefficients of every level
 // and the last two smooth coefficients.  The n-point residual of a chain is
-// never written to memory:
+// never written to memory.  The kernels that read the model (k_dwt_reg_model,
+// k_dwt_pass, k_dwt_last) are in dwt_kernel.cuh, shared with the user models of
+// jit.cu; this file has the passes over given rows or coefficients (k_dwt_reg),
+// the schedule, the launches and the standalone transform.
 //
-//   k_dwt_pass  one warp per chain, 8 chains per CTA sharing the x/data tile.
-//               A tile of T inputs + halo H = 2^(L+1)-2 (taken modulo n, which
-//               reproduces the periodic wrap) goes through L levels inside
-//               shared memory; the T/2^L smooth outputs go to a workspace, the
-//               per-level detail sums stay in registers across the tiles of a
-//               span -> sums[chain, level, span].
-//   k_dwt_last  finishes the pyramid of the <=512 remaining coefficients in
-//               shared memory, adds the span sums in fixed order and evaluates
-//               the likelihood terms.
-//
-// For n = 2^20: pass(L=5) -> 2^15, pass(L=6) -> 512, last.  Bound: FP64 pipe
-// (about 8 FMA-class instructions per input point over all levels + model).
+// For n = 2^20: reg(4 levels) -> 2^16, reg -> 2^12, pass(L=3) -> 512, last.  Bound:
+// FP64 pipe (about 8 FMA-class instructions per input point over all levels + model).
 #include <type_traits>
-#include "models.cuh"
+#include "dwt_kernel.cuh"
 
 namespace {
 
-constexpr int CH = 8;          // chains (warps) per CTA
-constexpr int T = 512;         // inputs per tile
-constexpr int LMAX = 6;        // levels per pass
-constexpr int LASTMAX = 512;   // coefficients finished by k_dwt_last
-constexpr int MAXSPAN = 64;
-constexpr int MAXLEV = 40;
-
-__device__ __constant__ double kC[4] = {0.4829629131445341, 0.83651630373780772, 0.22414386804201339,
-                                        -0.12940952255126034};
-
-enum { SRC_MODEL = 0, SRC_GIVEN = 1, SRC_ARRAY = 2 };
-
-struct PassArgs {
-    const double* params; int64_t ldp; int64_t nchains;
-    const double* x; const double* data;         // SRC_MODEL / SRC_GIVEN
-    const double* rows; int64_t ldr;              // SRC_GIVEN: model rows; SRC_ARRAY: input coefficients
-    int64_t n_in;                                 // input length (2^k)
-    int L;                                        // levels in this pass
-    int lev0;                                     // levels done before this pass
-    int spans, tiles_per_span;
-    double* out; int64_t ldo;                     // smooth output rows
-    double* sums;                                 // [nchains, MAXLEV, MAXSPAN]
-};
-
-template <int SRC, class M>
-__global__ void __launch_bounds__(CH * 32) k_dwt_pass(PassArgs a) {
-    extern __shared__ __align__(16) double smem[];
-    const int H = (2 << a.L) - 2;
-    const int len0 = T + H;
-    double* sx = smem;                               // [len0] (SRC_MODEL)
-    double* sd = sx + (T + (2 << LMAX));             // [len0]
-    double* wbuf = sd + (T + (2 << LMAX));           // per warp: buf0[len0max] + buf1[len0max/2]
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    constexpr int B0 = T + (2 << LMAX), B1 = B0 / 2;
-    double* buf0 = wbuf + (size_t)warp * (B0 + B1);
-    double* buf1 = buf0 + B0;
-
-    int64_t c = (int64_t)blockIdx.x * CH + warp;
-    const bool live = c < a.nchains;
-    if (!live) c = a.nchains - 1;
-    M mdl;
-    if (SRC == SRC_MODEL) mdl.load(a.params + c * a.ldp);
-    const double c0 = kC[0], c1 = kC[1], c2 = kC[2], c3 = kC[3];
-    double acc[LMAX];
-#pragma unroll
-    for (int l = 0; l < LMAX; l++) acc[l] = 0.0;
-    const int64_t mask = a.n_in - 1;
-
-    for (int ts = 0; ts < a.tiles_per_span; ts++) {
-        const int64_t tile = (int64_t)blockIdx.y * a.tiles_per_span + ts;
-        const int64_t g0 = tile * T;
-        if (SRC == SRC_MODEL) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < len0; i += CH * 32) {
-                const int64_t g = (g0 + i) & mask;
-                sx[i] = a.x[g];
-                sd[i] = a.data[g];
-            }
-            __syncthreads();
-            for (int i = lane; i < len0; i += 32) buf0[i] = sd[i] - mdl.eval_safe(sx[i]);
-        } else if (SRC == SRC_GIVEN) {
-            const double* m = a.rows + c * a.ldr;
-            for (int i = lane; i < len0; i += 32) {
-                const int64_t g = (g0 + i) & mask;
-                buf0[i] = a.data[g] - m[g];
-            }
-        } else {
-            const double* m = a.rows + c * a.ldr;
-            for (int i = lane; i < len0; i += 32) buf0[i] = m[(g0 + i) & mask];
-        }
-        __syncwarp();
-        double* in = buf0;
-        double* ot = buf1;
-        int len = len0;
-#pragma unroll
-        for (int l = 1; l <= LMAX; l++) {
-            if (l <= a.L) {
-                const int lo = (len - 2) >> 1;
-                const int own = T >> l;
-                double s2 = 0.0;
-                for (int j = lane; j < lo; j += 32) {
-                    const double a0 = in[2 * j], a1 = in[2 * j + 1], a2 = in[2 * j + 2], a3 = in[2 * j + 3];
-                    ot[j] = c0 * a0 + c1 * a1 + c2 * a2 + c3 * a3;
-                    if (j < own) {
-                        const double d = c3 * a0 - c2 * a1 + c1 * a2 - c0 * a3;
-                        s2 = fma(d, d, s2);
-                    }
-                }
-                acc[l - 1] += s2;
-                __syncwarp();
-                double* t = in; in = ot; ot = t;
-                len = lo;
-            }
-        }
-        if (live) {
-            double* o = a.out + c * a.ldo + (g0 >> a.L);
-            for (int j = lane; j < (T >> a.L); j += 32) o[j] = in[j];
-        }
-        __syncwarp();
-    }
-#pragma unroll
-    for (int l = 0; l < LMAX; l++) {
-        if (l < a.L) {
-            double v = acc[l];
-            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-            if (lane == 0 && live) a.sums[(c * MAXLEV + (a.lev0 + l)) * MAXSPAN + blockIdx.y] = v;
-        }
-    }
-}
-
-// ---- register stage: 4 levels per pass without the shared-memory round trips --
-// A warp takes blocks of 512 consecutive inputs of its chain (read modulo n).
-// The block is loaded/evaluated coalesced, transposed once through a padded
-// shared-memory row so that lane l owns inputs [16 l, 16 l + 16), and the four
-// levels then run in registers: each level needs two values of the next lane
-// (shuffle) and halves the lane's values (16 -> 8 -> 4 -> 2 -> 1).  Lane 31 has
-// no right neighbour, so the last 2 of the 32 level-4 outputs are not valid:
-// blocks advance by 480 inputs (30 outputs) and an output is counted by the
-// block that owns its first input.  Shared-memory traffic drops from ~64 to 16
-// bytes per input; the FP64 pipe becomes the limiter.
-constexpr int RB = 512;             // inputs per block
-constexpr int RADV = 480;           // block advance (30 lanes x 16)
-
-struct RegArgs {
-    const double* params; int64_t ldp; int64_t nchains;
-    const double* x; const double* data;
-    const double* rows; int64_t ldr;
-    int64_t n_in;
-    int lev0;
-    int64_t nblocks; int blocks_per_span;
-    double* out; int64_t ldo;
-    double* sums;
-};
-
+// The register stage (dwt_kernel.cuh) over given model rows or over the coefficients of
+// an earlier pass: every warp reads its own chain's row and transposes it.
 template <int SRC, class M>
 __global__ void __launch_bounds__(CH * 32) k_dwt_reg(RegArgs a) {
     __shared__ double tr[CH][RB + RB / 16];          // padded transpose rows (stride 17)
@@ -242,174 +103,6 @@ __global__ void __launch_bounds__(CH * 32) k_dwt_reg(RegArgs a) {
     }
 }
 
-// Built-in models: the 8 chains of a CTA walk the same blocks, so x and data are
-// staged ONCE per CTA (double-buffered, padded rows of 18 so that a lane's 16
-// consecutive values are conflict-free 16-byte reads) and every warp evaluates
-// its own chain's residuals straight into the lane-contiguous registers -- no
-// per-warp transpose.  L1/shared-memory wavefronts per block and warp: ~80
-// instead of 128.
-constexpr int RPAD = 18;                         // doubles per 16-value row
-
-template <class M>
-__global__ void __launch_bounds__(CH * 32) k_dwt_reg_model(RegArgs a) {
-    __shared__ __align__(16) double sxd[2][2][32 * RPAD];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    int64_t c = (int64_t)blockIdx.x * CH + warp;
-    const bool live = c < a.nchains;
-    if (!live) c = a.nchains - 1;
-    M mdl;
-    mdl.load(a.params + c * a.ldp);
-    const double c0 = kC[0], c1 = kC[1], c2 = kC[2], c3 = kC[3];
-    const int64_t mask = a.n_in - 1;
-    double acc[4] = {0.0, 0.0, 0.0, 0.0};
-    const int64_t b_begin = (int64_t)blockIdx.y * a.blocks_per_span;
-    int64_t b_end = b_begin + a.blocks_per_span;
-    if (b_end > a.nblocks) b_end = a.nblocks;
-    auto fill = [&](int64_t b, int buf) {
-        const int64_t g0 = b * RADV;
-#pragma unroll
-        for (int q = 0; q < RB / (CH * 32); q++) {
-            const int idx = q * CH * 32 + threadIdx.x;
-            const int64_t g = (g0 + idx) & mask;
-            const int pos = (idx >> 4) * RPAD + (idx & 15);
-            sxd[buf][0][pos] = a.x[g];
-            sxd[buf][1][pos] = a.data[g];
-        }
-    };
-    if (b_begin < b_end) fill(b_begin, 0);
-    // One block; INTERIOR (compile time): every output the block owns exists, so the
-    // squares are summed without a per-element select (the ALU pipe was as busy as the
-    // FP64 pipe: profiles/r2_dwt_reg_model.md).
-    auto do_block = [&](int64_t b, int buf, auto interior_tag) {
-        constexpr bool interior = decltype(interior_tag)::value;
-        const int64_t g0 = b * RADV;
-        double v[18];
-        const double2* px = reinterpret_cast<const double2*>(&sxd[buf][0][lane * RPAD]);
-        const double2* pd = reinterpret_cast<const double2*>(&sxd[buf][1][lane * RPAD]);
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-            const double2 xv = px[k], dv = pd[k];
-            v[2 * k] = dv.x - mdl.eval_safe(xv.x);
-            v[2 * k + 1] = dv.y - mdl.eval_safe(xv.y);
-        }
-        int cnt = 16;
-#pragma unroll
-        for (int l = 0; l < 4; l++) {
-            v[cnt] = __shfl_down_sync(0xffffffffu, v[0], 1);
-            v[cnt + 1] = __shfl_down_sync(0xffffffffu, v[1], 1);
-            const int half = cnt >> 1;
-            const int64_t lev_pos0 = (g0 >> (l + 1)) + (int64_t)lane * half;
-            const int64_t lev_n = a.n_in >> (l + 1);
-            double s2 = 0.0;
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-                if (j < half) {
-                    const double a0 = v[2 * j], a1 = v[2 * j + 1], a2 = v[2 * j + 2], a3 = v[2 * j + 3];
-                    const double sm = fma(c3, a3, fma(c2, a2, fma(c1, a1, c0 * a0)));
-                    const double d = fma(-c0, a3, fma(c1, a2, fma(-c2, a1, c3 * a0)));
-                    if (interior) s2 = fma(d, d, s2);
-                    else s2 = fma(d, (lev_pos0 + j < lev_n) ? d : 0.0, s2);
-                    v[j] = sm;
-                }
-            }
-            acc[l] += (lane < 30) ? s2 : 0.0;
-            cnt = half;
-        }
-        const int64_t o = (g0 >> 4) + lane;
-        if (live && lane < 30 && (interior || o < (a.n_in >> 4))) a.out[c * a.ldo + o] = v[0];
-    };
-    for (int64_t b = b_begin; b < b_end; b++) {
-        const int buf = (int)((b - b_begin) & 1);
-        __syncthreads();                             // tile b is complete; tile b-1 is no longer read
-        if (b + 1 < b_end) fill(b + 1, buf ^ 1);
-        if (b * RADV + RB <= a.n_in) do_block(b, buf, std::true_type{});
-        else do_block(b, buf, std::false_type{});
-    }
-#pragma unroll
-    for (int l = 0; l < 4; l++) {
-        double t = acc[l];
-        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-        if (lane == 0 && live) a.sums[(c * MAXLEV + (a.lev0 + l)) * MAXSPAN + blockIdx.y] = t;
-    }
-}
-
-struct LastArgs {
-    const double* params; int64_t ldp; int npars; int64_t nchains;
-    const double* x; const double* data;
-    const double* rows; int64_t ldr;
-    int n0;                      // coefficients to finish (4..512, 2^j)
-    int lev0;                    // levels done by the passes
-    int kbits;                   // n = 2^kbits
-    const double* sums;          // [nchains, MAXLEV, MAXSPAN]
-    int spans_of_level[MAXLEV];  // spans that hold level l (levels done by the passes)
-    double* chisq;
-};
-constexpr int CHL = 4;           // chains (warps) per CTA of k_dwt_last
-
-template <int SRC, class M>
-__global__ void __launch_bounds__(CHL * 32) k_dwt_last(LastArgs a) {
-    __shared__ double wb[CHL][LASTMAX + LASTMAX / 2];
-    __shared__ double lev_s2[CHL][MAXLEV];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    int64_t c = (int64_t)blockIdx.x * CHL + warp;
-    const bool live = c < a.nchains;
-    if (!live) c = a.nchains - 1;
-    double* in = wb[warp];
-    double* ot = in + LASTMAX;
-    const double c0 = kC[0], c1 = kC[1], c2 = kC[2], c3 = kC[3];
-    if (SRC == SRC_MODEL) {
-        M mdl;
-        mdl.load(a.params + c * a.ldp);
-        for (int i = lane; i < a.n0; i += 32) in[i] = a.data[i] - mdl.eval_safe(a.x[i]);
-    } else if (SRC == SRC_GIVEN) {
-        const double* m = a.rows + c * a.ldr;
-        for (int i = lane; i < a.n0; i += 32) in[i] = a.data[i] - m[i];
-    } else {
-        const double* m = a.rows + c * a.ldr;
-        for (int i = lane; i < a.n0; i += 32) in[i] = m[i];
-    }
-    __syncwarp();
-    int lev = a.lev0;
-    for (int nn = a.n0; nn >= 4; nn >>= 1, lev++) {
-        const int nh = nn >> 1;
-        double s2 = 0.0;
-        for (int j = lane; j < nh; j += 32) {
-            const double a0 = in[2 * j], a1 = in[2 * j + 1], a2 = in[(2 * j + 2) & (nn - 1)],
-                         a3 = in[(2 * j + 3) & (nn - 1)];
-            ot[j] = c0 * a0 + c1 * a1 + c2 * a2 + c3 * a3;
-            const double d = c3 * a0 - c2 * a1 + c1 * a2 - c0 * a3;
-            s2 = fma(d, d, s2);
-        }
-        for (int o = 16; o > 0; o >>= 1) s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-        if (lane == 0) lev_s2[warp][lev] = s2;
-        __syncwarp();
-        double* t = in; in = ot; ot = t;
-    }
-    // levels done by the passes: add their span sums in span order
-    for (int l = lane; l < a.lev0; l += 32) {
-        double s = 0.0;
-        const int ns = a.spans_of_level[l];
-        const double* p = a.sums + (c * MAXLEV + l) * MAXSPAN;
-        for (int k = 0; k < ns; k++) s += p[k];
-        lev_s2[warp][l] = s;
-    }
-    __syncwarp();
-    if (lane == 0 && live) {                        // _dwt.c:96-110
-        const double* p = a.params + c * a.ldp;
-        const double gamma = p[a.npars - 3], sr = p[a.npars - 2], sw = p[a.npars - 1];
-        const double g = 0.72134752;
-        const double sS2 = sr * sr * pow(2.0, -gamma) * g + sw * sw;
-        double chi = in[0] * in[0] / sS2 + in[1] * in[1] / sS2 + 2.0 * log(2.0 * M_PI * sS2);
-        const int Msc = a.kbits;
-        for (int m = 1; m < Msc; m++) {
-            const double sW2 = sr * sr * pow(2.0, -gamma * m) + sw * sw;
-            const double cnt = (double)(1 << m);
-            chi += lev_s2[warp][Msc - 1 - m] / sW2 + cnt * log(2.0 * M_PI * sW2);
-        }
-        a.chisq[c] = chi;
-    }
-}
-
 // ---- standalone transform (one array) ---------------------------------------
 __global__ void k_d4_fwd(const double* src, double* smooth, double* detail, int64_t nn) {
     const int64_t nh = nn >> 1;
@@ -469,8 +162,6 @@ Schedule make_schedule(int64_t n) {
     return s;
 }
 
-size_t pass_smem() { return (size_t)(2 * (T + (2 << LMAX)) + CH * ((T + (2 << LMAX)) * 3 / 2)) * sizeof(double); }
-
 }  // namespace
 
 extern "C" int64_t mc3b_dwt_workspace(int64_t nchains, int64_t n) {
@@ -485,29 +176,38 @@ extern "C" int64_t mc3b_dwt_workspace(int64_t nchains, int64_t n) {
     return words * 8;
 }
 
+// u: a user model (SRC_MODEL, M unused), whose first pass runs on the kernels of its module;
+// nullptr for the built-in M
 template <int SRC, class M>
 static int dwt_run(const Schedule& sc, int kbits, const double* params, int64_t ldp, int64_t nchains, int npars,
                    const double* x, const double* model, int64_t ldm, const double* data, int64_t n, double* ws,
-                   double* chisq, cudaStream_t st) {
+                   double* chisq, cudaStream_t st, const DwtUserModel* u = nullptr) {
+    const double* xs[MC3B_MAX_INPUTS] = {};
+    for (int j = 0; u && j < u->nx; j++) xs[j] = u->xs[j];
+    const double* uconst = u ? u->consts : nullptr;
     double* ping = ws;
     double* pong = ping + (sc.npass > 0 ? nchains * (n >> sc.L[0]) : 0);
     double* sums = pong + (sc.npass > 1 ? nchains * (n >> (sc.L[0] + sc.L[1])) : 0);
-    LastArgs la;
+    LastArgsX la;
     for (int l = 0; l < MAXLEV; l++) la.spans_of_level[l] = 0;
     const unsigned groups = (unsigned)ceil_div64(nchains, CH);
     const double* cur_rows = model; int64_t cur_ld = ldm;
     int lev0 = 0;
     for (int p = 0; p < sc.npass; p++) {
         if (sc.kind[p] == 1) {
-            RegArgs r;
+            RegArgsX r;
             r.params = params; r.ldp = ldp; r.nchains = nchains; r.x = x; r.data = data;
             r.rows = cur_rows; r.ldr = cur_ld; r.n_in = sc.nin[p]; r.lev0 = lev0;
             r.nblocks = sc.nblocks[p]; r.blocks_per_span = sc.tps[p];
             r.out = (p % 2 == 0) ? ping : pong; r.ldo = sc.nin[p] >> 4; r.sums = sums;
+            for (int j = 0; j < MC3B_MAX_INPUTS; j++) r.xs[j] = xs[j];
+            r.uconst = uconst;
             // spans actually needed with whole blocks per span
             const int spans = (int)ceil_div64(sc.nblocks[p], sc.tps[p]);
             dim3 grid(groups, (unsigned)spans);
-            if (p == 0 && SRC == SRC_MODEL) k_dwt_reg_model<M><<<grid, CH * 32, 0, st>>>(r);
+            void* args[] = {&r};
+            if (p == 0 && u) MC3B_CUDA(cudaLaunchKernel(u->reg, grid, dim3(CH * 32), args, 0, st));
+            else if (p == 0 && SRC == SRC_MODEL) k_dwt_reg_model<M, RegArgs><<<grid, CH * 32, 0, st>>>(r);
             else if (p == 0) k_dwt_reg<SRC, M><<<grid, CH * 32, 0, st>>>(r);
             else k_dwt_reg<SRC_ARRAY, BoxModel<double>><<<grid, CH * 32, 0, st>>>(r);
             MC3B_CHECK_LAUNCH("k_dwt_reg");
@@ -516,20 +216,25 @@ static int dwt_run(const Schedule& sc, int kbits, const double* params, int64_t 
             cur_rows = r.out; cur_ld = r.ldo;
             continue;
         }
-        PassArgs a;
+        PassArgsX a;
         a.params = params; a.ldp = ldp; a.nchains = nchains; a.x = x; a.data = data;
         a.rows = cur_rows; a.ldr = cur_ld; a.n_in = sc.nin[p]; a.L = sc.L[p]; a.lev0 = lev0;
         a.spans = sc.spans[p]; a.tiles_per_span = sc.tps[p];
         a.out = (p % 2 == 0) ? ping : pong; a.ldo = sc.nin[p] >> sc.L[p]; a.sums = sums;
+        for (int j = 0; j < MC3B_MAX_INPUTS; j++) a.xs[j] = xs[j];
+        a.uconst = uconst;
         dim3 grid(groups, (unsigned)sc.spans[p]);
-        const size_t sm = pass_smem();
-        if (p == 0) {
-            MC3B_CUDA(cudaFuncSetAttribute(k_dwt_pass<SRC, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-            k_dwt_pass<SRC, M><<<grid, CH * 32, sm, st>>>(a);
+        const size_t sm = pass_smem(1);
+        void* args[] = {&a};
+        if (p == 0 && u) {
+            MC3B_CUDA(cudaLaunchKernel(u->pass, grid, dim3(CH * 32), args, pass_smem(u->nx), st));
+        } else if (p == 0) {
+            MC3B_CUDA(cudaFuncSetAttribute(k_dwt_pass<SRC, M, PassArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            k_dwt_pass<SRC, M, PassArgs><<<grid, CH * 32, sm, st>>>(a);
         } else {
-            MC3B_CUDA(cudaFuncSetAttribute(k_dwt_pass<SRC_ARRAY, M>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            MC3B_CUDA(cudaFuncSetAttribute(k_dwt_pass<SRC_ARRAY, M, PassArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)sm));
-            k_dwt_pass<SRC_ARRAY, M><<<grid, CH * 32, sm, st>>>(a);
+            k_dwt_pass<SRC_ARRAY, M, PassArgs><<<grid, CH * 32, sm, st>>>(a);
         }
         MC3B_CHECK_LAUNCH("k_dwt_pass");
         for (int l = 0; l < sc.L[p]; l++) la.spans_of_level[lev0 + l] = sc.spans[p];
@@ -539,22 +244,34 @@ static int dwt_run(const Schedule& sc, int kbits, const double* params, int64_t 
     la.params = params; la.ldp = ldp; la.npars = npars; la.nchains = nchains; la.x = x; la.data = data;
     la.rows = cur_rows; la.ldr = cur_ld; la.n0 = sc.n0; la.lev0 = lev0; la.kbits = kbits; la.sums = sums;
     la.chisq = chisq;
+    for (int j = 0; j < MC3B_MAX_INPUTS; j++) la.xs[j] = xs[j];
+    la.uconst = uconst;
     const unsigned lgroups = (unsigned)ceil_div64(nchains, CHL);
-    if (sc.npass == 0) k_dwt_last<SRC, M><<<lgroups, CHL * 32, 0, st>>>(la);
-    else k_dwt_last<SRC_ARRAY, M><<<lgroups, CHL * 32, 0, st>>>(la);
+    void* args[] = {&la};
+    if (sc.npass == 0 && u) MC3B_CUDA(cudaLaunchKernel(u->last, dim3(lgroups), dim3(CHL * 32), args, 0, st));
+    else if (sc.npass == 0) k_dwt_last<SRC, M, LastArgs><<<lgroups, CHL * 32, 0, st>>>(la);
+    else k_dwt_last<SRC_ARRAY, M, LastArgs><<<lgroups, CHL * 32, 0, st>>>(la);
     MC3B_CHECK_LAUNCH("k_dwt_last");
+    return MC3B_OK;
+}
+
+// the checks every wavelet chi-squared runs: kbits = log2 n
+static int dwt_check(const double* params, int64_t ldp, int64_t nchains, int npars, const double* data, int64_t n,
+                     void* workspace, double* chisq, int* kbits) {
+    MC3B_CHECK_ARG(params && data && chisq && workspace && nchains > 0, "bad arguments");
+    MC3B_CHECK_ARG(n >= 4 && (n & (n - 1)) == 0, "dwt_chisq needs n = 2^k >= 4 (got %lld)", (long long)n);
+    MC3B_CHECK_ARG(npars >= 3 && npars <= ldp, "wavelet chisq needs at least three parameters");
+    *kbits = ilog2(n);
+    MC3B_CHECK_ARG(*kbits < MAXLEV, "n too large");
     return MC3B_OK;
 }
 
 extern "C" int mc3b_dwt_chisq(int model_id, const double* params, int64_t ldp, int64_t nchains, int npars, int nmodel,
                               const double* x, const double* model, int64_t ldm, const double* data, int64_t n,
                               void* workspace, double* chisq, void* stream) {
-    MC3B_CHECK_ARG(params && data && chisq && workspace && nchains > 0, "bad arguments");
-    MC3B_CHECK_ARG(n >= 4 && (n & (n - 1)) == 0, "dwt_chisq needs n = 2^k >= 4 (got %lld)", (long long)n);
-    MC3B_CHECK_ARG(npars >= 3 && npars <= ldp, "wavelet chisq needs at least three parameters");
+    int kbits = 0;
+    if (int rc = dwt_check(params, ldp, nchains, npars, data, n, workspace, chisq, &kbits)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const int kbits = ilog2(n);
-    MC3B_CHECK_ARG(kbits < MAXLEV, "n too large");
     Schedule sc = make_schedule(n);
     double* ws = (double*)workspace;
     if (model_id < 0) {
@@ -570,6 +287,18 @@ extern "C" int mc3b_dwt_chisq(int model_id, const double* params, int64_t ldp, i
                         return (dwt_run<SRC_MODEL, M>(sc, kbits, params, ldp, nchains, npars, x, model, ldm, data, n,
                                                       ws, chisq, st)));
     return MC3B_OK;
+}
+
+int mc3b_dwt_chisq_user(const DwtUserModel& u, const double* params, int64_t ldp, int64_t nchains, int npars,
+                        const double* data, int64_t n, void* workspace, double* chisq, cudaStream_t st) {
+    int kbits = 0;
+    if (int rc = dwt_check(params, ldp, nchains, npars, data, n, workspace, chisq, &kbits)) return rc;
+    MC3B_CHECK_ARG(u.nmodel <= npars - 3, "the model takes %d parameters, more than npars - 3 = %d", u.nmodel,
+                   npars - 3);
+    for (int j = 0; j < u.nx; j++) MC3B_CHECK_ARG(u.xs[j] != nullptr, "null pointer (input %d)", j);
+    // M is unused: pass 0 (or the last pass) runs on u's kernels, later passes on SRC_ARRAY
+    return dwt_run<SRC_MODEL, BoxModel<double>>(make_schedule(n), kbits, params, ldp, nchains, npars, u.xs[0],
+                                                 nullptr, 0, data, n, (double*)workspace, chisq, st, &u);
 }
 
 extern "C" int mc3b_daub4(const double* in, int64_t n2, int isign, void* workspace, double* out, void* stream) {

@@ -25,6 +25,7 @@
 #include <string>
 #include <vector>
 #include "chisq_args.cuh"
+#include "dwt_kernel.cuh"
 #include "jit_headers.inc"
 
 namespace {
@@ -136,9 +137,27 @@ std::string eval_symbol(const Desc& d) {
     return "_ZN8mc3b_jit14k_model_eval_xINS_" + w + "EEEvPKdlN10mc3b_chisq10EvalInputsElPd";
 }
 
+// The D4 kernels of an fp64 module that read the model (dwt_kernel.cuh): the wavelet
+// likelihood's first pass.  [0] k_dwt_reg_model, [1] k_dwt_pass<SRC_MODEL>, [2] k_dwt_last<SRC_MODEL>
+std::string dwt_expr(const Desc& d, int k) {
+    const std::string w = wrapper_expr(d);
+    if (k == 0) return "mc3b_jit::k_dwt_reg_model<" + w + ", mc3b_jit::RegArgsX>";
+    if (k == 1) return "mc3b_jit::k_dwt_pass<mc3b_jit::SRC_MODEL, " + w + ", mc3b_jit::PassArgsX>";
+    return "mc3b_jit::k_dwt_last<mc3b_jit::SRC_MODEL, " + w + ", mc3b_jit::LastArgsX>";
+}
+std::string dwt_symbol(const Desc& d, int k) {
+    const std::string w = wrapper_symbol(d);
+    if (k == 0) return "_ZN8mc3b_jit15k_dwt_reg_modelINS_" + w + "ENS_8RegArgsXEEEvT0_";
+    if (k == 1) return "_ZN8mc3b_jit10k_dwt_passILi0ENS_" + w + "ENS_9PassArgsXEEEvT1_";
+    return "_ZN8mc3b_jit10k_dwt_lastILi0ENS_" + w + "ENS_9LastArgsXEEEvT1_";
+}
+// sizes of the three argument blocks, one entry of the ABI record
+constexpr long long kDwtArgsSizes =
+    (long long)sizeof(RegArgsX) | (long long)sizeof(PassArgsX) << 16 | (long long)sizeof(LastArgsX) << 32;
+
 // What the module reports about itself (mc3b_jit_abi), checked before any launch.
 enum { ABI_VERSION, ABI_ARGS_SIZE, ABI_DTYPE, ABI_NMODEL, ABI_WARPS, ABI_TILE, ABI_NINPUTS, ABI_NCONST, ABI_NWORK,
-       ABI_PREPARE, ABI_N };
+       ABI_PREPARE, ABI_DWT_ARGS, ABI_N };
 
 // The user's source in its namespace, with `real` defined and line numbers of model.cu.
 std::string user_unit(const char* user, int dtype) {
@@ -154,7 +173,7 @@ std::string user_unit(const char* user, int dtype) {
 // Translation unit around the user's source; model_line / prepare_line: the lines of
 // `model` and `prepare` in it.
 std::string jit_source(const char* user, const Desc& d, int model_line, int prepare_line) {
-    std::string s = user_unit(user, d.dtype);
+    std::string s = "#include \"dwt_kernel.cuh\"\n" + user_unit(user, d.dtype);
     const int ninputs = d.ninputs;
     if (ninputs > 1) {
         // the call of the wrapper, reported at the line of `model`: a model of another
@@ -231,10 +250,11 @@ std::string jit_source(const char* user, const Desc& d, int model_line, int prep
              "};\n";
     }
     s += "}  // namespace mc3b_jit\n";
-    char b[320];
+    char b[480];
     snprintf(b, sizeof(b),
              "extern \"C\" __device__ long long mc3b_jit_abi[%d] = {MC3B_VERSION, sizeof(ChisqArgs<mc3b_user::real>), "
-             "%d, %d, WARPS, tilecfg<mc3b_user::real>::TILE, %d, %d, %d, %d};\n",
+             "%d, %d, WARPS, tilecfg<mc3b_user::real>::TILE, %d, %d, %d, %d, (long long)sizeof(mc3b_jit::RegArgsX) | "
+             "(long long)sizeof(mc3b_jit::PassArgsX) << 16 | (long long)sizeof(mc3b_jit::LastArgsX) << 32};\n",
              (int)ABI_N, d.dtype, d.nmodel, ninputs, d.nconst, d.nwork, d.prepare ? 1 : 0);
     s += b;
     return s;
@@ -320,6 +340,7 @@ struct mc3b_user_model {
     cudaLibrary_t lib;
     cudaKernel_t chisq[2][3];      // [uniform sigma][LC = 32, 8, 1]
     cudaKernel_t eval;             // k_model_eval, k_model_eval_x (ninputs > 1) or k_model_eval_k (Desc::k)
+    cudaKernel_t dwt[3];           // fp64: dwt_expr's kernels; fp32: none
     Desc d;
     std::vector<char> image;       // the CUBIN, kept for the lifetime of the library
 };
@@ -426,6 +447,10 @@ extern "C" int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* 
         }
     exprs.push_back(eval_expr(d));
     symbols.push_back(eval_symbol(d));
+    for (int k = 0; d.dtype == MC3B_F64 && k < 3; k++) {
+        exprs.push_back(dwt_expr(d, k));
+        symbols.push_back(dwt_symbol(d, k));
+    }
     for (const std::string& e : exprs) nv->add_name(prog, e.c_str());
     r = nv->compile(prog, 5, kOpts);
     program_log(nv, prog, log, logcap);
@@ -501,7 +526,8 @@ extern "C" int mc3b_user_model_load_desc(const void* cubin, int64_t size, const 
                                    (long long)(dtype == MC3B_F64 ? sizeof(ChisqArgs<double>) : sizeof(ChisqArgs<float>)),
                                    dtype, desc->nmodel, WARPS,
                                    dtype == MC3B_F64 ? tilecfg<double>::TILE : tilecfg<float>::TILE, desc->ninputs,
-                                   desc->nconst, desc->nwork, abi[ABI_PREPARE] == 1 || desc->nwork > 0 ? 1 : 0};
+                                   desc->nconst, desc->nwork, abi[ABI_PREPARE] == 1 || desc->nwork > 0 ? 1 : 0,
+                                   kDwtArgsSizes};
     for (int i = 0; i < ABI_N; i++) {
         if (abi[i] != want[i]) {
             mc3b_set_error("the module does not match this library (ABI entry %d: %lld, expected %lld): "
@@ -517,6 +543,20 @@ extern "C" int mc3b_user_model_load_desc(const void* cubin, int64_t size, const 
         }
     e = cudaLibraryGetKernel(&m->eval, m->lib, eval_symbol(m->d).c_str());
     if (e != cudaSuccess) { mc3b_set_error("cudaLibraryGetKernel: %s", cudaGetErrorString(e)); return fail(MC3B_ERR_CUDA); }
+    if (dtype == MC3B_F64) {
+        for (int k = 0; k < 3; k++) {
+            e = cudaLibraryGetKernel(&m->dwt[k], m->lib, dwt_symbol(m->d, k).c_str());
+            if (e != cudaSuccess) { mc3b_set_error("cudaLibraryGetKernel: %s", cudaGetErrorString(e)); return fail(MC3B_ERR_CUDA); }
+        }
+        // k_dwt_pass takes more than 48 KB of dynamic shared memory: set here, once per device,
+        // so that no launch (or graph capture) has to
+        int ndev = 0;
+        e = cudaGetDeviceCount(&ndev);
+        for (int dev = 0; e == cudaSuccess && dev < ndev; dev++)
+            e = cudaKernelSetAttributeForDevice(m->dwt[1], cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                (int)pass_smem(m->d.ninputs), dev);
+        if (e != cudaSuccess) { mc3b_set_error("k_dwt_pass shared memory: %s", cudaGetErrorString(e)); return fail(MC3B_ERR_CUDA); }
+    }
     *out = m;
     return MC3B_OK;
 }
@@ -662,4 +702,19 @@ extern "C" int mc3b_user_model_eval_consts(const mc3b_user_model_t* m, const dou
     MC3B_CHECK_ARG(nx == m->d.ninputs, "this model takes %d inputs, got %d", m->d.ninputs, nx);
     MC3B_CHECK_ARG(nk == m->d.nconst, "this model takes %d constants, got %d", m->d.nconst, nk);
     return user_eval(m, params, ldp, nchains, xs, consts, n, out, stream);
+}
+
+extern "C" int mc3b_user_model_dwt_chisq(const mc3b_user_model_t* m, const double* params, int64_t ldp,
+                                         int64_t nchains, int npars, const double* const* xs, int nx,
+                                         const double* consts, int nk, const double* data, int64_t n,
+                                         void* workspace, double* chisq, void* stream) {
+    MC3B_CHECK_ARG(m && xs, "null pointer");
+    MC3B_CHECK_ARG(m->d.dtype == MC3B_F64,
+                   "the wavelet likelihood takes the fp64 module of a user model; this handle is fp32");
+    MC3B_CHECK_ARG(nx == m->d.ninputs, "this model takes %d inputs, got %d", m->d.ninputs, nx);
+    MC3B_CHECK_ARG(nk == m->d.nconst, "this model takes %d constants, got %d", m->d.nconst, nk);
+    MC3B_CHECK_ARG(consts || m->d.nconst == 0, "null pointer (constants)");
+    const DwtUserModel u = {(const void*)m->dwt[0], (const void*)m->dwt[1], (const void*)m->dwt[2], nx, m->d.nmodel,
+                            xs, consts};
+    return mc3b_dwt_chisq_user(u, params, ldp, nchains, npars, data, n, workspace, chisq, (cudaStream_t)stream);
 }

@@ -638,6 +638,11 @@ class Population:
                           _lib.ld(P), nb, self.npars, self.nmodel,
                           self.d_x.data_ptr(), None, 0, self.d_data.data_ptr(),
                           self.ndata, ws.data_ptr(), out.data_ptr(), st)
+            elif self.kind == 'cuda':
+                # the model is evaluated inside the D4 kernels of its fp64 module: no rows
+                _lib.call('mc3b_user_model_dwt_chisq', self.jit_eval, P.data_ptr(), _lib.ld(P), nb,
+                          self.npars, self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst,
+                          self.d_data.data_ptr(), self.ndata, ws.data_ptr(), out.data_ptr(), st)
             else:
                 m = self._model_rows(P)
                 _lib.call('mc3b_dwt_chisq', -1, P.data_ptr(), _lib.ld(P), nb,
