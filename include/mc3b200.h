@@ -121,9 +121,10 @@ int mc3b_model_chisq(int model_id, int dtype, const double* params, int64_t ldp,
  *                rows (split order) plus priors and takes their Metropolis step, exactly
  *                as mc3b_metropolis(fuse, partial, ldpartial, nsplit, c_off, gen, zrow0,
  *                c_off, c_off + nchains) would -- without the second launch.  fuse_done:
- *                device int32[groups + 1] (groups <= nchains/32 + 1), zero before the
- *                first use, left zero by every launch.  advance: the last group also
- *                increments *fuse->gen_dev (replaces mc3b_advance).
+ *                device int32[groups + 3] (groups <= nchains/32 + 1), 8-byte aligned, zero
+ *                before the first use, left zero by every launch: a counter per group, then
+ *                the launch's 64-bit arrival word at the first 8-byte-aligned slot after them.
+ *                advance: the last group also increments *fuse->gen_dev (replaces mc3b_advance).
  * folded         non-NULL (fp64, MC3B_MODEL_SINUSOID_GRID, uniform_sigma): the copy of
  *                `data` written by mc3b_fold_data; the kernel then works on point pairs
  *                mirrored about block centres (3.3 instead of 6 FP64 instructions per

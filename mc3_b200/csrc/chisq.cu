@@ -234,7 +234,8 @@ int mc3b_chisq_setup(const double* params, int64_t ldp, int64_t nchains, const v
     MC3B_CHECK_ARG(groups <= 0x7fffffff, "too many chains for one launch");
     A.f.on = 0;
     if (o.fuse != nullptr) {
-        MC3B_CHECK_ARG(o.fuse_done != nullptr, "the fused Metropolis epilogue needs its counters (fuse_done)");
+        MC3B_CHECK_ARG(o.fuse_done != nullptr && ((uintptr_t)o.fuse_done & 7) == 0,
+                       "the fused Metropolis epilogue needs its counters (fuse_done, 8-byte aligned)");
         MC3B_CHECK_ARG(o.gen >= 0 || (o.fuse->gen_dev && o.fuse->thinning > 0),
                        "device-driven generations need gen_dev and thinning");
         MC3B_CHECK_ARG(!o.advance || o.fuse->gen_dev, "advance needs gen_dev");

@@ -38,7 +38,7 @@ constexpr int SCHED_MAX = 384;      // splits a size schedule can describe (else
 struct FuseArgs {
     int on;
     int advance;                    // bump *S.gen_dev when every group is done
-    int32_t* done;                  // [groups + 1] arrival counters; zero before the first launch, self-resetting
+    int32_t* done;                  // arrival counters (fused_metropolis_end); zero before the first launch, self-resetting
     int64_t c_off;                  // global id of the chain in row 0 of params
     int64_t gen, zrow0;             // as mc3b_metropolis (gen < 0: device-driven)
     mc3b_sampler_t S;
@@ -106,37 +106,62 @@ static __device__ __noinline__ void fused_metropolis_step(const mc3b_sampler_t* 
 }
 
 // Hook between the sum of a chain's partial rows and its Metropolis step; called by
-// every thread of the reducer CTA (it may use CTA barriers).  recording(): the thread
-// whose arrival completes the launch calls record(g), g = generations completed, after
-// every group's hook has run.
+// every thread of the reducer CTA (it may use CTA barriers), it returns the CTA's count of
+// hits (chains it sent to another evaluation), the same in every thread.  counter(): where
+// the hits of every launch are added up (nullptr: not counted); recording(): the thread
+// whose arrival completes the launch calls record(g, hits), g = generations completed,
+// hits = the counter's new value.
 struct NoFix {
-    __device__ __forceinline__ void operator()(bool, int64_t, double&) const {}
+    __device__ __forceinline__ int operator()(bool, int64_t, double&) const { return 0; }
+    __device__ __forceinline__ int32_t* counter() const { return nullptr; }
     __device__ __forceinline__ bool recording() const { return false; }
-    __device__ __forceinline__ void record(int64_t) const {}
+    __device__ __forceinline__ void record(int64_t, int) const {}
 };
+// *fix.counter() read by thread 0 (the one that uses it), early in the launch
+template <class Fix>
+__device__ __forceinline__ int fix_count_base(const Fix& fix) {
+    const int32_t* c = fix.counter();
+    return threadIdx.x == 0 && c ? __ldcg(c) : 0;
+}
 
-// After every thread's step: the CTA counts its arrival, and the thread whose arrival completes
-// the launch records and bumps the generation counter.  gdev: *S.gen_dev as read earlier in the
-// launch (whenever f.advance is set); nothing else writes it while the launch runs.
+// After every thread's step: thread 0 of each CTA counts the CTA's arrival and its hits in one
+// 64-bit word, (arrivals << 32) | hits, at the first 8-byte-aligned slot of f.done after the
+// group counters; the CTA whose arrival completes the launch stores the hit counter, the
+// record, the generation counter and the word's reset.  base: *fix.counter() as thread 0 read it
+// earlier in the launch; gdev: *S.gen_dev as read earlier in the launch (whenever f.advance is
+// set).  Nothing else writes either while the launch runs.
+// No fence on one device: the values the last CTA stores are read only by later kernels or by
+// the host after the kernel ends, which the kernel boundary orders after every store of the
+// launch, and the one value that crosses CTAs within the launch, the hit count, travels in the
+// arrival atomic itself.  Every CTA consumed its load of *S.gen_dev before the barrier that
+// precedes its arrival, so the bump cannot overtake it.  Peer mode: the generation flags tell
+// the other devices that this device's peer stores are performed, so every CTA fences them at
+// system scope (cumulative over the barrier) before it arrives.
+// A launch without advance or record has no arrival: each CTA with hits adds them to the counter.
 template <class Fix>
 __device__ __forceinline__ void fused_metropolis_end(const FuseArgs& f, const mc3b_sampler_t& S, const Fix& fix,
-                                                     int64_t gen, int64_t gdev) {
+                                                     int64_t gen, int64_t gdev, int hits, int base) {
     __syncthreads();
-    const bool rec = fix.recording();              // false for NoFix: its code is unchanged
-    if (threadIdx.x == 0 && (f.advance || rec)) {
-        // one fence for the CTA's stores (cumulative over the barrier): system scope when they
-        // went to peer devices, so that the flag below needs no fence of its own
-        if (S.X_peers) __threadfence_system(); else __threadfence();
-        if (atomicAdd(&f.done[gridDim.x], 1) == (int)gridDim.x - 1) {
-            f.done[gridDim.x] = 0;
-            __threadfence();
-            if (rec) fix.record(gen + 1);
-            if (f.advance) {
-                const int64_t g = gdev + 1;
-                *S.gen_dev = g;
-                if (S.F_peers) flags_publish(S, g);      // every group's peer stores are performed
-            }
-        }
+    const bool rec = fix.recording();              // false for NoFix
+    int32_t* const count = fix.counter();          // nullptr for NoFix
+    if (threadIdx.x != 0) return;
+    if (!f.advance && !rec) {
+        if (count && hits) atomicAdd(count, hits);
+        return;
+    }
+    if (S.X_peers) __threadfence_system();
+    unsigned long long* word = reinterpret_cast<unsigned long long*>(f.done) + (gridDim.x + 1) / 2;
+    const unsigned long long own = (1ull << 32) + (uint32_t)hits;
+    const unsigned long long old = atomicAdd(word, own);
+    if ((uint32_t)(old >> 32) != gridDim.x - 1) return;
+    *word = 0;
+    const int total = base + (int)(uint32_t)(old + own);
+    if (count) *count = total;
+    if (rec) fix.record(gen + 1, total);
+    if (f.advance) {
+        const int64_t g = gdev + 1;
+        *S.gen_dev = g;
+        if (S.F_peers) flags_publish(S, g);          // every CTA's peer stores are performed
     }
 }
 
@@ -165,6 +190,7 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
         }
         return;
     }
+    const int base = fix_count_base(fix);
     if (threadIdx.x == 0) {
         sS = f.S;                                  // constant bank -> shared, static offsets only
         if (others > 0) {
@@ -210,9 +236,9 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
         inb = sS.inb[f.c_off + cl] != 0;
         if (inb) nxt = sum_partials<true>(partial, ldpartial, (int)gridDim.y, cl);
     }
-    fix(inb, cl, nxt);
+    const int hits = fix(inb, cl, nxt);
     if (mine) fused_metropolis_step(&sS, nxt, f.c_off + cl, gen, zrow0);
-    fused_metropolis_end(f, sS, fix, gen, gdev);
+    fused_metropolis_end(f, sS, fix, gen, gdev, hits, base);
 }
 
 // The one-split launch of k_spectral_chisq, whose thread t of CTA b owns chain b * WARPS * 32 + t,
@@ -224,20 +250,25 @@ __device__ __forceinline__ void fused_metropolis(const FuseArgs& f, const double
 struct FusedEntry {
     int64_t gen;                    // generation of the step (f.gen, or *gen_dev when device-driven)
     int64_t gdev;                   // *gen_dev when the launch bumps it or is device-driven
+    int base;                       // fix_count_base
     ChainState st;
 };
-__device__ __forceinline__ FusedEntry fused_metropolis_load(const FuseArgs& f, double* vbuf, int64_t cl) {
+template <class Fix>
+__device__ __forceinline__ FusedEntry fused_metropolis_load(const FuseArgs& f, const Fix& fix, double* vbuf,
+                                                            int64_t cl) {
     FusedEntry e;
     e.gdev = f.gen < 0 || f.advance ? *f.S.gen_dev : 0;
     e.gen = f.gen < 0 ? e.gdev : f.gen;
+    e.base = fix_count_base(fix);
     e.st = metropolis_load(f.S, e.gen, f.c_off + cl);
     stage_vectors_load<WARPS * 32>(f.S, vbuf, threadIdx.x);
     stage_peers_load(f.S, vbuf, threadIdx.x, WARPS * 32);
     return e;
 }
 // Every thread of the CTA, after its partial row is written: guard(act, nxt) is the Fix hook
-// (a CTA-wide call) with the chain's inputs already in registers; mine: the thread owns a chain,
-// whose only row is `row`, added from the register (0.0 + row: the bits of the split-order sum).
+// (a CTA-wide call, returning the CTA's hits) with the chain's inputs already in registers;
+// mine: the thread owns a chain, whose only row is `row`, added from the register (0.0 + row:
+// the bits of the split-order sum).
 template <class Fix, class Guard>
 __device__ __forceinline__ void fused_metropolis_apply(const FuseArgs& f, const FusedEntry& e, double* vbuf, int64_t cl,
                                                        bool mine, double row, const Fix& fix, Guard guard) {
@@ -249,9 +280,9 @@ __device__ __forceinline__ void fused_metropolis_apply(const FuseArgs& f, const 
     if (f.gen < 0) zrow0 = ((gen + 1) % S.thinning == 0) ? S.M0 + ((gen + 1) / S.thinning - 1) * S.nchains : -1;
     const bool inb = mine && e.st.inb != 0;
     double nxt = inb ? 0.0 + row : 0.0;
-    guard(inb, nxt);
+    const int hits = guard(inb, nxt);
     if (mine) metropolis_apply(S, e.st, nxt, gen, zrow0, f.c_off + cl);
-    fused_metropolis_end(f, S, fix, gen, e.gdev);
+    fused_metropolis_end(f, S, fix, gen, e.gdev, hits, e.base);
 }
 
 #ifndef __CUDACC_RTC__

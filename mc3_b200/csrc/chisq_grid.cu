@@ -326,17 +326,18 @@ __global__ void __launch_bounds__(128) k_fold_consts(const double* __restrict__ 
 // returns to k_sinefold<MOM=false> when it is not rare (high signal-to-noise data).
 struct MomentFix {
     const ChisqArgs<double>& a;
-    // `act`: this thread owns a chain whose proposal is inside the bounds; nxt = its data chi-squared
-    __device__ __forceinline__ void operator()(bool act, int64_t cl, double& nxt) const {
+    // `act`: this thread owns a chain whose proposal is inside the bounds; nxt = its data chi-squared.
+    // Returns the CTA's count of chains sent to the point-by-point evaluation.
+    __device__ __forceinline__ int operator()(bool act, int64_t cl, double& nxt) const {
         const double* p = a.params + cl * a.ldp;
         double pa = 0.0, pc = 0.0, ps = 0.0;
         if (act) { pa = p[0]; pc = p[3]; ps = p[4]; }
-        guard(act, p, pa, pc, ps, a.w[0], nxt);
+        return guard(act, p, pa, pc, ps, a.w[0], nxt);
     }
     // the same with the chain's amplitude, intercept and slope (p[0], p[3], p[4]; read when act)
     // and the weight w0 in registers
-    __device__ __forceinline__ void guard(bool act, const double* p, double pa, double pc, double ps, double w0,
-                                          double& nxt) const {
+    __device__ __forceinline__ int guard(bool act, const double* p, double pa, double pc, double ps, double w0,
+                                         double& nxt) const {
         const MomentArgs& m = a.m;
         bool bad = false;
         if (act) {
@@ -347,7 +348,8 @@ struct MomentFix {
             const double mag = (fabs(pa) + lmax) * sqrt(n) + sqrt(m.d2tot);
             bad = !(mag * mag * (w0 * w0) <= m.amp_max * nxt);        // NaN: exact path too
         }
-        if (!__syncthreads_or(bad)) return;
+        const int hits = __syncthreads_count(bad);
+        if (!hits) return 0;
         // rare: the flagged chains one at a time, in thread order, the whole CTA over the data
         __shared__ double prm[5], red[WARPS];
         __shared__ uint32_t mask[WARPS];
@@ -359,10 +361,8 @@ struct MomentFix {
             while (mk) {
                 const int t = w * 32 + __ffs(mk) - 1;
                 mk &= mk - 1;
-                if ((int)threadIdx.x == t) {
+                if ((int)threadIdx.x == t)
                     for (int j = 0; j < 5; j++) prm[j] = p[j];
-                    if (m.guard_hits) atomicAdd(m.guard_hits, 1);
-                }
                 __syncthreads();
                 const double amp = prm[0], k = 6.283185307179586476925287 / prm[1], ph = prm[2], c0 = prm[3], sl = prm[4];
                 double q = 0.0;
@@ -382,15 +382,14 @@ struct MomentFix {
                 __syncthreads();
             }
         }
+        return hits;
     }
+    __device__ __forceinline__ int32_t* counter() const { return a.m.guard_hits; }
     // Guard record of the fused epilogue (include/mc3b200.h mc3b_moment_t.record): the host reads
-    // the count of generation g without a copy on the stream.  Called after the fence that
-    // follows every group's arrival, so every hit of the launch (each counted before its CTA's
-    // barrier and fence) is in; one aligned 64-bit store, stamp in the high word.
+    // the count of generation g without a copy on the stream.  hits: guard_hits once every hit of
+    // the launch is in (fused_metropolis_end); one aligned 64-bit store, stamp in the high word.
     __device__ __forceinline__ bool recording() const { return a.m.record != nullptr; }
-    __device__ __forceinline__ void record(int64_t g) const {
-        int hits;
-        asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(hits) : "l"(a.m.guard_hits) : "memory");
+    __device__ __forceinline__ void record(int64_t g, int hits) const {
         const unsigned long long v = ((unsigned long long)(uint32_t)g << 32) | (uint32_t)hits;
         asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(a.m.record + (g & (MC3B_GUARD_RECORDS - 1))), "l"(v)
                      : "memory");
@@ -808,7 +807,8 @@ __global__ void __launch_bounds__(WARPS * 32) k_moment_finish(ChisqArgs<double> 
     double acc = 0.0;
     if (mine)
         for (int s = 0; s < nsplit; s++) acc += a.partial[(int64_t)s * a.ldpartial + c];
-    MomentFix{a}(mine, c, acc);
+    const int hits = MomentFix{a}(mine, c, acc);
+    if (threadIdx.x == 0 && hits && a.m.guard_hits) atomicAdd(a.m.guard_hits, hits);
     if (!mine) return;
     if (prior != nullptr) {
         double pr = 0.0;
@@ -991,8 +991,9 @@ __global__ void __maxnreg__(168) k_spectral_chisq(ChisqArgs<double> a) {
     const double amp = p[0], om = 6.283185307179586476925287 / p[1], ph = p[2], p3 = p[3], p4 = p[4];
 #ifndef MC3B_NO_FUSE_CODE
     __shared__ double vbuf[STAGE_DOUBLES];
+    const MomentFix fix{a};
     FusedEntry fe;
-    if (a.f.on) fe = fused_metropolis_load(a.f, vbuf, c);
+    if (a.f.on) fe = fused_metropolis_load(a.f, fix, vbuf, c);
 #endif
     const double b = p4 - m.slref;
     const double ac = fma(b, m.sxc, p3 - m.c0ref);             // L' at the centre
@@ -1034,11 +1035,10 @@ __global__ void __maxnreg__(168) k_spectral_chisq(ChisqArgs<double> a) {
     }
     if (live) a.partial[c] = q;
 #ifndef MC3B_NO_FUSE_CODE
-    if (a.f.on) {
-        const MomentFix fix{a};
-        fused_metropolis_apply(a.f, fe, vbuf, c, live, q, fix,
-                               [&](bool act, double& nxt) { fix.guard(act, p, amp, p3, p4, w0, nxt); });
-    }
+    if (a.f.on)
+        fused_metropolis_apply(a.f, fe, vbuf, c, live, q, fix, [&](bool act, double& nxt) {
+            return fix.guard(act, p, amp, p3, p4, w0, nxt);
+        });
 #endif
 }
 
