@@ -569,6 +569,37 @@ int mc3b_run_small(const mc3b_sampler_t* s, int model_id, int nmodel,
                    const double* x, const double* data, const double* invsig,
                    int64_t n, int64_t gen0, int64_t ngen, void* stream);
 
+/* Many independent small problems at once, one resident CTA each (a catalogue of
+ * fits on different data).  problems[b] describes problem b exactly as
+ * mc3b_run_small takes it (pointers into that problem's own slices of the state,
+ * its own seed, vectors and history); every problem has the nchains, npars, nfree,
+ * sampler, M0, zlen and thinning of problem 0.  Problem b owns the data points
+ * [offsets[b], offsets[b+1]) of x, data and invsig. */
+typedef struct mc3b_batch {
+    int64_t nproblems;
+    const mc3b_sampler_t* problems;   /* [nproblems], device memory: each problem's state (pointers into its slices) */
+    const int64_t* offsets;           /* [nproblems + 1], device: problem b owns points [offsets[b], offsets[b+1]) */
+    const double* x; const double* data; const double* invsig;
+    int32_t* status;                  /* [nproblems], device: 0 ok, 1 initial population not filled,
+                                         2 shape differs from problem 0's or no data points */
+} mc3b_batch_t;
+
+/* Initial population of every problem (mcmc_driver.py:229-278), one CTA per
+ * problem: the trial points of mc3b_init_trials (same Philox counters and kickoff
+ * rules), in rounds sized as Population.init_population sizes them (trials
+ * min(max(M0 - got, 64) 1.25 + 64, 100 M0 - tried); the first need + max(8, need/100)
+ * in-bounds ones evaluated, a warp per trial, chi-squared + prior terms; the first
+ * `need` with a finite log-posterior taken in draw order; at most 100 M0 trials).
+ * Writes Z[0:M0], log_post[0:M0], X = Z[0:nchains], chisq_cur = -2 log_post[0:nchains]
+ * and status[b].  model_id / nmodel / kickoff as mc3b_run_small / mc3b_init_trials. */
+int mc3b_batch_init(const mc3b_batch_t* b, int model_id, int nmodel, int kickoff, void* stream);
+
+/* mc3b_run_small over every problem whose status is 0, one CTA per problem
+ * (Chain.run, mc3/chain.py:183-299): generations gen0 .. gen0+ngen-1, the same
+ * arithmetic, bit for bit, as mc3b_run_small on that problem alone.  The per-problem
+ * gen_dev is ignored.  Split into launches of at most 200 000 generations. */
+int mc3b_batch_run(const mc3b_batch_t* b, int model_id, int nmodel, int64_t gen0, int64_t ngen, void* stream);
+
 /* Trial points of the initial population (mcmc_driver.py:229-262):
  * trial[t, :] = params0 with free entries drawn N(params0, pstep) (kickoff 0)
  * or U(pmin, pmax) (kickoff 1), shared parameters filled; ok[t] = 1 when all

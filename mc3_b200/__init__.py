@@ -12,10 +12,11 @@ through a C ABI (include/mc3b200.h) with ctypes.  There is no CPU fallback.
 from . import models
 from .models import BuiltinModel, CudaModel, TorchModel
 from .sampler_driver import sample, __version__
+from .batch_driver import sample_batch
 from .fit_driver import fit
 from . import stats
 from . import utils
 from .utils import Log
 
-__all__ = ['sample', 'fit', 'stats', 'utils', 'models', 'BuiltinModel',
+__all__ = ['sample', 'sample_batch', 'fit', 'stats', 'utils', 'models', 'BuiltinModel',
            'CudaModel', 'TorchModel', 'Log', '__version__']

@@ -44,6 +44,12 @@ class SamplerStruct(ctypes.Structure):
     ]
 
 
+class BatchStruct(ctypes.Structure):
+    """mc3b_batch_t."""
+    _fields_ = [('nproblems', c_i64), ('problems', c_vp), ('offsets', c_vp),
+                ('x', c_vp), ('data', c_vp), ('invsig', c_vp), ('status', c_vp)]
+
+
 class SpectralStruct(ctypes.Structure):
     """mc3b_spectral_t."""
     _fields_ = [('table', c_vp), ('w1', c_dbl), ('w2', c_dbl), ('delta', c_dbl), ('xc', c_dbl),
@@ -145,6 +151,8 @@ _SIGS = {
     'mc3b_advance': (c_int, [ctypes.POINTER(SamplerStruct), c_vp]),
     'mc3b_run_small': (c_int, [ctypes.POINTER(SamplerStruct), c_int, c_int, c_vp, c_vp, c_vp,
                                c_i64, c_i64, c_i64, c_vp]),
+    'mc3b_batch_init': (c_int, [ctypes.POINTER(BatchStruct), c_int, c_int, c_int, c_vp]),
+    'mc3b_batch_run': (c_int, [ctypes.POINTER(BatchStruct), c_int, c_int, c_i64, c_i64, c_vp]),
     'mc3b_init_trials': (c_int, [ctypes.POINTER(SamplerStruct), c_int, c_i64, c_i64,
                                  c_vp, c_vp, c_vp]),
     'mc3b_log_prior': (c_int, [c_vp, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,

@@ -92,26 +92,7 @@ __global__ void __launch_bounds__(128) k_init_trials(mc3b_sampler_t S, int kicko
                                                      double* trial, int32_t* ok) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= ntrials) return;
-    const Philox ph(S.seed);
-    double* v = trial + t * S.npars;
-    for (int k = 0; k < S.npars; k++) v[k] = S.params0[k];
-    int good = 1;
-    for (int j = 0; j < S.nfree; j += 2) {
-        const uint4 w = ph((uint32_t)t, (uint32_t)(j >> 1), (uint32_t)round, 0xFFFFFFFFu);
-        double d0, d1;
-        if (kickoff == 0) box_muller(u01(w.x, w.y), u01(w.z, w.w), d0, d1);
-        else { d0 = u01(w.x, w.y); d1 = u01(w.z, w.w); }
-        for (int q = 0; q < 2 && j + q < S.nfree; q++) {
-            const int k = S.ifree[j + q];
-            const double d = q ? d1 : d0;
-            v[k] = kickoff == 0 ? S.params0[k] + S.pstep[k] * d : S.pmin[k] + (S.pmax[k] - S.pmin[k]) * d;
-        }
-    }
-    for (int k = 0; k < S.npars; k++)
-        if (S.pstep[k] < 0.0) v[k] = v[-(int)S.pstep[k] - 1];
-    for (int k = 0; k < S.npars; k++)
-        if (v[k] > S.pmax[k] || v[k] < S.pmin[k]) good = 0;     // mcmc_driver.py:252
-    ok[t] = good;
+    ok[t] = init_trial(S, kickoff, t, round, trial + t * S.npars);
 }
 
 __global__ void k_advance(mc3b_sampler_t S) {

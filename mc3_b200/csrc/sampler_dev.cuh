@@ -1,5 +1,5 @@
 // mc3_b200 -- per-chain device functions of the sampler (shared by the
-// per-generation kernels of sampler.cu and the persistent kernel of small.cu).
+// per-generation kernels of sampler.cu and the persistent kernels of small.cu and batch.cu).
 #pragma once
 #include "common.cuh"
 
@@ -458,5 +458,30 @@ __device__ __forceinline__ void metropolis_chain(const mc3b_sampler_t& S, double
     metropolis_apply(S, metropolis_load(S, gen, c), nxt_data, gen, zrow0, c);
 }
 
+// Trial point t of round `round` of the initial population (mcmc_driver.py:229-262): v[0..npars)
+// = params0 with the free entries drawn N(params0, pstep) (kickoff 0) or U(pmin, pmax) (kickoff 1)
+// from Philox counter (t, slot, round, 0xFFFFFFFF), shared parameters filled.  Returns 1 when
+// every parameter is inside [pmin, pmax] (mcmc_driver.py:252).
+__device__ __forceinline__ int init_trial(const mc3b_sampler_t& S, int kickoff, int64_t t, int64_t round, double* v) {
+    const Philox ph(S.seed);
+    for (int k = 0; k < S.npars; k++) v[k] = S.params0[k];
+    int good = 1;
+    for (int j = 0; j < S.nfree; j += 2) {
+        const uint4 w = ph((uint32_t)t, (uint32_t)(j >> 1), (uint32_t)round, 0xFFFFFFFFu);
+        double d0, d1;
+        if (kickoff == 0) box_muller(u01(w.x, w.y), u01(w.z, w.w), d0, d1);
+        else { d0 = u01(w.x, w.y); d1 = u01(w.z, w.w); }
+        for (int q = 0; q < 2 && j + q < S.nfree; q++) {
+            const int k = S.ifree[j + q];
+            const double d = q ? d1 : d0;
+            v[k] = kickoff == 0 ? S.params0[k] + S.pstep[k] * d : S.pmin[k] + (S.pmax[k] - S.pmin[k]) * d;
+        }
+    }
+    for (int k = 0; k < S.npars; k++)
+        if (S.pstep[k] < 0.0) v[k] = v[-(int)S.pstep[k] - 1];
+    for (int k = 0; k < S.npars; k++)
+        if (v[k] > S.pmax[k] || v[k] < S.pmin[k]) good = 0;
+    return good;
+}
 
 }  // namespace

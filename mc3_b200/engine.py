@@ -55,6 +55,23 @@ def to_host(t):
     return buf.numpy()
 
 
+def column_statistics(blk, quantile=0.683):
+    """[5, cols] device tensor: median, mean, std and central-quantile bounds of every
+    column of blk [n, cols] (stats.py:764-802 'med_central'; numpy's linear percentile
+    rule, population std)."""
+    n = blk.shape[0]
+    srt, _ = torch.sort(blk, dim=0)
+
+    def pct(q):
+        pos = q*(n - 1)
+        i0 = int(np.floor(pos))
+        i1 = min(i0 + 1, n - 1)
+        fr = pos - i0
+        return srt[i0] + (srt[i1] - srt[i0])*fr
+    return torch.stack([pct(0.5), blk.mean(dim=0), blk.std(dim=0, unbiased=False),
+                        pct(0.5*(1 - quantile)), pct(0.5*(1 + quantile))])
+
+
 def on_device(fn):
     """Run a Population method with the population's device current: the C ABI
     launches on the current CUDA device and on its current stream."""
@@ -1133,19 +1150,7 @@ class Population:
         percentile rule) and fetched with one copy.  Sorting is torch.sort:
         post-processing, not the hot path."""
         lo, hi = self.M0 + zburn*self.nchains, self.zsize()
-        blk = self.Z[lo:hi]
-        n = blk.shape[0]
-        srt, _ = torch.sort(blk, dim=0)
-
-        def pct(q):
-            pos = q*(n - 1)
-            i0 = int(np.floor(pos))
-            i1 = min(i0 + 1, n - 1)
-            fr = pos - i0
-            return srt[i0] + (srt[i1] - srt[i0])*fr
-        out = torch.stack([pct(0.5), blk.mean(dim=0), blk.std(dim=0, unbiased=False),
-                           pct(0.5*(1 - quantile)), pct(0.5*(1 + quantile))]).cpu().numpy()
-        return tuple(out)
+        return tuple(column_statistics(self.Z[lo:hi], quantile).cpu().numpy())
 
     def gelman_rubin_async(self, zburn):
         """PSRF per free parameter over every chain's samples after burn-in

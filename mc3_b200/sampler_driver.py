@@ -41,33 +41,8 @@ def _need_array(value, name, log):
     return value
 
 
-def sample(data=None, uncert=None, func=None, params=None,
-           indparams=[], indparams_dict={},
-           pmin=None, pmax=None, pstep=None,
-           prior=None, priorlow=None, priorup=None,
-           sampler=None, ncpu=None, leastsq=None, chisqscale=False,
-           nchains=7, nsamples=None, burnin=0, thinning=1,
-           grtest=True, grbreak=0.0, grnmin=0.5, wlike=False,
-           fgamma=1.0, fepsilon=0.0, hsize=10, kickoff='normal',
-           plots=False, theme='blue', statistics='med_central',
-           ioff=False, showbp=True,
-           savefile=None, resume=False,
-           rms=False, log=None, pnames=None, texnames=None,
-           **kwargs):
-    if isinstance(log, str):
-        log = mu.Log(log, append=resume)
-        closelog = True
-    else:
-        closelog = False
-        if log is None:
-            log = mu.Log()
-
-    log.msg(
-        f"\n{log.sep}\n"
-        "  mc3_b200: B200-native Markov-chain Monte Carlo with the mc3 API.\n"
-        f"  Version {__version__} ({date.today().year}).\n"
-        f"{log.sep}\n\n")
-
+def check_sampler(sampler, nsamples, leastsq, log):
+    """The run options sample() checks first."""
     if sampler is None:
         log.error("'sampler' is a required argument")
     if nsamples is None and sampler in ['MRW', 'DEMC', 'snooker', 'mrw', 'demc']:
@@ -80,6 +55,11 @@ def sample(data=None, uncert=None, func=None, params=None,
         log.error(f"Invalid 'sampler' input ({sampler}). Must select from "
                   "['mrw', 'demc', 'snooker']")
 
+
+def read_arrays(params, data, uncert, pmin, pmax, pstep, prior, priorlow, priorup, log):
+    """params (or its 2-D file form), data and uncert as float arrays; returns (params,
+    data, uncert, pmin, pmax, pstep, prior, priorlow, priorup) with the vectors the 2-D
+    params form carries taken from it."""
     params = _need_array(params, 'params', log)
     if np.ndim(params) > 1:                       # sampler_driver.py:284-297
         ninfo = np.shape(params)[0]
@@ -102,20 +82,14 @@ def sample(data=None, uncert=None, func=None, params=None,
     uncert = np.array(uncert, dtype=float)        # a copy: never mutate the caller's
     data = np.asarray(data, dtype=float)
 
-    resume = resume and (savefile is not None)
-    if resume:
-        log.msg(f"\n\n{log.sep}\n{log.sep}  Resuming previous MCMC run.\n\n")
+    return params, data, uncert, pmin, pmax, pstep, prior, priorlow, priorup
 
-    if isinstance(func, (list, tuple, np.ndarray)):   # :320-327
-        sys.path.append(func[2] if len(func) == 3 else os.getcwd())
-        func = getattr(importlib.import_module(func[1]), func[0])
-    elif not callable(func):
-        log.error(
-            "'func' must be either a callable or an iterable of strings "
-            "with the model function, file, and path names")
 
+def fill_vectors(params, pnames, texnames, pmin, pmax, pstep, prior, priorlow, priorup, log):
+    """Names, default bounds, steps and priors, and the initial-guess bounds check;
+    returns (pnames, texnames, pmin, pmax, pstep, prior,
+    priorlow, priorup, nfree, ifree, ishare)."""
     nparams = len(params)
-    ndata = len(data)
     if pnames is None and texnames is not None:
         pnames = texnames
     elif pnames is not None and texnames is None:
@@ -150,6 +124,59 @@ def sample(data=None, uncert=None, func=None, params=None,
     nfree = int(np.sum(pstep > 0))
     ifree = np.where(pstep > 0)[0]
     ishare = np.where(pstep < 0)[0]
+
+    return pnames, texnames, pmin, pmax, pstep, prior, priorlow, priorup, nfree, ifree, ishare
+
+
+def sample(data=None, uncert=None, func=None, params=None,
+           indparams=[], indparams_dict={},
+           pmin=None, pmax=None, pstep=None,
+           prior=None, priorlow=None, priorup=None,
+           sampler=None, ncpu=None, leastsq=None, chisqscale=False,
+           nchains=7, nsamples=None, burnin=0, thinning=1,
+           grtest=True, grbreak=0.0, grnmin=0.5, wlike=False,
+           fgamma=1.0, fepsilon=0.0, hsize=10, kickoff='normal',
+           plots=False, theme='blue', statistics='med_central',
+           ioff=False, showbp=True,
+           savefile=None, resume=False,
+           rms=False, log=None, pnames=None, texnames=None,
+           **kwargs):
+    if isinstance(log, str):
+        log = mu.Log(log, append=resume)
+        closelog = True
+    else:
+        closelog = False
+        if log is None:
+            log = mu.Log()
+
+    log.msg(
+        f"\n{log.sep}\n"
+        "  mc3_b200: B200-native Markov-chain Monte Carlo with the mc3 API.\n"
+        f"  Version {__version__} ({date.today().year}).\n"
+        f"{log.sep}\n\n")
+
+    check_sampler(sampler, nsamples, leastsq, log)
+
+    (params, data, uncert, pmin, pmax, pstep, prior, priorlow, priorup) = read_arrays(
+        params, data, uncert, pmin, pmax, pstep, prior, priorlow, priorup, log)
+
+    resume = resume and (savefile is not None)
+    if resume:
+        log.msg(f"\n\n{log.sep}\n{log.sep}  Resuming previous MCMC run.\n\n")
+
+    if isinstance(func, (list, tuple, np.ndarray)):   # :320-327
+        sys.path.append(func[2] if len(func) == 3 else os.getcwd())
+        func = getattr(importlib.import_module(func[1]), func[0])
+    elif not callable(func):
+        log.error(
+            "'func' must be either a callable or an iterable of strings "
+            "with the model function, file, and path names")
+
+    nparams = len(params)
+    ndata = len(data)
+    (pnames, texnames, pmin, pmax, pstep, prior, priorlow, priorup, nfree, ifree,
+     ishare) = fill_vectors(params, pnames, texnames, pmin, pmax, pstep, prior, priorlow,
+                            priorup, log)
 
     fpar = params[0:-3] if wlike else params
     model0 = func(fpar, *indparams, **indparams_dict)     # :394-400
