@@ -537,8 +537,8 @@ int mc3b_metropolis(const mc3b_sampler_t* s, const double* partial,
  * one box).  mc3b_peer_alloc: zero-filled device buffer on the current device +
  * its 64-byte IPC handle [host].  mc3b_peer_open: map another process's buffer
  * into this one (peer access is enabled on demand); *ptr [host] receives the local
- * address.  mc3b_peer_close / mc3b_peer_free undo them.  These four and
- * mc3b_user_model_load are the only entry points that allocate. */
+ * address.  mc3b_peer_close / mc3b_peer_free undo them.  These four,
+ * mc3b_user_model_load and mc3b_user_batch_load are the only entry points that allocate. */
 int mc3b_peer_alloc(int64_t nbytes, void** ptr, unsigned char* handle64);
 int mc3b_peer_open(const unsigned char* handle64, void** ptr);
 int mc3b_peer_close(void* ptr);
@@ -599,6 +599,47 @@ int mc3b_batch_init(const mc3b_batch_t* b, int model_id, int nmodel, int kickoff
  * arithmetic, bit for bit, as mc3b_run_small on that problem alone.  The per-problem
  * gen_dev is ignored.  Split into launches of at most 200 000 generations. */
 int mc3b_batch_run(const mc3b_batch_t* b, int model_id, int nmodel, int64_t gen0, int64_t ngen, void* stream);
+
+/* The batch of a user model (mc3b_user_model_desc_t, fp64 only): k_init_batch, k_run_batch
+ * and a batched model-value kernel compiled by NVRTC into a module of their own, so that
+ * mc3b_user_model_compile_desc's module and compile time do not change.  A handle of one
+ * kind cannot be launched as the other.  Each launch takes, besides the batch:
+ *   xs [host]     nx == ninputs device pointers, input j of every problem concatenated as
+ *                 mc3b_batch_t.x is (problem b owns [offsets[b], offsets[b+1])), xs[0] == b->x
+ *   consts        [nproblems, nk] device, nk == nconst: problem b's constants in row b (the
+ *                 values its chains see in p[nmodel .. nmodel + nk)); NULL only when nk == 0
+ * and every problem has npars == nmodel.  mc3b_user_batch_compile / _load as
+ * mc3b_user_model_compile_desc / _load_desc (the module carries its own ABI record: one
+ * built against another sampler or batch layout is refused, MC3B_ERR_ARG). */
+typedef struct mc3b_user_batch mc3b_user_batch_t;          /* opaque */
+
+int mc3b_user_batch_compile(const char* nvrtc_path, const char* source,
+                            const mc3b_user_model_desc_t* desc /*[host]*/,
+                            void* cubin /*[host]*/, int64_t cap, int64_t* size /*[host]*/,
+                            char* log /*[host]*/, int64_t logcap);
+int mc3b_user_batch_load(const void* cubin /*[host]*/, int64_t size,
+                         const mc3b_user_model_desc_t* desc /*[host]*/,
+                         mc3b_user_batch_t** out /*[host]*/);
+int mc3b_user_batch_free(mc3b_user_batch_t* m);
+
+/* mc3b_batch_init for a user model (mcmc_driver.py:229-278, one CTA per problem). */
+int mc3b_user_batch_init(const mc3b_user_batch_t* m, const mc3b_batch_t* b,
+                         const double* const* xs /*[host] nx device pointers*/, int nx,
+                         const double* consts, int nk, int kickoff, void* stream);
+
+/* mc3b_batch_run for a user model (Chain.run, mc3/chain.py:183-299): launches of at most
+ * 200 000 generations. */
+int mc3b_user_batch_run(const mc3b_user_batch_t* m, const mc3b_batch_t* b,
+                        const double* const* xs /*[host] nx device pointers*/, int nx,
+                        const double* consts, int nk, int64_t gen0, int64_t ngen, void* stream);
+
+/* mc3b_model_eval for a user model and every problem of a batch in one launch (the
+ * best_model of each output dictionary): out[i] = model(params + b * ldp) at point i of
+ * problem b, for i in [offsets[b], offsets[b+1]); out has the layout of b->x. */
+int mc3b_user_batch_eval(const mc3b_user_batch_t* m, const mc3b_batch_t* b,
+                         const double* const* xs /*[host] nx device pointers*/, int nx,
+                         const double* consts, int nk, const double* params, int64_t ldp,
+                         double* out, void* stream);
 
 /* Trial points of the initial population (mcmc_driver.py:229-262):
  * trial[t, :] = params0 with free entries drawn N(params0, pstep) (kickoff 0)

@@ -1,13 +1,15 @@
 """Many independent small fits at once: sample_batch() runs B problems of the same
 shape (a catalogue of light curves, one fit per star, transit or band) in one
-launch, one persistent CTA per problem (csrc/batch.cu).  Problem b is
+launch, one persistent CTA per problem (csrc/batch_dev.cuh).  Problem b is
 
     sample(data[b], uncert[b], func, params[b], indparams[b], ...)
 
 with the problem's own seed, and its output dictionary has the keys and meaning of
-sample()'s.  What the batch shares: the model (a built-in, fp64), the sampler and its
-options, and the pattern of free, shared and fixed parameters.  It writes no files
-and no log output.
+sample()'s.  What the batch shares: the model (a built-in or a CudaModel, fp64), the
+sampler and its options, and the pattern of free, shared and fixed parameters.  A
+CudaModel's per-point inputs and run-time constants are the problem's own: indparams[b]
+is read as sample() reads it (CudaModel.split_args), and the kernels are those of the
+model's batch module (CudaModel.batch_handle).  It writes no files and no log output.
 """
 import ctypes
 
@@ -17,7 +19,7 @@ import torch
 from . import _lib
 from . import stats as ms
 from .engine import column_statistics, to_host
-from .models import BuiltinModel
+from .models import BuiltinModel, CudaModel
 from .sampler_driver import check_sampler, read_arrays, fill_vectors
 
 MAX_CHAINS = 256                  # SW * 32 threads of mc3b_batch_run's CTA
@@ -65,19 +67,22 @@ def sample_batch(data, uncert, func, params, indparams,
 
     data, uncert  sequences of B 1-D arrays (lengths may differ between problems)
     params        [B, npars]
-    indparams     sequence of B lists [x_b], as sample() takes them
+    indparams     sequence of B lists, as sample() takes them: [x_b] for a built-in model;
+                  for a CudaModel its ninputs arrays of data[b]'s shape, then its nconst
+                  constants (they may differ between problems)
     pmin, pmax, pstep, prior, priorlow, priorup
                   [npars] shared by all problems, or [B, npars]; the sign pattern of
                   pstep (free / fixed / shared) must be the same for every problem
-    func          a BuiltinModel (polynomial, sinusoid, gaussian, box), fp64
+    func          a BuiltinModel (polynomial, sinusoid, gaussian, box) or a CudaModel, fp64
     seed          int s (problem b takes s + b), B ints, or None (one drawn as sample()
                   draws it, then s + b)
     The other options mean what they mean in sample(); nchains <= 256.  _state=True
     returns the device state after the generations instead (for tests)."""
     check_sampler(sampler, nsamples, None, _Log0())
-    if not isinstance(func, BuiltinModel):
+    if not isinstance(func, (BuiltinModel, CudaModel)):
         raise ValueError('sample_batch needs a built-in model (mc3_b200.models.polynomial, sinusoid, '
-                         f'gaussian or box), got {func!r}')
+                         f'gaussian or box) or a CudaModel, got {func!r}')
+    user = isinstance(func, CudaModel)
     if wlike or dtype != 'f64':
         raise ValueError('sample_batch runs the fp64 chi-squared likelihood only (no wlike, no f32)')
     nchains, thinning, hsize = int(nchains), int(thinning), int(hsize)
@@ -115,17 +120,22 @@ def sample_batch(data, uncert, func, params, indparams,
             vecs['prior'][b], vecs['priorlow'][b], vecs['priorup'][b], log)
         (pn, tn, lo, hi, st, pr, plo, pup, nfree, ifree, ishare) = fill_vectors(
             p, pnames, texnames, lo, hi, st, pr, plo, pup, log)
-        x = np.asarray(indparams[b][0], dtype=float) if np.iterable(indparams[b]) and len(indparams[b]) else None
-        if x is None or len(indparams[b]) != 1 or x.ndim != 1:
-            log.error('built-in models need indparams=[x] with the same shape as data')
-        if np.shape(x) != np.shape(d):                       # a built-in model returns x's shape
-            log.error(f"The size of the data array ({np.size(d)}) does not "
-                      f"match the size of the func() output ({np.size(x)})")
+        if user:
+            xs, k = _user_inputs(func, indparams[b], d, log)
+            x = xs[0]
+        else:
+            x = np.asarray(indparams[b][0], dtype=float) if np.iterable(indparams[b]) and len(indparams[b]) else None
+            if x is None or len(indparams[b]) != 1 or x.ndim != 1:
+                log.error('built-in models need indparams=[x] with the same shape as data')
+            if np.shape(x) != np.shape(d):                       # a built-in model returns x's shape
+                log.error(f"The size of the data array ({np.size(d)}) does not "
+                          f"match the size of the func() output ({np.size(x)})")
+            xs, k = [x], None
         try:
             func.nmodel(p.size)
         except ValueError as e:
             log.error(str(e))
-        probs.append(dict(params=p, data=d, uncert=u, x=x, pmin=lo, pmax=hi, pstep=st, prior=pr,
+        probs.append(dict(params=p, data=d, uncert=u, x=x, xs=xs, consts=k, pmin=lo, pmax=hi, pstep=st, prior=pr,
                           priorlow=plo, priorup=pup, pnames=pn, texnames=tn, ifree=ifree, ishare=ishare))
     npars = probs[0]['params'].size
     def pattern(q):                                 # which parameters are free, fixed, shared with which
@@ -162,7 +172,8 @@ def sample_batch(data, uncert, func, params, indparams,
         dev = torch.device('cuda', torch.cuda.current_device())
     with torch.cuda.device(dev):
         sizes = np.array([q['data'].size for q in probs], dtype=np.int64)
-        need = _state_bytes(B, nchains, npars, nfree, zlen, int(sizes.sum()))
+        need = _state_bytes(B, nchains, npars, nfree, zlen, int(sizes.sum()), len(probs[0]['xs']),
+                            func.nconst if user else 0)
         free = torch.cuda.mem_get_info(dev)[0]
         if need > free:
             raise ValueError(f'the state of {B} problems needs {need} bytes of device memory, '
@@ -176,6 +187,24 @@ def sample_batch(data, uncert, func, params, indparams,
         return run.outputs(func, zburn, nzchain, probs)
 
 
+def _user_inputs(func, args, d, log):
+    """(per-point arrays, constants [nconst]) of a CudaModel's indparams for data d, as
+    sample() reads them (CudaModel.split_args); errors name the problem through log."""
+    if not np.iterable(args) or isinstance(args, (str, bytes)):
+        log.error(f'{func.name} needs indparams=[x1, ..., x{func.ninputs}, constants...] per problem')
+    try:
+        xs, k = func.split_args(list(args))
+    except ValueError as e:
+        log.error(str(e))
+    if len(xs) != func.ninputs:
+        log.error(f'{func.name} takes {func.ninputs} input array(s), got {len(xs)}')
+    xs = [np.asarray(a, dtype=float) for a in xs]
+    for j, a in enumerate(xs):
+        if a.shape != np.shape(d):
+            log.error(f'input {j} of {func.name} has shape {a.shape}, the data {np.shape(d)}')
+    return xs, np.zeros(0) if k is None else k
+
+
 class _Log0:
     """sample()'s run-option checks raise as they do there, without log output."""
 
@@ -183,11 +212,12 @@ class _Log0:
         raise exception(message)
 
 
-def _state_bytes(B, nchains, npars, nfree, zlen, ntot):
-    """Device bytes of the batched state (history, per-chain arrays, data) and of the
-    post-processing copies of the history (chi-squared column)."""
+def _state_bytes(B, nchains, npars, nfree, zlen, ntot, ninputs=1, nconst=0):
+    """Device bytes of the batched state (history, per-chain arrays, data, a CudaModel's
+    further inputs and constants) and of the post-processing copies of the history
+    (chi-squared column)."""
     per = zlen*(nfree*8 + 8 + 4 + 8) + nchains*(2*nfree*8 + npars*8 + 4*8 + 2*4) + nfree*4 + 7*npars*8
-    return B*per + 3*ntot*8
+    return B*per + 3*ntot*8 + (ninputs - 1)*ntot*8 + B*nconst*8
 
 
 class _BatchRun:
@@ -206,6 +236,11 @@ class _BatchRun:
         self.off = off
         cat = lambda k: torch.from_numpy(np.concatenate([q[k] for q in probs])).to(dev)  # noqa: E731
         self.d_x, self.d_data = cat('x'), cat('data')
+        # a CudaModel's inputs 2..ninputs, concatenated as x, and its constants [B, nconst]
+        self.d_xs = [self.d_x] + [torch.from_numpy(np.concatenate([q['xs'][j] for q in probs])).to(dev)
+                                  for j in range(1, len(probs[0]['xs']))]
+        k = np.stack([q['consts'] for q in probs]) if probs[0]['consts'] is not None else None
+        self.d_consts = torch.from_numpy(k).to(dev) if k is not None and k.size else None
         self.d_invsig = 1.0/cat('uncert')
         self.d_off = torch.from_numpy(off).to(dev)
         stack = lambda k: torch.from_numpy(np.stack([q[k] for q in probs])).to(dev)  # noqa: E731
@@ -260,11 +295,20 @@ class _BatchRun:
         S.status = self.status.data_ptr()
         self.S = S
 
+    def _extra(self, func):
+        """(xs, nx, consts, nk) of the mc3b_user_batch_* entry points."""
+        return _lib.ptrs(self.d_xs), len(self.d_xs), _lib.ptr(self.d_consts), func.nconst
+
     def init(self, kickoff, func):
-        """Initial population of every problem (mc3b_batch_init); the problems that could
-        not be populated raise the reference's error."""
-        _lib.call('mc3b_batch_init', ctypes.byref(self.S), func.model_id, func.nmodel(self.npars),
-                  {'normal': 0, 'uniform': 1}[kickoff], _lib.stream_ptr())
+        """Initial population of every problem (mc3b_batch_init, mc3b_user_batch_init); the
+        problems that could not be populated raise the reference's error."""
+        k = {'normal': 0, 'uniform': 1}[kickoff]
+        if isinstance(func, CudaModel):
+            _lib.call('mc3b_user_batch_init', func.batch_handle(), ctypes.byref(self.S), *self._extra(func), k,
+                      _lib.stream_ptr())
+        else:
+            _lib.call('mc3b_batch_init', ctypes.byref(self.S), func.model_id, func.nmodel(self.npars), k,
+                      _lib.stream_ptr())
         bad = np.flatnonzero(self.status.cpu().numpy())
         if bad.size:
             who = f'problem {bad[0]}' if bad.size == 1 else 'problems ' + ', '.join(str(b) for b in bad)
@@ -275,8 +319,12 @@ class _BatchRun:
                 'non-finite values.')
 
     def run(self, ngen, func):
-        _lib.call('mc3b_batch_run', ctypes.byref(self.S), func.model_id, func.nmodel(self.npars),
-                  0, ngen, _lib.stream_ptr())
+        if isinstance(func, CudaModel):
+            _lib.call('mc3b_user_batch_run', func.batch_handle(), ctypes.byref(self.S), *self._extra(func), 0, ngen,
+                      _lib.stream_ptr())
+        else:
+            _lib.call('mc3b_batch_run', ctypes.byref(self.S), func.model_id, func.nmodel(self.npars),
+                      0, ngen, _lib.stream_ptr())
 
     def outputs(self, func, zburn, nzchain, probs):
         """Output dictionaries (mcmc_driver.update_output + sample()'s statistics)."""
@@ -315,10 +363,14 @@ class _BatchRun:
         model = torch.empty(int(self.off[-1]), dtype=torch.float64, device=dev)
         nmodel = func.nmodel(npars)
         st = _lib.stream_ptr()
-        for b in range(B):
-            o, k = int(self.off[b]), int(self.off[b + 1] - self.off[b])
-            _lib.call('mc3b_model_eval', func.model_id, bestp[b].data_ptr(), npars, 1, nmodel,
-                      self.d_x[o:].data_ptr(), k, model[o:].data_ptr(), st)
+        if isinstance(func, CudaModel):                 # every problem in one launch
+            _lib.call('mc3b_user_batch_eval', func.batch_handle(), ctypes.byref(self.S), *self._extra(func),
+                      bestp.data_ptr(), npars, model.data_ptr(), st)
+        else:
+            for b in range(B):
+                o, k = int(self.off[b]), int(self.off[b + 1] - self.off[b])
+                _lib.call('mc3b_model_eval', func.model_id, bestp[b].data_ptr(), npars, 1, nmodel,
+                          self.d_x[o:].data_ptr(), k, model[o:].data_ptr(), st)
 
         # chi-squared column: -2 (log_post - log_prior) of every history row
         K = nzchain

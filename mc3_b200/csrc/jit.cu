@@ -16,6 +16,10 @@
 // The headers NVRTC needs are embedded in the library (jit_headers.inc, written by
 // build.py), so nothing reads the source tree at run time.  NVRTC itself is dlopen'ed
 // from the path the caller gives: nothing links against it.
+//
+// sample_batch takes a model's batch module (mc3b_user_batch_*) instead: the kernels of
+// batch_dev.cuh over the same wrapper, fp64, compiled by a program of their own
+// (batch_source), so that a sample() user compiles and loads neither more nor other code.
 #include <dlfcn.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -24,6 +28,7 @@
 #include <mutex>
 #include <string>
 #include <vector>
+#include "batch_dev.cuh"
 #include "chisq_args.cuh"
 #include "dwt_kernel.cuh"
 #include "jit_headers.inc"
@@ -159,6 +164,24 @@ constexpr long long kDwtArgsSizes =
 enum { ABI_VERSION, ABI_ARGS_SIZE, ABI_DTYPE, ABI_NMODEL, ABI_WARPS, ABI_TILE, ABI_NINPUTS, ABI_NCONST, ABI_NWORK,
        ABI_PREPARE, ABI_DWT_ARGS, ABI_N };
 
+// The batch module of an fp64 user model (batch_dev.cuh): [0] k_init_batch, [1] k_run_batch,
+// [2] k_batch_eval, over the wrapper of wrapper_expr.
+std::string batch_expr(const Desc& d, int k) {
+    static const char* const name[3] = {"k_init_batch", "k_run_batch", "k_batch_eval"};
+    return std::string("mc3b_jit::") + name[k] + "<" + wrapper_expr(d) + ">";
+}
+std::string batch_symbol(const Desc& d, int k) {
+    const std::string w = wrapper_symbol(d);
+    if (k == 0) return "_ZN8mc3b_jit12k_init_batchINS_" + w + "EEEv10mc3b_batchiiiiNS_10BatchExtraE";
+    if (k == 1) return "_ZN8mc3b_jit11k_run_batchINS_" + w + "EEEv10mc3b_batchiiillNS_10BatchExtraE";
+    return "_ZN8mc3b_jit12k_batch_evalINS_" + w + "EEEvPKdl10mc3b_batchNS_10BatchExtraEPd";
+}
+
+// What a batch module reports about itself (mc3b_jit_batch_abi), checked at load: a module
+// built against another sampler or batch layout is compiled again, never launched.
+enum { BABI_VERSION, BABI_SAMPLER_SIZE, BABI_BATCH_SIZE, BABI_WARPS, BABI_NMODEL, BABI_NINPUTS, BABI_NCONST,
+       BABI_NWORK, BABI_PREPARE, BABI_N };
+
 // The user's source in its namespace, with `real` defined and line numbers of model.cu.
 std::string user_unit(const char* user, int dtype) {
     std::string s;
@@ -170,10 +193,11 @@ std::string user_unit(const char* user, int dtype) {
     return s;
 }
 
-// Translation unit around the user's source; model_line / prepare_line: the lines of
-// `model` and `prepare` in it.
-std::string jit_source(const char* user, const Desc& d, int model_line, int prepare_line) {
-    std::string s = "#include \"dwt_kernel.cuh\"\n" + user_unit(user, d.dtype);
+// The user's model behind the interface of the built-in ones, after user_unit: the calls
+// of `model` and `prepare` (reported at model_line / prepare_line of model.cu) and the
+// wrapper of wrapper_expr in namespace mc3b_jit.
+std::string wrapper_source(const Desc& d, int model_line, int prepare_line) {
+    std::string s;
     const int ninputs = d.ninputs;
     if (ninputs > 1) {
         // the call of the wrapper, reported at the line of `model`: a model of another
@@ -250,12 +274,35 @@ std::string jit_source(const char* user, const Desc& d, int model_line, int prep
              "};\n";
     }
     s += "}  // namespace mc3b_jit\n";
+    return s;
+}
+
+// Translation unit around the user's source; model_line / prepare_line: the lines of
+// `model` and `prepare` in it.
+std::string jit_source(const char* user, const Desc& d, int model_line, int prepare_line) {
+    std::string s = "#include \"dwt_kernel.cuh\"\n" + user_unit(user, d.dtype);
+    s += wrapper_source(d, model_line, prepare_line);
+    const int ninputs = d.ninputs;
     char b[480];
     snprintf(b, sizeof(b),
              "extern \"C\" __device__ long long mc3b_jit_abi[%d] = {MC3B_VERSION, sizeof(ChisqArgs<mc3b_user::real>), "
              "%d, %d, WARPS, tilecfg<mc3b_user::real>::TILE, %d, %d, %d, %d, (long long)sizeof(mc3b_jit::RegArgsX) | "
              "(long long)sizeof(mc3b_jit::PassArgsX) << 16 | (long long)sizeof(mc3b_jit::LastArgsX) << 32};\n",
              (int)ABI_N, d.dtype, d.nmodel, ninputs, d.nconst, d.nwork, d.prepare ? 1 : 0);
+    s += b;
+    return s;
+}
+
+// Translation unit of the batch module: the batched kernels, the user's source and the
+// wrapper of jit_source, and the module's ABI record.
+std::string batch_source(const char* user, const Desc& d, int model_line, int prepare_line) {
+    std::string s = "#include \"batch_dev.cuh\"\n" + user_unit(user, d.dtype);
+    s += wrapper_source(d, model_line, prepare_line);
+    char b[320];
+    snprintf(b, sizeof(b),
+             "extern \"C\" __device__ long long mc3b_jit_batch_abi[%d] = {MC3B_VERSION, sizeof(mc3b_sampler_t), "
+             "sizeof(mc3b_batch_t), SW, %d, %d, %d, %d, %d};\n",
+             (int)BABI_N, d.nmodel, d.ninputs, d.nconst, d.nwork, d.prepare ? 1 : 0);
     s += b;
     return s;
 }
@@ -405,11 +452,16 @@ int check_desc(const mc3b_user_model_desc_t* d) {
 }
 }  // namespace
 
-extern "C" int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* source,
-                                            const mc3b_user_model_desc_t* desc, void* cubin, int64_t cap,
-                                            int64_t* size, char* log, int64_t logcap) {
+namespace {
+// The two modules of a user model: the sampler's kernels (jit_source) and the batch's (batch_source).
+enum Kind { KIND_CHISQ, KIND_BATCH };
+
+// source -> the CUBIN of one module, with the checks of mc3b_user_model_compile_desc
+int compile_module(Kind kind, const char* nvrtc_path, const char* source, const mc3b_user_model_desc_t* desc,
+                   void* cubin, int64_t cap, int64_t* size, char* log, int64_t logcap) {
     MC3B_CHECK_ARG(nvrtc_path && source && size, "null pointer");
     if (int rc = check_desc(desc)) return rc;
+    MC3B_CHECK_ARG(kind != KIND_BATCH || desc->dtype == MC3B_F64, "the batch module of a user model is fp64 only");
     MC3B_CHECK_ARG(cap >= 0 && (cap == 0 || cubin != nullptr), "bad CUBIN buffer");
     Desc d = {desc->nmodel, desc->ninputs, desc->nconst, desc->nwork, desc->dtype, false};
     *size = 0;
@@ -435,21 +487,29 @@ extern "C" int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* 
         return MC3B_ERR_ARG;
     }
 
-    const std::string src = jit_source(source, d, line, pline);
+    const std::string src =
+        kind == KIND_CHISQ ? jit_source(source, d, line, pline) : batch_source(source, d, line, pline);
     nvrtcProgram_t prog = nullptr;
     int r = nv->create(&prog, src.c_str(), "mc3b_user_model.cu", kJitNHeaders, kJitHeaderSources, kJitHeaderNames);
     if (r != 0) { mc3b_set_error("nvrtcCreateProgram: %s", nv->error_string(r)); return MC3B_ERR_CUDA; }
     std::vector<std::string> exprs, symbols;
-    for (int u = 0; u < 2; u++)
-        for (int l = 0; l < 3; l++) {
-            exprs.push_back(chisq_expr(d, kLC[l], u == 1));
-            symbols.push_back(chisq_symbol(d, kLC[l], u == 1));
+    if (kind == KIND_BATCH) {
+        for (int k = 0; k < 3; k++) {
+            exprs.push_back(batch_expr(d, k));
+            symbols.push_back(batch_symbol(d, k));
         }
-    exprs.push_back(eval_expr(d));
-    symbols.push_back(eval_symbol(d));
-    for (int k = 0; d.dtype == MC3B_F64 && k < 3; k++) {
-        exprs.push_back(dwt_expr(d, k));
-        symbols.push_back(dwt_symbol(d, k));
+    } else {
+        for (int u = 0; u < 2; u++)
+            for (int l = 0; l < 3; l++) {
+                exprs.push_back(chisq_expr(d, kLC[l], u == 1));
+                symbols.push_back(chisq_symbol(d, kLC[l], u == 1));
+            }
+        exprs.push_back(eval_expr(d));
+        symbols.push_back(eval_symbol(d));
+        for (int k = 0; d.dtype == MC3B_F64 && k < 3; k++) {
+            exprs.push_back(dwt_expr(d, k));
+            symbols.push_back(dwt_symbol(d, k));
+        }
     }
     for (const std::string& e : exprs) nv->add_name(prog, e.c_str());
     r = nv->compile(prog, 5, kOpts);
@@ -480,6 +540,13 @@ extern "C" int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* 
     }
     nv->destroy(&prog);
     return rc;
+}
+}  // namespace
+
+extern "C" int mc3b_user_model_compile_desc(const char* nvrtc_path, const char* source,
+                                            const mc3b_user_model_desc_t* desc, void* cubin, int64_t cap,
+                                            int64_t* size, char* log, int64_t logcap) {
+    return compile_module(KIND_CHISQ, nvrtc_path, source, desc, cubin, cap, size, log, logcap);
 }
 
 extern "C" int mc3b_user_model_compile_ex(const char* nvrtc_path, const char* source, int nmodel, int ninputs,
@@ -717,4 +784,158 @@ extern "C" int mc3b_user_model_dwt_chisq(const mc3b_user_model_t* m, const doubl
     const DwtUserModel u = {(const void*)m->dwt[0], (const void*)m->dwt[1], (const void*)m->dwt[2], nx, m->d.nmodel,
                             xs, consts};
     return mc3b_dwt_chisq_user(u, params, ldp, nchains, npars, data, n, workspace, chisq, (cudaStream_t)stream);
+}
+
+// ---- the batch module of a user model (mc3b_user_batch_*) -------------------------------
+struct mc3b_user_batch {
+    cudaLibrary_t lib;
+    cudaKernel_t init, run, eval;  // batch_expr's kernels
+    Desc d;
+    std::vector<char> image;       // the CUBIN, kept for the lifetime of the library
+};
+
+extern "C" int mc3b_user_batch_compile(const char* nvrtc_path, const char* source, const mc3b_user_model_desc_t* desc,
+                                       void* cubin, int64_t cap, int64_t* size, char* log, int64_t logcap) {
+    return compile_module(KIND_BATCH, nvrtc_path, source, desc, cubin, cap, size, log, logcap);
+}
+
+extern "C" int mc3b_user_batch_load(const void* cubin, int64_t size, const mc3b_user_model_desc_t* desc,
+                                    mc3b_user_batch_t** out) {
+    MC3B_CHECK_ARG(cubin && out && size >= 64, "bad arguments");
+    MC3B_CHECK_ARG(memcmp(cubin, "\x7f" "ELF", 4) == 0, "not a CUBIN (no ELF header)");
+    if (int rc = check_desc(desc)) return rc;
+    MC3B_CHECK_ARG(desc->dtype == MC3B_F64, "the batch module of a user model is fp64 only");
+    mc3b_user_batch* m = new mc3b_user_batch();
+    m->image.assign((const char*)cubin, (const char*)cubin + size);
+    m->d = Desc{desc->nmodel, desc->ninputs, desc->nconst, desc->nwork, desc->dtype, false};
+    cudaError_t e = cudaLibraryLoadData(&m->lib, m->image.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+    if (e != cudaSuccess) {
+        delete m;
+        mc3b_set_error("cudaLibraryLoadData: %s", cudaGetErrorString(e));
+        return MC3B_ERR_CUDA;
+    }
+    auto fail = [&](int rc) { cudaLibraryUnload(m->lib); delete m; return rc; };
+    // ABI guard, as mc3b_user_model_load_desc's: a stale cached module is refused
+    void* dabi = nullptr;
+    size_t bytes = 0;
+    long long abi[BABI_N] = {};
+    e = cudaLibraryGetGlobal(&dabi, &bytes, m->lib, "mc3b_jit_batch_abi");
+    if (e == cudaSuccess && bytes == sizeof(abi)) e = cudaMemcpy(abi, dabi, sizeof(abi), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess || bytes != sizeof(abi)) {
+        cudaGetLastError();                         // a missing symbol must not fail a later launch check
+        mc3b_set_error("the module has no batch ABI record (%s)", e != cudaSuccess ? cudaGetErrorString(e) : "size");
+        return fail(e != cudaSuccess ? MC3B_ERR_CUDA : MC3B_ERR_ARG);
+    }
+    const long long want[BABI_N] = {MC3B_VERSION, (long long)sizeof(mc3b_sampler_t), (long long)sizeof(mc3b_batch_t),
+                                    SW, desc->nmodel, desc->ninputs, desc->nconst, desc->nwork,
+                                    abi[BABI_PREPARE] == 1 || desc->nwork > 0 ? 1 : 0};
+    for (int i = 0; i < BABI_N; i++) {
+        if (abi[i] != want[i]) {
+            mc3b_set_error("the batch module does not match this library (ABI entry %d: %lld, expected %lld): "
+                           "compile it again", i, abi[i], want[i]);
+            return fail(MC3B_ERR_ARG);
+        }
+    }
+    m->d.prepare = abi[BABI_PREPARE] == 1;
+    cudaKernel_t* k[3] = {&m->init, &m->run, &m->eval};
+    for (int i = 0; i < 3; i++) {
+        e = cudaLibraryGetKernel(k[i], m->lib, batch_symbol(m->d, i).c_str());
+        if (e != cudaSuccess) { mc3b_set_error("cudaLibraryGetKernel: %s", cudaGetErrorString(e)); return fail(MC3B_ERR_CUDA); }
+    }
+    // k_run_batch takes up to 200 KB of dynamic shared memory (mc3b_user_batch_run): set here,
+    // once per device, so that no launch has to
+    int ndev = 0;
+    e = cudaGetDeviceCount(&ndev);
+    for (int dev = 0; e == cudaSuccess && dev < ndev; dev++)
+        e = cudaKernelSetAttributeForDevice(m->run, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024, dev);
+    if (e != cudaSuccess) { mc3b_set_error("k_run_batch shared memory: %s", cudaGetErrorString(e)); return fail(MC3B_ERR_CUDA); }
+    *out = m;
+    return MC3B_OK;
+}
+
+extern "C" int mc3b_user_batch_free(mc3b_user_batch_t* m) {
+    if (m == nullptr) return MC3B_OK;
+    const cudaError_t e = cudaLibraryUnload(m->lib);
+    delete m;
+    MC3B_CUDA(e);
+    return MC3B_OK;
+}
+
+namespace {
+// The inputs and constants of a launch against the module: nx == ninputs with xs[0] == b->x,
+// nk == nconst (consts may be NULL only when it is 0) -> the kernels' BatchExtra.
+int batch_extra(const mc3b_user_batch_t* m, const mc3b_batch_t* b, const double* const* xs, int nx,
+                const double* consts, int nk, BatchExtra* X) {
+    MC3B_CHECK_ARG(m && b && xs, "null pointer");
+    MC3B_CHECK_ARG(nx == m->d.ninputs, "this model takes %d inputs, got %d", m->d.ninputs, nx);
+    MC3B_CHECK_ARG(nk == m->d.nconst, "this model takes %d constants, got %d", m->d.nconst, nk);
+    MC3B_CHECK_ARG(consts || nk == 0, "null pointer (constants)");
+    MC3B_CHECK_ARG(xs[0] == b->x, "xs[0] must be the batch's x");
+    *X = BatchExtra{};
+    for (int j = 1; j < nx; j++) {
+        MC3B_CHECK_ARG(xs[j], "null pointer (input %d)", j);
+        X->xe[j - 1] = xs[j];
+    }
+    X->consts = consts;
+    X->nk = nk;
+    return MC3B_OK;
+}
+
+// mc3b_batch_shape, and the parameter count of the module
+int user_batch_shape(const mc3b_user_batch_t* m, const mc3b_batch_t* b, mc3b_sampler_t* s, cudaStream_t st) {
+    if (int rc = mc3b_batch_shape(b, s, st)) return rc;
+    MC3B_CHECK_ARG(s->npars == m->d.nmodel, "this model takes %d parameters, the problems have %d", m->d.nmodel,
+                   s->npars);
+    return MC3B_OK;
+}
+}  // namespace
+
+extern "C" int mc3b_user_batch_init(const mc3b_user_batch_t* m, const mc3b_batch_t* b, const double* const* xs, int nx,
+                                    const double* consts, int nk, int kickoff, void* stream) {
+    BatchExtra X;
+    if (int rc = batch_extra(m, b, xs, nx, consts, nk, &X)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    mc3b_sampler_t s;
+    if (int rc = user_batch_shape(m, b, &s, st)) return rc;
+    MC3B_CHECK_ARG(kickoff == 0 || kickoff == 1, "kickoff must be 0 (normal) or 1 (uniform)");
+    mc3b_batch_t bb = *b;
+    int nch = (int)s.nchains, npars = s.npars, nfree = s.nfree;
+    void* args[] = {&bb, &kickoff, &nch, &npars, &nfree, &X};
+    MC3B_CUDA(cudaLaunchKernel((const void*)m->init, dim3((unsigned)b->nproblems), dim3(SW * 32), args, 0, st));
+    return MC3B_OK;
+}
+
+extern "C" int mc3b_user_batch_run(const mc3b_user_batch_t* m, const mc3b_batch_t* b, const double* const* xs, int nx,
+                                   const double* consts, int nk, int64_t gen0, int64_t ngen, void* stream) {
+    BatchExtra X;
+    if (int rc = batch_extra(m, b, xs, nx, consts, nk, &X)) return rc;
+    MC3B_CHECK_ARG(gen0 >= 0 && ngen > 0, "bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    mc3b_sampler_t s;
+    if (int rc = user_batch_shape(m, b, &s, st)) return rc;
+    const SmallLayout L = small_layout((int)s.nchains, s.npars, s.nfree);
+    MC3B_CHECK_ARG(L.bytes <= 200 * 1024, "population too large for the persistent kernel");
+    mc3b_batch_t bb = *b;
+    int nch = (int)s.nchains, npars = s.npars, nfree = s.nfree;
+    for (int64_t done = 0; done < ngen;) {           // as mc3b_batch_run
+        int64_t g = gen0 + done, step = ngen - done < 200000 ? ngen - done : 200000;
+        void* args[] = {&bb, &nch, &npars, &nfree, &g, &step, &X};
+        MC3B_CUDA(cudaLaunchKernel((const void*)m->run, dim3((unsigned)b->nproblems), dim3(SW * 32), args,
+                                   (size_t)L.bytes, st));
+        done += step;
+    }
+    return MC3B_OK;
+}
+
+extern "C" int mc3b_user_batch_eval(const mc3b_user_batch_t* m, const mc3b_batch_t* b, const double* const* xs, int nx,
+                                    const double* consts, int nk, const double* params, int64_t ldp, double* out,
+                                    void* stream) {
+    BatchExtra X;
+    if (int rc = batch_extra(m, b, xs, nx, consts, nk, &X)) return rc;
+    MC3B_CHECK_ARG(params && out && b->nproblems > 0 && b->offsets && b->x && m->d.nmodel <= ldp, "bad arguments");
+    mc3b_batch_t bb = *b;
+    const unsigned gy = b->nproblems < 65535 ? (unsigned)b->nproblems : 65535u;
+    void* args[] = {&params, &ldp, &bb, &X, &out};
+    MC3B_CUDA(cudaLaunchKernel((const void*)m->eval, dim3(8, gy), dim3(256), args, 0, (cudaStream_t)stream));
+    return MC3B_OK;
 }

@@ -19,7 +19,7 @@
 //     threads 0..nchains-1   metropolis_chain()         (priors, accept, write)
 //     __syncthreads
 //
-// (small_generations in small_dev.cuh, which the batched kernels of batch.cu share).
+// (small_generations in small_dev.cuh, which the batched kernels of batch_dev.cuh share).
 // Same Philox streams, same proposal and acceptance code as the per-generation
 // kernels; only the order in which a chain's chi-squared terms are added
 // differs (rounding-level).  Bound: latency (one CTA by construction).
@@ -33,7 +33,7 @@ __global__ void __launch_bounds__(SW * 32) k_run_small(mc3b_sampler_t G, const d
                                                        const double* __restrict__ w, int64_t n, int64_t gen0,
                                                        int64_t ngen) {
     extern __shared__ __align__(16) double sm[];
-    small_generations<M>(G, x, d, w, n, gen0, ngen, sm);
+    small_generations<M>(G, x, ModelExtra{}, d, w, n, gen0, ngen, sm);
 }
 
 template <class M>

@@ -1,6 +1,7 @@
 // mc3_b200 -- the generation loop of the persistent small-population kernel, as device
 // functions of one CTA: k_run_small (small.cu) runs it over one problem, k_run_batch and
-// k_init_batch (batch.cu) over one problem per CTA.
+// k_init_batch (batch_dev.cuh) over one problem per CTA.  NVRTC compiles it too, into the
+// batch module of a user model (jit.cu).
 #pragma once
 #include "models.cuh"
 #include "sampler_dev.cuh"
@@ -8,6 +9,37 @@
 namespace {
 
 constexpr int SW = 8;       // warps
+
+// What a user model reads besides x (models.cuh ninputs_of, takes_consts): inputs 2..NX of
+// the problem's points, xe[j - 1][i], and the problem's row of run-time constants k.  The
+// built-in models read neither, so their code does not change.
+struct ModelExtra {
+    const double* xe[MC3B_MAX_INPUTS - 1];
+    const double* k;
+};
+
+// load(p), or load(p, k) for a model of constants or a prepare step
+template <class M>
+__device__ __forceinline__ void load_model(M& m, const double* p, const ModelExtra& e) {
+    if constexpr (takes_consts<M>::value) m.load(p, e.k);
+    else m.load(p);
+}
+
+// the model's value at point i: v[0] = x[i], v[j] = xe[j - 1][i]
+template <class M>
+__device__ __forceinline__ double model_at(const M& m, const double* __restrict__ x, const ModelExtra& e,
+                                           int64_t i) {
+    constexpr int NX = ninputs_of<M>::value;
+    if constexpr (NX == 1) {
+        return m.eval_safe(x[i]);
+    } else {
+        double v[NX];
+        v[0] = x[i];
+#pragma unroll
+        for (int j = 1; j < NX; j++) v[j] = e.xe[j - 1][i];
+        return m.eval_safe(v);
+    }
+}
 
 // Shared-memory image of the per-chain state: every array a generation touches
 // except the history (Z, log_post, zchain) lives on chip for the whole launch.
@@ -38,24 +70,26 @@ __host__ __device__ inline SmallLayout small_layout(int nch, int npars, int nfre
 // Data chi-squared of the model m over n points, by one warp: lanes stride the points
 // with two accumulators, then a fixed-order lane tree (every lane returns the sum).
 template <class M>
-__device__ __forceinline__ double warp_chisq(const M& m, const double* __restrict__ x, const double* __restrict__ d,
-                                             const double* __restrict__ w, int64_t n, int lane) {
+__device__ __forceinline__ double warp_chisq(const M& m, const double* __restrict__ x, const ModelExtra& e,
+                                             const double* __restrict__ d, const double* __restrict__ w, int64_t n,
+                                             int lane) {
     double a0 = 0.0, a1 = 0.0;
     int64_t i = lane;
     for (; i + 32 < n; i += 64) {
-        const double r0 = (m.eval_safe(x[i]) - d[i]) * w[i];
-        const double r1 = (m.eval_safe(x[i + 32]) - d[i + 32]) * w[i + 32];
+        const double r0 = (model_at(m, x, e, i) - d[i]) * w[i];
+        const double r1 = (model_at(m, x, e, i + 32) - d[i + 32]) * w[i + 32];
         a0 = fma(r0, r0, a0);
         a1 = fma(r1, r1, a1);
     }
-    if (i < n) { const double r0 = (m.eval_safe(x[i]) - d[i]) * w[i]; a0 = fma(r0, r0, a0); }
+    if (i < n) { const double r0 = (model_at(m, x, e, i) - d[i]) * w[i]; a0 = fma(r0, r0, a0); }
     double a = a0 + a1;
     for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
     return a;
 }
 
 // Generations gen0 .. gen0+ngen-1 of the population G inside the calling CTA (SW * 32
-// threads; sm: small_layout(...).bytes of dynamic shared memory):
+// threads; sm: small_layout(...).bytes of dynamic shared memory; e: what a user model
+// reads besides x):
 //
 //     threads 0..nchains-1   propose_chain()            (sampler_dev.cuh)
 //     __syncthreads
@@ -68,8 +102,9 @@ __device__ __forceinline__ double warp_chisq(const M& m, const double* __restric
 // only the history rows go to global memory.
 template <class M>
 __device__ __forceinline__ void small_generations(const mc3b_sampler_t& G, const double* __restrict__ x,
-                                                  const double* __restrict__ d, const double* __restrict__ w,
-                                                  int64_t n, int64_t gen0, int64_t ngen, double* sm) {
+                                                  const ModelExtra& e, const double* __restrict__ d,
+                                                  const double* __restrict__ w, int64_t n, int64_t gen0,
+                                                  int64_t ngen, double* sm) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, tid = threadIdx.x;
     const int nch = (int)G.nchains, npars = G.npars, nfree = G.nfree;
     const SmallLayout L = small_layout(nch, npars, nfree);
@@ -109,8 +144,8 @@ __device__ __forceinline__ void small_generations(const mc3b_sampler_t& G, const
         for (int c = warp; c < nch; c += SW) {
             if (S.inb[c]) {                              // chain.py:241: no evaluation out of bounds
                 M m;
-                m.load(S.nextp + (int64_t)c * npars);
-                const double a = warp_chisq(m, x, d, w, n, lane);
+                load_model(m, S.nextp + (int64_t)c * npars, e);
+                const double a = warp_chisq(m, x, e, d, w, n, lane);
                 if (lane == 0) chisq_new[c] = a;
             }
         }

@@ -15,6 +15,10 @@ the number of inputs, constants and work slots, the dtype, MC3B_VERSION, the NVR
 embedded kernel headers (not the values of the constants: they are run-time data); the
 loader also checks the module's own ABI record, so a stale file is compiled again
 rather than launched.
+
+A model has two kinds of module: 'chisq', the kernels of sample() (mc3b_user_model_*), and
+'batch', the kernels of sample_batch() (mc3b_user_batch_*, fp64), compiled only when a batch
+asks for it.  The batch kind appends its name to the key.
 """
 import ctypes
 import hashlib
@@ -29,6 +33,9 @@ _CUBINS = {}                  # key -> bytes
 _HANDLES = {}                 # key -> mc3b_user_model_t* (process lifetime)
 _LOCK = threading.Lock()
 _HEADERS = None
+# kind -> (compile, load) entry points of include/mc3b200.h
+_KINDS = {'chisq': ('mc3b_user_model_compile_desc', 'mc3b_user_model_load_desc'),
+          'batch': ('mc3b_user_batch_compile', 'mc3b_user_batch_load')}
 
 
 def nvrtc_candidates():
@@ -90,10 +97,10 @@ def _headers_digest():
     return _HEADERS
 
 
-def cache_key(source, nmodel, dtype, ninputs=1, nconst=0, nwork=0):
+def cache_key(source, nmodel, dtype, ninputs=1, nconst=0, nwork=0, kind='chisq'):
     """Hex key of one compiled model (dtype: _lib.F64 or _lib.F32).  A model of one
     input and no constants or work slots keeps the key it had before models took
-    several inputs."""
+    several inputs; the 'chisq' module keeps the key it had before the 'batch' kind."""
     _, ver = find_nvrtc()
     h = hashlib.sha256()
     parts = [source, str(int(nmodel)), str(int(dtype)), str(_lib.load().mc3b_version()),
@@ -104,6 +111,8 @@ def cache_key(source, nmodel, dtype, ninputs=1, nconst=0, nwork=0):
         parts.append(f'nconst={int(nconst)}')
     if int(nwork) != 0:
         parts.append(f'nwork={int(nwork)}')
+    if kind != 'chisq':
+        parts.append(f'kind={kind}')
     for part in parts:
         h.update(part.encode() + b'\0')
     return h.hexdigest()
@@ -113,18 +122,19 @@ def _desc(nmodel, dtype, ninputs, nconst, nwork):
     return ctypes.byref(_lib.UserModelDesc(int(nmodel), int(ninputs), int(nconst), int(nwork), int(dtype)))
 
 
-def compile_cubin(source, nmodel, dtype, name='model', ninputs=1, nconst=0, nwork=0):
-    """NVRTC: source -> sm_100a CUBIN bytes.  ValueError with the log when the source
-    does not compile."""
+def compile_cubin(source, nmodel, dtype, name='model', ninputs=1, nconst=0, nwork=0, kind='chisq'):
+    """NVRTC: source -> sm_100a CUBIN bytes of the module `kind`.  ValueError with the log
+    when the source does not compile."""
     path, _ = find_nvrtc()
+    entry = _KINDS[kind][0]
     size = ctypes.c_int64(0)
     cap = 1 << 22
     log = ctypes.create_string_buffer(1 << 16)
     lib = _lib.load()
     while True:
         buf = ctypes.create_string_buffer(cap)
-        rc = lib.mc3b_user_model_compile_desc(path.encode(), source.encode(), _desc(nmodel, dtype, ninputs, nconst, nwork),
-                                              buf, cap, ctypes.byref(size), log, len(log))
+        rc = getattr(lib, entry)(path.encode(), source.encode(), _desc(nmodel, dtype, ninputs, nconst, nwork),
+                                 buf, cap, ctypes.byref(size), log, len(log))
         if rc == _lib.ERR_ARG and size.value > cap:
             cap = size.value
             continue
@@ -133,23 +143,22 @@ def compile_cubin(source, nmodel, dtype, name='model', ninputs=1, nconst=0, nwor
         msg = lib.mc3b_last_error().decode('utf-8', 'replace')
         raise ValueError(f'CudaModel {name!r}: {msg}\n{log.value.decode("utf-8", "replace")}')
     if rc != _lib.OK:
-        raise _lib.Mc3bError('mc3b_user_model_compile failed: '
-                             + lib.mc3b_last_error().decode('utf-8', 'replace'))
+        raise _lib.Mc3bError(f"{entry.removesuffix('_desc')} failed: " + lib.mc3b_last_error().decode('utf-8', 'replace'))
     return buf.raw[:size.value]
 
 
-def _load(cubin, nmodel, dtype, ninputs=1, nconst=0, nwork=0):
+def _load(cubin, nmodel, dtype, ninputs=1, nconst=0, nwork=0, kind='chisq'):
     h = ctypes.c_void_p()
-    rc = _lib.load().mc3b_user_model_load_desc(cubin, len(cubin), _desc(nmodel, dtype, ninputs, nconst, nwork),
+    rc = getattr(_lib.load(), _KINDS[kind][1])(cubin, len(cubin), _desc(nmodel, dtype, ninputs, nconst, nwork),
                                                ctypes.byref(h))
     return h if rc == _lib.OK else rc
 
 
-def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1, nconst=0, nwork=0):
-    """Loaded module of (source, nmodel, dtype, ninputs, nconst, nwork): compiled once per process
-    (and taken from MC3B_JIT_CACHE when it is there).  stats, a dict, receives where
+def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1, nconst=0, nwork=0, kind='chisq'):
+    """Loaded module `kind` of (source, nmodel, dtype, ninputs, nconst, nwork): compiled once per
+    process (and taken from MC3B_JIT_CACHE when it is there).  stats, a dict, receives where
     the CUBIN came from ('memory', 'disk', 'nvrtc') and the seconds it took."""
-    key = cache_key(source, nmodel, dtype, ninputs, nconst, nwork)
+    key = cache_key(source, nmodel, dtype, ninputs, nconst, nwork, kind)
     with _LOCK:
         h = _HANDLES.get(key)
         if h is not None:
@@ -165,10 +174,10 @@ def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1, nconst=0,
             with open(fpath, 'rb') as f:
                 cubin = f.read()
             origin = 'disk'
-        h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork) if cubin is not None else None
+        h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork, kind) if cubin is not None else None
         if not isinstance(h, ctypes.c_void_p):
             # not compiled yet, or a stale file that the loader refused: compile
-            cubin = compile_cubin(source, nmodel, dtype, name, ninputs, nconst, nwork)
+            cubin = compile_cubin(source, nmodel, dtype, name, ninputs, nconst, nwork, kind)
             origin = 'nvrtc'
             if fpath:
                 os.makedirs(cdir, exist_ok=True)
@@ -176,9 +185,9 @@ def handle(source, nmodel, dtype, name='model', stats=None, ninputs=1, nconst=0,
                 with open(tmp, 'wb') as f:
                     f.write(cubin)
                 os.replace(tmp, fpath)
-            h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork)
+            h = _load(cubin, nmodel, dtype, ninputs, nconst, nwork, kind)
             if not isinstance(h, ctypes.c_void_p):
-                raise _lib.Mc3bError('mc3b_user_model_load failed: '
+                raise _lib.Mc3bError(f"{_KINDS[kind][1].removesuffix('_desc')} failed: "
                                      + _lib.load().mc3b_last_error().decode('utf-8', 'replace'))
         _CUBINS[key] = cubin
         _HANDLES[key] = h

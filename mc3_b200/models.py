@@ -187,6 +187,13 @@ class CudaModel:
         return jit.handle(self.source, self.nparams, dtype, self.name, stats, self.ninputs, self.nconst,
                           self.nwork)
 
+    def batch_handle(self, stats=None):
+        """mc3b_user_batch_t* of this model: the fp64 kernels of sample_batch, a module of
+        their own (compiled on first use, not by sample())."""
+        from . import jit
+        return jit.handle(self.source, self.nparams, _lib.F64, self.name, stats, self.ninputs, self.nconst,
+                          self.nwork, kind='batch')
+
     def __call__(self, params, *args):
         import torch
         xs, k = self.split_args(args)
