@@ -581,7 +581,8 @@ typedef struct mc3b_batch {
     const int64_t* offsets;           /* [nproblems + 1], device: problem b owns points [offsets[b], offsets[b+1]) */
     const double* x; const double* data; const double* invsig;
     int32_t* status;                  /* [nproblems], device: 0 ok, 1 initial population not filled,
-                                         2 shape differs from problem 0's or no data points */
+                                         2 shape differs from problem 0's or no data points,
+                                         3 stopped by the convergence test (mc3b_batch_gelman_rubin) */
 } mc3b_batch_t;
 
 /* Initial population of every problem (mcmc_driver.py:229-278), one CTA per
@@ -599,6 +600,20 @@ int mc3b_batch_init(const mc3b_batch_t* b, int model_id, int nmodel, int kickoff
  * arithmetic, bit for bit, as mc3b_run_small on that problem alone.  The per-problem
  * gen_dev is ignored.  Split into launches of at most 200 000 generations. */
 int mc3b_batch_run(const mc3b_batch_t* b, int model_id, int nmodel, int64_t gen0, int64_t ngen, void* stream);
+
+/* Gelman-Rubin at report point k (k thinned steps done) of every problem whose status is
+ * 0 (mcmc_driver.py:325-346, gelman.py:36-92), one CTA per problem; model-independent, so
+ * it serves mc3b_batch_run and mc3b_user_batch_run alike:
+ *   psrf[b * ldpsrf + p]  PSRF of free parameter p over thinned steps [zburn, k) (lock-step
+ *                         rows M0 + k' nchains + c), bit for bit mc3b_gelman_rubin on that
+ *                         problem's history; left untouched for the problems it skips
+ *   grbreak > 0, every psrf < grbreak (NaN never passes) and M0 + k nchains > grnmin:
+ *                         status[b] = 3 and kstop[b] = k, so that later mc3b_batch_run /
+ *                         mc3b_user_batch_run launches skip the problem.
+ * Needs nchains >= 2, 0 <= zburn < k, M0 + k nchains <= zlen, ldpsrf >= nfree; kstop may
+ * be NULL when grbreak <= 0.  Reads problem 0's description back as mc3b_batch_run does. */
+int mc3b_batch_gelman_rubin(const mc3b_batch_t* b, int64_t k, int64_t zburn, double grbreak,
+                            int64_t grnmin, double* psrf, int64_t ldpsrf, int64_t* kstop, void* stream);
 
 /* The batch of a user model (mc3b_user_model_desc_t, fp64 only): k_init_batch, k_run_batch
  * and a batched model-value kernel compiled by NVRTC into a module of their own, so that

@@ -153,6 +153,8 @@ _SIGS = {
                                c_i64, c_i64, c_i64, c_vp]),
     'mc3b_batch_init': (c_int, [ctypes.POINTER(BatchStruct), c_int, c_int, c_int, c_vp]),
     'mc3b_batch_run': (c_int, [ctypes.POINTER(BatchStruct), c_int, c_int, c_i64, c_i64, c_vp]),
+    'mc3b_batch_gelman_rubin': (c_int, [ctypes.POINTER(BatchStruct), c_i64, c_i64, c_dbl, c_i64, c_vp, c_i64, c_vp,
+                                        c_vp]),
     'mc3b_user_batch_compile': (c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.POINTER(UserModelDesc), c_vp, c_i64,
                                         ctypes.POINTER(c_i64), ctypes.c_char_p, c_i64]),
     'mc3b_user_batch_load': (c_int, [ctypes.c_char_p, c_i64, ctypes.POINTER(UserModelDesc), ctypes.POINTER(c_vp)]),

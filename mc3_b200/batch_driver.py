@@ -10,6 +10,11 @@ sampler and its options, and the pattern of free, shared and fixed parameters.  
 CudaModel's per-point inputs and run-time constants are the problem's own: indparams[b]
 is read as sample() reads it (CudaModel.split_args), and the kernels are those of the
 model's batch module (CudaModel.batch_handle).  It writes no files and no log output.
+
+With grtest, the Gelman-Rubin test runs on the device at sample()'s report points
+(mcmc_driver.report_points) for every problem at once (mc3b_batch_gelman_rubin); with
+grbreak, a problem that passes stops there and gives up its CTA to the problems still
+running, and its output covers the thinned steps it ran.
 """
 import ctypes
 
@@ -20,6 +25,7 @@ from . import _lib
 from . import stats as ms
 from .engine import column_statistics, to_host
 from .models import BuiltinModel, CudaModel
+from .mcmc_driver import gr_min_size, report_points
 from .sampler_driver import check_sampler, read_arrays, fill_vectors
 
 MAX_CHAINS = 256                  # SW * 32 threads of mc3b_batch_run's CTA
@@ -60,6 +66,7 @@ def _per_problem(name, value, B):
 def sample_batch(data, uncert, func, params, indparams,
                  pmin=None, pmax=None, pstep=None, prior=None, priorlow=None, priorup=None,
                  sampler=None, nchains=7, nsamples=None, burnin=0, thinning=1,
+                 grtest=False, grbreak=0.0, grnmin=0.5,
                  fgamma=1.0, fepsilon=0.0, hsize=10, kickoff='normal',
                  pnames=None, texnames=None, seed=None, device=None, wlike=False, dtype='f64',
                  _state=False):
@@ -76,6 +83,12 @@ def sample_batch(data, uncert, func, params, indparams,
     func          a BuiltinModel (polynomial, sinusoid, gaussian, box) or a CudaModel, fp64
     seed          int s (problem b takes s + b), B ints, or None (one drawn as sample()
                   draws it, then s + b)
+    grtest, grbreak, grnmin
+                  as in sample(), problem by problem: with grtest each output gains 'psrf',
+                  the PSRF of the problem's last Gelman-Rubin evaluation; with grbreak > 0 a
+                  problem stops at the first report where every PSRF < grbreak and its
+                  history exceeds grnmin, and its outputs cover the steps it ran.  grtest is
+                  off by default (sample() turns it on), since the batch prints no log.
     The other options mean what they mean in sample(); nchains <= 256.  _state=True
     returns the device state after the generations instead (for tests)."""
     check_sampler(sampler, nsamples, None, _Log0())
@@ -91,6 +104,8 @@ def sample_batch(data, uncert, func, params, indparams,
                          '(sample() runs larger populations)')
     if sampler == 'demc' and nchains < 3:
         raise ValueError(f'demc needs at least 3 chains, got {nchains}')
+    if grtest and nchains < 2:
+        raise ValueError(f'the Gelman-Rubin test needs at least 2 chains, got {nchains}')
     if kickoff not in ('normal', 'uniform'):
         raise ValueError(f"kickoff must be 'normal' or 'uniform', got {kickoff!r}")
 
@@ -162,6 +177,8 @@ def sample_batch(data, uncert, func, params, indparams,
         raise ValueError('the burned-in sample of a problem must hold at least 2 rows')
     M0 = hsize*nchains
     zlen = M0 + nzchain*nchains
+    grmin = gr_min_size(grnmin, nchains, nzchain, zburn, thinning, M0, _Log0())
+    reports = report_points(nzchain)
 
     # ---- device ----
     _lib.load()
@@ -173,7 +190,7 @@ def sample_batch(data, uncert, func, params, indparams,
     with torch.cuda.device(dev):
         sizes = np.array([q['data'].size for q in probs], dtype=np.int64)
         need = _state_bytes(B, nchains, npars, nfree, zlen, int(sizes.sum()), len(probs[0]['xs']),
-                            func.nconst if user else 0)
+                            func.nconst if user else 0, len(reports) if grtest else 0)
         free = torch.cuda.mem_get_info(dev)[0]
         if need > free:
             raise ValueError(f'the state of {B} problems needs {need} bytes of device memory, '
@@ -181,7 +198,10 @@ def sample_batch(data, uncert, func, params, indparams,
         run = _BatchRun(probs, seeds, sizes, dev, sampler, nchains, npars, nfree, ifree, M0, zlen,
                         thinning, fgamma, fepsilon)
         run.init(kickoff, func)
-        run.run(niter, func)
+        if grtest:
+            run.run_gr(func, reports, zburn, float(grbreak), grmin)
+        else:
+            run.run(niter, func)
         if _state:
             return run
         return run.outputs(func, zburn, nzchain, probs)
@@ -212,12 +232,14 @@ class _Log0:
         raise exception(message)
 
 
-def _state_bytes(B, nchains, npars, nfree, zlen, ntot, ninputs=1, nconst=0):
+def _state_bytes(B, nchains, npars, nfree, zlen, ntot, ninputs=1, nconst=0, nreports=0):
     """Device bytes of the batched state (history, per-chain arrays, data, a CudaModel's
-    further inputs and constants) and of the post-processing copies of the history
+    further inputs and constants, with the Gelman-Rubin test the PSRF table of nreports
+    reports and the stop points) and of the post-processing copies of the history
     (chi-squared column)."""
     per = zlen*(nfree*8 + 8 + 4 + 8) + nchains*(2*nfree*8 + npars*8 + 4*8 + 2*4) + nfree*4 + 7*npars*8
-    return B*per + 3*ntot*8 + (ninputs - 1)*ntot*8 + B*nconst*8
+    gr = B*(nreports*nfree*8 + 8) if nreports else 0
+    return B*per + 3*ntot*8 + (ninputs - 1)*ntot*8 + B*nconst*8 + gr
 
 
 class _BatchRun:
@@ -261,6 +283,7 @@ class _BatchRun:
         self.best_x = torch.zeros((B, n, nfree), **f64)
         self.best_gen = torch.zeros((B, n), dtype=torch.int64, device=dev)
         self.status = torch.zeros(B, **i32)
+        self.psrf = self.kstop = None               # run_gr: [B, nreports, nfree], [B]
 
         # one mc3b_sampler_t per problem, as engine.Population._make_struct fills it
         tab = np.zeros(B, dtype=np.dtype(_lib.SamplerStruct))
@@ -318,13 +341,33 @@ class _BatchRun:
                 'beyond the parameter boundaries or where the model returns '
                 'non-finite values.')
 
-    def run(self, ngen, func):
+    def run(self, ngen, func, gen0=0):
         if isinstance(func, CudaModel):
-            _lib.call('mc3b_user_batch_run', func.batch_handle(), ctypes.byref(self.S), *self._extra(func), 0, ngen,
-                      _lib.stream_ptr())
+            _lib.call('mc3b_user_batch_run', func.batch_handle(), ctypes.byref(self.S), *self._extra(func), gen0,
+                      ngen, _lib.stream_ptr())
         else:
             _lib.call('mc3b_batch_run', ctypes.byref(self.S), func.model_id, func.nmodel(self.npars),
-                      0, ngen, _lib.stream_ptr())
+                      gen0, ngen, _lib.stream_ptr())
+
+    def run_gr(self, func, reports, zburn, grbreak, grmin):
+        """The run with the Gelman-Rubin test (mcmc_driver.py:297-348).  grbreak > 0: report
+        blocks, and the test at every report past burn-in, where the problems that pass stop
+        (status 3, kstop); otherwise one run and one test at the last report.  psrf[b, i] is
+        problem b's PSRF at report i (NaN where not evaluated); kstop[b] the thinned steps it
+        ran.  Nothing returns to the host in between."""
+        B, nf, th = self.B, self.nfree, self.thinning
+        self.reports = reports
+        self.psrf = torch.full((B, len(reports), nf), float('nan'), dtype=torch.float64, device=self.dev)
+        self.kstop = torch.full((B,), reports[-1], dtype=torch.int64, device=self.dev)
+        k0 = 0
+        for i, k in enumerate(reports):
+            if grbreak <= 0.0 and k < reports[-1]:
+                continue
+            self.run((k - k0)*th, func, gen0=k0*th)
+            k0 = k
+            if k > zburn:                                           # :325
+                _lib.call('mc3b_batch_gelman_rubin', ctypes.byref(self.S), k, zburn, grbreak, grmin,
+                          self.psrf[:, i].data_ptr(), len(reports)*nf, self.kstop.data_ptr(), _lib.stream_ptr())
 
     def outputs(self, func, zburn, nzchain, probs):
         """Output dictionaries (mcmc_driver.update_output + sample()'s statistics)."""
@@ -372,52 +415,65 @@ class _BatchRun:
                 _lib.call('mc3b_model_eval', func.model_id, bestp[b].data_ptr(), npars, 1, nmodel,
                           self.d_x[o:].data_ptr(), k, model[o:].data_ptr(), st)
 
+        # thinned steps problem b ran: nzchain, or where the Gelman-Rubin test stopped it
+        Ks = np.full(B, nzchain, dtype=np.int64) if self.kstop is None else to_host(self.kstop)
+
         # chi-squared column: -2 (log_post - log_prior) of every history row
-        K = nzchain
-        rows = K*n
-        chisq = torch.empty((B, rows), dtype=torch.float64, device=dev)
+        chisq = torch.empty((B, nzchain*n), dtype=torch.float64, device=dev)
         for b in range(B):
-            _lib.call('mc3b_log_prior', self.Z[b, M0:].data_ptr(), rows, nfree, self.d_ifree.data_ptr(),
+            _lib.call('mc3b_log_prior', self.Z[b, M0:].data_ptr(), int(Ks[b])*n, nfree, self.d_ifree.data_ptr(),
                       self.vec['prior'][b].data_ptr(), self.vec['priorlow'][b].data_ptr(),
                       self.vec['priorup'][b].data_ptr(), self.log_post[b, M0:].data_ptr(), None,
                       chisq[b].data_ptr(), st)
 
         # posterior statistics: the burned sample (utils.burn's lock-step closed form), at most
-        # 20000 rows picked as sample() picks them -- the same rows for every problem
-        zmask = (np.arange(zburn, K)[None, :]*n + np.arange(n)[:, None]).ravel()
-        pick = zmask
-        if zmask.size > 20000:
-            pick = zmask[np.random.default_rng(314159).choice(zmask.size, 20000, replace=False)]
-        blk = self.Z[:, M0 + torch.from_numpy(pick).to(dev)]          # [B, nstat, nfree]
-        blk = blk.permute(1, 0, 2).reshape(blk.shape[1], B*nfree).contiguous()
-        cs = column_statistics(blk, 0.683)                              # [5, B nfree]
-        hpd = torch.empty((3, B*nfree), dtype=torch.float64, device=dev)
-        step = 65535                                 # k_kde_grid: one grid.y per column
-        ws = torch.empty(max(_lib.load().mc3b_hpd_workspace(min(step, B*nfree)), 8)//8,
-                         dtype=torch.float64, device=dev)
-        for c0 in range(0, B*nfree, step):
-            c1 = min(c0 + step, B*nfree)
-            chunk = blk[:, c0:c1].contiguous()
-            o = torch.empty((3, c1 - c0), dtype=torch.float64, device=dev)
-            _lib.call('mc3b_hpd', chunk.data_ptr(), chunk.shape[0], c1 - c0, 0.683, ws.data_ptr(),
-                      o.data_ptr(), st)
-            hpd[:, c0:c1] = o
-        free_stats = torch.cat([cs, hpd]).view(8, B, nfree)
+        # 20000 rows picked as sample() picks them -- the same rows for every problem that ran
+        # the same number of steps; one pass per such group (at most one per report)
+        free_stats = torch.empty((8, B, nfree), dtype=torch.float64, device=dev)
+        zmasks = {}
+        for K in np.unique(Ks):
+            grp = np.flatnonzero(Ks == K)
+            G = grp.size
+            zmask = (np.arange(zburn, K)[None, :]*n + np.arange(n)[:, None]).ravel()
+            pick = zmask
+            if zmask.size > 20000:
+                pick = zmask[np.random.default_rng(314159).choice(zmask.size, 20000, replace=False)]
+            zmasks[K] = zmask
+            g = torch.from_numpy(grp).to(dev)
+            blk = self.Z[g[:, None], M0 + torch.from_numpy(pick).to(dev)[None, :]]     # [G, nstat, nfree]
+            blk = blk.permute(1, 0, 2).reshape(blk.shape[1], G*nfree).contiguous()
+            cs = column_statistics(blk, 0.683)                              # [5, G nfree]
+            hpd = torch.empty((3, G*nfree), dtype=torch.float64, device=dev)
+            step = 65535                                 # k_kde_grid: one grid.y per column
+            ws = torch.empty(max(_lib.load().mc3b_hpd_workspace(min(step, G*nfree)), 8)//8,
+                             dtype=torch.float64, device=dev)
+            for c0 in range(0, G*nfree, step):
+                c1 = min(c0 + step, G*nfree)
+                chunk = blk[:, c0:c1].contiguous()
+                o = torch.empty((3, c1 - c0), dtype=torch.float64, device=dev)
+                _lib.call('mc3b_hpd', chunk.data_ptr(), chunk.shape[0], c1 - c0, 0.683, ws.data_ptr(),
+                          o.data_ptr(), st)
+                hpd[:, c0:c1] = o
+            free_stats[:, g] = torch.cat([cs, hpd]).view(8, G, nfree)
 
         # to the host, one copy per array
         h = {k: to_host(v) for k, v in (
             ('Z', self.Z[:, M0:]), ('zchain', self.zchain[:, M0:]), ('log_post', self.log_post[:, M0:]),
             ('chisq', chisq), ('model', model), ('bestp', bestp), ('best_chi', best_chi),
             ('numaccept', numaccept), ('free', free_stats))}
-        nsample = K*n*self.thinning
+        if self.psrf is not None:
+            h['psrf'] = to_host(self.psrf)
         outs = []
         for b, q in enumerate(probs):
             o0, o1 = self.off[b], self.off[b + 1]
+            K = int(Ks[b])
+            rows = K*n
+            nsample = rows*self.thinning
             bp = h['bestp'][b].copy()
             out = {'pnames': q['pnames'], 'texnames': q['texnames'], 'pstep': q['pstep'],
                    'ifree': q['ifree'], 'burnin': zburn,
-                   'posterior': h['Z'][b], 'zchain': h['zchain'][b].astype(int),
-                   'chisq': h['chisq'][b], 'log_post': h['log_post'][b],
+                   'posterior': h['Z'][b, :rows], 'zchain': h['zchain'][b, :rows].astype(int),
+                   'chisq': h['chisq'][b, :rows], 'log_post': h['log_post'][b, :rows],
                    'acceptance_rate': int(h['numaccept'][b])*100.0/max(nsample, 1)}
             # calc_bestfit_statistics (stats.py:855-873) from the tracked best chi-squared
             ndata = int(o1 - o0)
@@ -432,7 +488,7 @@ class _BatchRun:
             out['best_log_post'] = best_log_post
             out['best_model'] = best_model
             out['stddev_residuals'] = np.std(best_model - q['data'])
-            out['zmask'] = zmask
+            out['zmask'] = zmasks[K]
             st8 = ms.expand_free_stats(tuple(h['free'][:, b]), bp, q['pstep'])
             for k, v in zip(('medianp', 'meanp', 'stdp', 'median_low_bounds', 'median_high_bounds',
                              'mode', 'hpd_low_bounds', 'hpd_high_bounds'), st8):
@@ -441,5 +497,7 @@ class _BatchRun:
             out['CRlo'] = out['hpd_low_bounds'] - bp
             out['CRhi'] = out['hpd_high_bounds'] - bp
             out['CRlo'][q['pstep'] == 0] = out['CRhi'][q['pstep'] == 0] = 0.0
+            if self.psrf is not None:               # the last evaluation: at K (the last report, or the stop)
+                out['psrf'] = h['psrf'][b, self.reports.index(K)].copy()
             outs.append(out)
         return outs

@@ -12,6 +12,7 @@
 // proposed points equal numpy's elementwise results.
 #include <stdlib.h>
 #include "sampler_dev.cuh"
+#include "gelman_dev.cuh"
 
 namespace {
 
@@ -172,7 +173,8 @@ __global__ void __launch_bounds__(128) k_log_prior(const double* Z, int64_t nrow
 // ---- Gelman-Rubin ----------------------------------------------------------
 // Stage 1: one thread per (chain, parameter): mean and population variance of
 // its niter samples (two passes, as numpy's var).  Stage 2: one CTA, fixed-order
-// sums over chains -> W, B, V, sqrt(V/W)   (gelman.py:75-92).
+// sums over chains -> W, B, V, sqrt(V/W)   (gelman.py:75-92).  The arithmetic is
+// gelman_dev.cuh's, which k_batch_gr (batch.cu) shares.
 __global__ void __launch_bounds__(128) k_gr_stats(const double* Z, int64_t nfree, int64_t nchains, int64_t M0,
                                                   const int64_t* rows, int64_t ldr, int64_t burnin, int64_t niter,
                                                   int64_t c_begin, int64_t c_end, double* work) {
@@ -188,7 +190,7 @@ __global__ void __launch_bounds__(128) k_gr_stats(const double* Z, int64_t nfree
     for (int64_t k = burnin; k < burnin + niter; k++) s += at(k);
     const double mu = s / (double)niter;
     double v = 0.0;
-    for (int64_t k = burnin; k < burnin + niter; k++) { const double d = at(k) - mu; v += d * d; }
+    for (int64_t k = burnin; k < burnin + niter; k++) v = gr_sq_add(v, at(k) - mu);
     work[t] = mu;
     work[nchains * nfree + t] = v / (double)niter;
 }
@@ -196,32 +198,8 @@ __global__ void __launch_bounds__(128) k_gr_stats(const double* Z, int64_t nfree
 __global__ void __launch_bounds__(256) k_gr_psrf(const double* work, int64_t nfree, int64_t nchains, int64_t niter,
                                                  double* psrf) {
     __shared__ double sh[256];
-    const int p = blockIdx.x;
-    const double* mu = work;
-    const double* var = work + nchains * nfree;
-    auto block_sum = [&](double v) -> double {
-        sh[threadIdx.x] = v;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) {
-            if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-            __syncthreads();
-        }
-        const double r = sh[0];
-        __syncthreads();
-        return r;
-    };
-    double a = 0.0, b = 0.0;
-    for (int64_t c = threadIdx.x; c < nchains; c += 256) { a += var[c * nfree + p]; b += mu[c * nfree + p]; }
-    const double W = block_sum(a) / (double)nchains;
-    const double mm = block_sum(b) / (double)nchains;
-    double d2 = 0.0;
-    for (int64_t c = threadIdx.x; c < nchains; c += 256) { const double d = mu[c * nfree + p] - mm; d2 += d * d; }
-    const double B = (double)niter / ((double)nchains - 1.0) * block_sum(d2);
-    if (threadIdx.x == 0) {
-        const double V = W * (((double)niter - 1.0) / (double)niter) +
-                         B * (((double)nchains + 1.0) / ((double)niter * (double)nchains));
-        psrf[p] = sqrt(V / W);
-    }
+    const double r = gr_psrf(work, work + nchains * nfree, nfree, nchains, niter, blockIdx.x, sh);
+    if (threadIdx.x == 0) psrf[blockIdx.x] = r;
 }
 
 int check_sampler(const mc3b_sampler_t* s, int64_t c_begin, int64_t c_end) {

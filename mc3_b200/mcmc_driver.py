@@ -94,6 +94,34 @@ def update_output(output, pop, hsize, counters=None):
     return nburned
 
 
+def report_points(nzchain):
+    """Thinned steps done at each report of a run of nzchain thinned steps: every
+    ceil(nzchain/10), the last at nzchain (mcmc_driver.py:297-348)."""
+    step = max(1, int(np.ceil(nzchain/10)))
+    ks, k = [], 0
+    while k < nzchain:
+        k = min(nzchain, k + step)
+        ks.append(k)
+    return ks
+
+
+def gr_min_size(grnmin, nchains, nzchain, zburn, thinning, M0, log):
+    """The grnmin rule (mcmc_driver.py:186-198): the history size (rows, M0 included)
+    that a Gelman-Rubin stop must exceed.  grnmin >= 1 counts samples, 0 < grnmin < 1
+    is the fraction of the burned-in sample; grnmin < 0 is an error (log.error)."""
+    if grnmin >= 1:
+        grnmin = int(grnmin/thinning)
+    elif grnmin > 0:
+        grnmin = int(grnmin*nchains*(nzchain - zburn))
+    elif grnmin < 0:
+        log.error(
+            "Invalid 'grnmin' argument (minimum number of samples to "
+            "stop the MCMC under GR convergence), must either be grnmin > 1"
+            "to set the minimum number of samples, or 0 < grnmin < 1"
+            "to set the fraction of samples required to evaluate.")
+    return grnmin + int(M0 + zburn*nchains)
+
+
 def mcmc(data, uncert, func, params, indparams, indparams_dict,
          pmin, pmax, pstep, prior, priorlow, priorup, nchains, ncpu, nsamples,
          sampler, wlike, fit_output, grtest, grbreak, grnmin, burnin, thinning,
@@ -123,17 +151,7 @@ def mcmc(data, uncert, func, params, indparams, indparams_dict,
             f"the number of iterations per chain ({niter})")
     zburn = int(burnin/thinning)
 
-    if grnmin >= 1:                                          # :186-198
-        grnmin = int(grnmin/thinning)
-    elif grnmin > 0:
-        grnmin = int(grnmin*nchains*(nzchain - zburn))
-    elif grnmin < 0:
-        log.error(
-            "Invalid 'grnmin' argument (minimum number of samples to "
-            "stop the MCMC under GR convergence), must either be grnmin > 1"
-            "to set the minimum number of samples, or 0 < grnmin < 1"
-            "to set the fraction of samples required to evaluate.")
-    grnmin += int(M0 + zburn*nchains)
+    grnmin = gr_min_size(grnmin, nchains, nzchain, zburn, thinning, M0, log)
 
     if seed is None:
         seed = int(np.random.randint(0, 2**31 - 1))
@@ -168,7 +186,6 @@ def mcmc(data, uncert, func, params, indparams, indparams_dict,
     # copies have landed: the device never waits for the host between blocks.  The
     # host only blocks where the reference's control flow needs the numbers: a
     # savefile to write, or a grbreak decision.
-    step_k = max(1, int(np.ceil(nzchain/10)))
     k_done = 0
     pending = []
 
@@ -202,8 +219,7 @@ def mcmc(data, uncert, func, params, indparams, indparams_dict,
                     return True
         return False
 
-    while k_done < nzchain:
-        k_next = min(nzchain, k_done + step_k)
+    for k_next in report_points(nzchain):
         pop.run((k_next - k_done)*thinning, use_graph=use_graph)
         k_done = k_next
         hc = pop.counters_async()
