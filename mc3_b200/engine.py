@@ -35,10 +35,9 @@ import numpy as np
 import torch
 
 from . import _lib
-from .models import BuiltinModel, CudaModel, TorchModel, SINUSOID, SINUSOID_GRID
-from . import gridseg, spectral
-from .parallel import chain_slice, allgather_rows, gather_history, sum_owned
-
+from .models import BuiltinModel, CudaModel, TorchModel
+from .chisq_form import choose_form
+from .parallel import chain_slice, allgather_rows, gather_history
 
 
 def to_host(t):
@@ -192,7 +191,6 @@ class Population:
         self.indparams_dict = dict(indparams_dict or {})
         self.wlike = bool(wlike)
         self.sampler = sampler
-        self.usig = False
         self.dtype = _DT[dtype]
         f64 = dict(dtype=torch.float64, device=self.dev)
 
@@ -239,168 +237,39 @@ class Population:
         self.d_data = torch.from_numpy(data).to(self.dev)
         self.d_uncert = torch.from_numpy(uncert).to(self.dev)
         self.nfunc = npars - 3 if self.wlike else npars
-        if isinstance(func, CudaModel) and self.shard == 'data':
-            raise ValueError("shard='data' needs a built-in model (a CudaModel runs with "
-                             "shard='chains')")
+        if self.shard == 'data' and not isinstance(func, BuiltinModel):
+            raise ValueError("shard='data' needs a built-in model (other models run with shard='chains')")
+        # the chi-squared form (chisq_form.choose_form); what does not apply stays unset
+        self.usig = self.grid = self.use_moment = False
+        self.chisq_model_id = self.seg = self.spectral_plan = self.d_tile_x = None
+        self.d_fold = self.moment = self.spectral = self.guard_hits = None
         if isinstance(func, (BuiltinModel, CudaModel)):
-            # a CudaModel takes the built-in path with its own compiled kernels
-            # (mc3b_user_model_*): never the sinusoid grid, fold or moment kernels
-            user = isinstance(func, CudaModel)
-            self.kind = 'cuda' if user else 'builtin'
-            self.nmodel = func.nmodel(self.nfunc)
-            self.jit = func.handle(self.dtype) if user else None
-            # model values are fp64 whatever the dtype, as mc3b_model_eval's
-            self.jit_eval = func.handle(_lib.F64) if user else None
-            nin = func.ninputs if user else 1
-            # a CudaModel of run-time constants: the indparams after its inputs, flattened
-            # (CudaModel.split_args); every rank builds its own copy
-            xargs, kc = func.split_args(self.indparams) if user else (self.indparams, None)
-            if nin > 1:
-                # a CudaModel of several inputs: one 1-D array per input, in the order of
-                # the arguments of its `model`
-                xin = [np.ascontiguousarray(a, dtype=np.double) for a in xargs]
-                if len(xin) != nin or any(a.ndim != 1 or a.size != self.ndata_total for a in xin):
-                    raise ValueError(f'CudaModel {func.name!r} takes {nin} inputs: it needs indparams=[x1, ..., '
-                                     f'x{nin}], {nin} 1-D arrays with the same shape as data (got '
-                                     f'{[np.shape(a) for a in self.indparams]} for data of {self.ndata_total})')
-            x = np.ascontiguousarray(self.indparams[0], dtype=np.double)
-            if x.size != self.ndata_total or x.ndim != 1:
-                raise ValueError(f'{"CUDA" if user else "built-in"} models need indparams=[x] '
-                                 'with the same shape as data')
-            x = x[lo:hi]
-            self.d_x = torch.from_numpy(x).to(self.dev)
-            # every input of the model on the device (d_xs[0] is d_x); their host array of
-            # pointers is what mc3b_user_model_eval_consts takes
-            self.d_xs = [self.d_x] + [torch.from_numpy(a[lo:hi]).to(self.dev) for a in xin[1:]] \
-                if nin > 1 else [self.d_x]
-            self.d_xptrs = _lib.ptrs(self.d_xs)
-            # ... and its constants, fp64 (model values) and in the kernel's dtype; None: none
-            self.d_kc = torch.from_numpy(kc).to(self.dev) if kc is not None and kc.size else None
-            self.nconst = func.nconst if user else 0
-            self.d_invsig = 1.0/self.d_uncert
-            # one uncertainty for all points: no weight stream, residuals are plain
-            # differences (mc3b_chisq_opts_t.uniform_sigma); MC3B_NO_USIG=1 disables
-            self.usig = bool(uncert.size > 0 and np.all(uncert == uncert[0])
-                             and not os.environ.get('MC3B_NO_USIG'))
-            # A sinusoid on a uniform abscissa grid takes the rotation-recurrence
-            # kernel (models.cuh SineGridModel); MC3B_NO_GRID=1 forces the plain one.
-            self.chisq_model_id = None if user else func.model_id
-            self.grid = False
-            self.seg = None                    # piecewise-uniform layout (gridseg.tile_layout) or None
-            kx, kd, kw = self.d_x, self.d_data, self.d_invsig     # what the model kernels read
-            nfold = self.ndata                 # leading entries of kd that form whole tiles
-            fold_ok = self.usig and not os.environ.get('MC3B_NO_FOLD')
-            if not user and func.model_id == SINUSOID and self.dtype == _lib.F64 and x.size >= 8 \
-                    and not os.environ.get('MC3B_NO_GRID'):
-                ideal = x[0] + np.arange(x.size)*((x[-1] - x[0])/(x.size - 1))
-                if x[-1] != x[0] and np.max(np.abs(x - ideal)) <= 8*np.finfo(float).eps*np.max(np.abs(x)):
-                    self.chisq_model_id = SINUSOID_GRID
-                    self.grid = True
-                elif not os.environ.get('MC3B_NO_SEG'):
-                    # constant cadence with gaps: whole 128-point tiles first, the points
-                    # that fill no tile last (include/mc3b200.h, tile_x)
-                    self.seg = gridseg.tile_layout(x)
-                    if self.seg is not None:
-                        self.chisq_model_id = SINUSOID_GRID
-                        self.grid = True
-                        with torch.cuda.device(self.dev):
-                            perm = torch.from_numpy(self.seg['perm']).to(self.dev)
-                            kx, kd = self.d_x[perm].contiguous(), self.d_data[perm].contiguous()
-                            if not self.usig:
-                                kw = self.d_invsig[perm].contiguous()
-                            self.d_tile_x = torch.from_numpy(np.ascontiguousarray(x[self.seg['starts']])).to(self.dev)
-                        nfold = 128*self.seg['starts'].size
-            # with one uncertainty for all points the grid kernel works on point pairs
-            # mirrored about block centres (csrc/chisq_grid.cu k_sinefold): the paired
-            # copy of the data is prepared once here.  MC3B_NO_FOLD=1 disables.
-            self.d_fold = None
-            if self.grid and fold_ok:
-                with torch.cuda.device(self.dev):
-                    self.d_fold = torch.zeros_like(kd)
-                    _lib.call('mc3b_fold_data', kd.data_ptr(), nfold,
-                              self.d_fold.data_ptr(), _lib.stream_ptr())
-            # ... and, inside the generation loop, on sufficient statistics of those pairs
-            # (k_sinefold<MOM>, one multiply-add per point; include/mc3b200.h mc3b_moment_t):
-            # the data are centred on their least-squares line first, which keeps the
-            # cancellation of the expansion at (signal/noise)^2.  A guard in the kernel
-            # re-evaluates every chain the expansion is not accurate enough for; when that
-            # is not rare (_moment_policy) the population returns to the pair kernel.
-            # MC3B_NO_MOMENT=1 disables.
-            self.moment = None
-            self.use_moment = False
-            self.spectral = None
-            if self.d_fold is not None and nfold >= 256 \
-                    and not os.environ.get('MC3B_NO_MOMENT') and not os.environ.get('MC3B_NO_FUSE'):
-                with torch.cuda.device(self.dev):
-                    # least-squares line through the data and the sum of squares about it,
-                    # on the device (a few small kernels and one read of three numbers)
-                    xm, dm = self.d_x.mean(), self.d_data.mean()
-                    xc = self.d_x - xm
-                    slr_t = torch.dot(xc, self.d_data - dm)/torch.dot(xc, xc)
-                    c0r_t = dm - slr_t*xm
-                    res = self.d_data - (c0r_t + slr_t*self.d_x)
-                    c0r, slr, d2tot = (float(v) for v in torch.stack([c0r_t, slr_t, torch.dot(res, res)]).cpu())
-                    self.d_mfold = torch.zeros_like(kd)
-                    self.d_mtiles = torch.zeros((max(nfold//128, 1), 4), **f64)
-                    self.guard_hits = torch.zeros(1, dtype=torch.int32, device=self.dev)
-                    dxg = self.seg['dx'] if self.seg else float((x[-1] - x[0])/(x.size - 1))
-                    # MC3B_MOM_LAYOUT=1: Pe, Po as FP64 tensor-core products (k_sinemma) instead of
-                    # FMAs (k_sinefold<MOM>): correct, measured slower (0.127 against 0.099 ms at config 2)
-                    layout = int(os.environ.get('MC3B_MOM_LAYOUT', 0))
-                    _lib.call('mc3b_moment_prepare', kd.data_ptr(), nfold//128, float(x[0]), dxg,
-                              self.d_tile_x.data_ptr() if self.seg else None, c0r, slr, layout,
-                              self.d_mfold.data_ptr(), self.d_mtiles.data_ptr(), _lib.stream_ptr())
-                M = _lib.MomentStruct()
-                M.folded, M.tiles = self.d_mfold.data_ptr(), self.d_mtiles.data_ptr()
-                M.c0ref, M.slref, M.d2tot = c0r, slr, d2tot
-                M.amp_max = float(os.environ.get('MC3B_MOMENT_AMP', 4000.0))
-                M.xlo, M.xhi = float(x.min()), float(x.max())
-                M.guard_hits = self.guard_hits.data_ptr()
-                M.layout = layout
-                # ... and, where it applies, the spectral form of the same sum (k_spectral_chisq,
-                # include/mc3b200.h mc3b_spectral_t): chi-squared from a precomputed spectrum of the
-                # data, O(1) per chain instead of O(n).  Not with a period band that reaches 0,
-                # beyond the table's caps (spectral.plan), with the k_sinemma layout or with
-                # MC3B_NO_SPECTRAL=1: k_sinefold<MOM> as above.
-                self.spectral = None
-                wband = spectral.band(self.params, self.pstep, self.pmin, self.pmax)
-                plan = spectral.plan(float(x.min()), float(x.max()), *wband, x.size) \
-                    if wband is not None and layout == 0 and not os.environ.get('MC3B_NO_SPECTRAL') else None
-                if plan is not None:
-                    S = _lib.SpectralStruct()
-                    S.w1, S.w2, S.delta, S.xc = plan['w1'], plan['w2'], plan['delta'], plan['xc']
-                    S.n1, S.n2, S.order = plan['n1'], plan['n2'], plan['order']
-                    size = ctypes.c_int64(0)
-                    _lib.call('mc3b_spectral_size', S.n1, S.n2, S.order, ctypes.byref(size))
-                    with torch.cuda.device(self.dev):
-                        self.d_spectral = torch.zeros(size.value, **f64)
-                        S.table = self.d_spectral.data_ptr()
-                        _lib.call('mc3b_spectral_prepare', kx.data_ptr(), kd.data_ptr(), x.size, c0r, slr,
-                                  ctypes.byref(S), _lib.stream_ptr())
-                    self.spectral = S
-                    self.spectral_plan = plan
-                    M.spectral = ctypes.pointer(S)
-                # the guard count of every generation, written by the fused epilogue into
-                # page-locked host memory (include/mc3b200.h mc3b_moment_t.record)
-                with torch.cuda.device(self.dev):
-                    self._guard_ring = torch.empty(_lib.GUARD_RECORDS, dtype=torch.int64).pin_memory()
-                    dptr = ctypes.c_void_p()
-                    _lib.call('mc3b_host_device_pointer', self._guard_ring.data_ptr(), ctypes.byref(dptr))
-                M.record = dptr.value
-                self._guard = GuardRecords(self._guard_ring.numpy())
-                self.moment = M
-                self.use_moment = True
-            if self.dtype == _lib.F32:
-                self.k_x, self.k_d, self.k_w = (t.float().contiguous() for t in
-                                                (self.d_x, self.d_data, self.d_invsig))
-                self.k_xs = [self.k_x] + [t.float().contiguous() for t in self.d_xs[1:]]
-            else:
-                self.k_x, self.k_d, self.k_w = kx, kd, kw
-                self.k_xs = [self.k_x] + self.d_xs[1:]
+            x = self._stage_model(func, lo, hi)
+            form = choose_form(func, x, uncert, self.dtype, self.params, self.pstep, self.pmin, self.pmax)
+            self.usig, self.grid, self.seg = form.usig, form.grid, form.seg
+            self.chisq_model_id, self.spectral_plan = form.model_id, form.spectral_plan
+            kx, kd, kw = self._prepare_seg(x) if form.seg is not None else (self.d_x, self.d_data, self.d_invsig)
+            if form.fold:                  # the mirrored-pair copy of the data (k_sinefold)
+                self.d_fold = torch.zeros_like(kd)
+                _lib.call('mc3b_fold_data', kd.data_ptr(), form.nfold, self.d_fold.data_ptr(),
+                          _lib.stream_ptr())
+            if form.moment:
+                # least-squares line through the data and the sum of squares about it, on the device (a few
+                # small kernels and one read of three numbers).  Its temporaries live until the constructor
+                # returns: where the later buffers land moved the generation kernel's time by 5% on a B200
+                xm, dm = self.d_x.mean(), self.d_data.mean()
+                xc = self.d_x - xm
+                slr_t = torch.dot(xc, self.d_data - dm)/torch.dot(xc, xc)
+                c0r_t = dm - slr_t*xm
+                res = self.d_data - (c0r_t + slr_t*self.d_x)
+                line = [float(v) for v in torch.stack([c0r_t, slr_t, torch.dot(res, res)]).cpu()]
+                self._prepare_moment(x, kx, kd, form, *line)
+            # what the chi-squared kernels read: the arrays of the form, or fp32 copies
+            cast = (lambda t: t.float().contiguous()) if self.dtype == _lib.F32 else (lambda t: t)
+            self.k_x, self.k_d, self.k_w = cast(kx), cast(kd), cast(kw)
+            self.k_xs = [self.k_x] + [cast(t) for t in self.d_xs[1:]]
             self.k_xptrs = _lib.ptrs(self.k_xs)
-            self.k_kc = self.d_kc.float() if self.d_kc is not None and self.dtype == _lib.F32 else self.d_kc
-        elif self.shard == 'data':
-            raise ValueError("shard='data' needs a built-in model")
+            self.k_kc = None if self.d_kc is None else cast(self.d_kc)
         elif isinstance(func, TorchModel):
             self.kind = 'torch'
             self.t_indparams = [torch.as_tensor(a, device=self.dev)
@@ -457,6 +326,8 @@ class Population:
         self.gen_dev = torch.zeros(1, dtype=torch.int64, device=self.dev)
         self.gen = 0                      # generations completed
         self.first_valid = self.M0        # first history row that is a chain sample
+        self.resumed_rows, self.resumed_accept = None, 0     # of a resumed run (mcmc_driver._resume)
+        self._gathered_k = 0              # thinned steps complete on every device (gather_history)
         self.bestp0 = np.copy(params)     # best of the initial population
         self.best_log_post0 = -np.inf
 
@@ -472,6 +343,7 @@ class Population:
         # launch: identical chi-squared bits however the population is spread over
         # launches / devices (include/mc3b200.h, mc3b_chisq_opts_t)
         self.plan_chains = int(plan_chains) if plan_chains else 0
+        self._plan_rows = 0
         # Metropolis step fused into the tail of the model kernel (2 launches per
         # generation instead of 4); MC3B_NO_FUSE=1 keeps the separate kernels
         self.fused = (self.kind in ('builtin', 'cuda') and not self.wlike and self.shard == 'chains'
@@ -481,6 +353,89 @@ class Population:
         self.set_jump_scales(fgamma, fepsilon)
         self.S.reflect = 1 if reflect else 0
         self.launches = 0                 # kernels launched by this object
+
+    def _stage_model(self, func, lo, hi):
+        """The model's inputs (d_x, d_xs), constants (d_kc) and 1/uncert on the device; returns the local x."""
+        user = isinstance(func, CudaModel)
+        self.kind = 'cuda' if user else 'builtin'
+        self.nmodel = func.nmodel(self.nfunc)
+        self.jit = func.handle(self.dtype) if user else None
+        # model values are fp64 whatever the dtype, as mc3b_model_eval's
+        self.jit_eval = func.handle(_lib.F64) if user else None
+        nin = func.ninputs if user else 1
+        # a CudaModel of run-time constants: the indparams after its inputs, flattened
+        # (CudaModel.split_args); every rank builds its own copy
+        xargs, kc = func.split_args(self.indparams) if user else (self.indparams, None)
+        if nin > 1:
+            # a CudaModel of several inputs: one 1-D array per input, in the order of
+            # the arguments of its `model`
+            xin = [np.ascontiguousarray(a, dtype=np.double) for a in xargs]
+            if len(xin) != nin or any(a.ndim != 1 or a.size != self.ndata_total for a in xin):
+                raise ValueError(f'CudaModel {func.name!r} takes {nin} inputs: it needs indparams=[x1, ..., '
+                                 f'x{nin}], {nin} 1-D arrays with the same shape as data (got '
+                                 f'{[np.shape(a) for a in self.indparams]} for data of {self.ndata_total})')
+        x = np.ascontiguousarray(self.indparams[0], dtype=np.double)
+        if x.size != self.ndata_total or x.ndim != 1:
+            raise ValueError(f'{"CUDA" if user else "built-in"} models need indparams=[x] '
+                             'with the same shape as data')
+        x = x[lo:hi]
+        self.d_x = torch.from_numpy(x).to(self.dev)
+        # every input of the model on the device (d_xs[0] is d_x); their host array of
+        # pointers is what mc3b_user_model_eval_consts takes
+        self.d_xs = [self.d_x] + [torch.from_numpy(a[lo:hi]).to(self.dev) for a in xin[1:]] \
+            if nin > 1 else [self.d_x]
+        self.d_xptrs = _lib.ptrs(self.d_xs)
+        # ... and its constants, fp64 (model values) and in the kernel's dtype; None: none
+        self.d_kc = torch.from_numpy(kc).to(self.dev) if kc is not None and kc.size else None
+        self.nconst = func.nconst if user else 0
+        self.d_invsig = 1.0/self.d_uncert
+        return x
+
+    def _prepare_seg(self, x):
+        """(x, data, 1/uncert) in the seg layout (include/mc3b200.h, tile_x), and the tiles' origins."""
+        perm = torch.from_numpy(self.seg['perm']).to(self.dev)
+        kx, kd = self.d_x[perm].contiguous(), self.d_data[perm].contiguous()
+        kw = self.d_invsig if self.usig else self.d_invsig[perm].contiguous()
+        self.d_tile_x = torch.from_numpy(np.ascontiguousarray(x[self.seg['starts']])).to(self.dev)
+        return kx, kd, kw
+
+    def _prepare_moment(self, x, kx, kd, form, c0r, slr, d2tot):
+        """The moment form about the data's least-squares line c0r + slr x (sum of squares d2tot about
+        it), which keeps the cancellation of the expansion at (signal/noise)^2: the mirrored pairs' sums,
+        guard records and spectral table.  A guard in the kernel re-evaluates every chain the expansion
+        is not accurate enough for; when that is not rare (_moment_policy) the pair kernel takes over."""
+        self.d_mfold = torch.zeros_like(kd)
+        self.d_mtiles = torch.zeros((max(form.nfold//128, 1), 4), dtype=torch.float64, device=self.dev)
+        self.guard_hits = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        dxg = self.seg['dx'] if self.seg else float((x[-1] - x[0])/(x.size - 1))
+        _lib.call('mc3b_moment_prepare', kd.data_ptr(), form.nfold//128, float(x[0]), dxg, _lib.ptr(self.d_tile_x),
+                  c0r, slr, form.layout, self.d_mfold.data_ptr(), self.d_mtiles.data_ptr(), _lib.stream_ptr())
+        if form.spectral_plan is not None:
+            self._prepare_spectral(form.spectral_plan, kx, kd, c0r, slr)
+        # the guard count of every generation, written by the fused epilogue into
+        # page-locked host memory (include/mc3b200.h mc3b_moment_t.record)
+        self._guard_ring = torch.empty(_lib.GUARD_RECORDS, dtype=torch.int64).pin_memory()
+        dptr = ctypes.c_void_p()
+        _lib.call('mc3b_host_device_pointer', self._guard_ring.data_ptr(), ctypes.byref(dptr))
+        self._guard = GuardRecords(self._guard_ring.numpy())
+        self.moment = _lib.MomentStruct(
+            folded=self.d_mfold.data_ptr(), tiles=self.d_mtiles.data_ptr(), c0ref=c0r, slref=slr, d2tot=d2tot,
+            amp_max=float(os.environ.get('MC3B_MOMENT_AMP', 4000.0)), xlo=float(x.min()), xhi=float(x.max()),
+            guard_hits=self.guard_hits.data_ptr(), layout=form.layout, record=dptr.value,
+            spectral=None if self.spectral is None else ctypes.pointer(self.spectral))
+        self.use_moment = True
+
+    def _prepare_spectral(self, plan, kx, kd, c0r, slr):
+        """The spectral form's table: the data's spectrum on the nodes of `plan` (spectral.plan), from
+        which the chi-squared of a chain takes O(1) instead of O(n)."""
+        S = _lib.SpectralStruct(**{k: plan[k] for k in ('w1', 'w2', 'delta', 'xc', 'n1', 'n2', 'order')})
+        size = ctypes.c_int64(0)
+        _lib.call('mc3b_spectral_size', S.n1, S.n2, S.order, ctypes.byref(size))
+        self.d_spectral = torch.zeros(size.value, dtype=torch.float64, device=self.dev)
+        S.table = self.d_spectral.data_ptr()
+        _lib.call('mc3b_spectral_prepare', kx.data_ptr(), kd.data_ptr(), self.ndata, c0r, slr,
+                  ctypes.byref(S), _lib.stream_ptr())
+        self.spectral = S
 
     # ------------------------------------------------------------------
     def _make_struct(self):
@@ -562,7 +517,7 @@ class Population:
         batch, the initial-population trials, is evaluated in per-device blocks)."""
         if not self.plan_chains:
             return nb
-        return max(self.plan_chains, getattr(self, '_plan_rows', 0), nb)
+        return max(self.plan_chains, self._plan_rows, nb)
 
     def _plan(self, nb, kind=0):
         """kind: 0 general, 1 moment form, 2 its spectral form (MC3B_PLAN_*)."""
@@ -582,23 +537,26 @@ class Population:
         return t
 
     def _model_rows(self, P):
-        """Model values [nb, N] on the device for non-built-in models."""
-        if self.kind == 'cuda':
-            rows = self._workspace(('mrows', P.shape[0]), (P.shape[0], self.ndata))
-            _lib.call('mc3b_user_model_eval_consts', self.jit_eval, P.data_ptr(), _lib.ld(P), P.shape[0],
-                      self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst, self.ndata,
-                      rows.data_ptr(), _lib.stream_ptr())
+        """Model values [nb, N] on the device."""
+        nb = P.shape[0]
+        if self.kind in ('builtin', 'cuda'):
+            rows = self._workspace(('mrows', nb), (nb, self.ndata))
+            if self.kind == 'cuda':
+                _lib.call('mc3b_user_model_eval_consts', self.jit_eval, P.data_ptr(), _lib.ld(P), nb,
+                          self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst, self.ndata,
+                          rows.data_ptr(), _lib.stream_ptr())
+            else:
+                _lib.call('mc3b_model_eval', self.func.model_id, P.data_ptr(), _lib.ld(P), nb,
+                          self.nmodel, self.d_x.data_ptr(), self.ndata, rows.data_ptr(), _lib.stream_ptr())
             self.launches += 1
             return rows
         if self.kind == 'torch':
-            Pm = P[:, :self.nfunc]
-            m = self.func.fn(Pm, *self.t_indparams, **self.indparams_dict)
+            m = self.func.fn(P[:, :self.nfunc], *self.t_indparams, **self.indparams_dict)
             return m.to(torch.float64).contiguous()
         Ph = P.cpu().numpy()
-        rows = np.empty((Ph.shape[0], self.ndata))
-        for i in range(Ph.shape[0]):     # the reference's per-chain host callable
-            rows[i] = self.func(Ph[i, :self.nfunc], *self.indparams,
-                                **self.indparams_dict)
+        rows = np.empty((nb, self.ndata))
+        for i in range(nb):     # the reference's per-chain host callable
+            rows[i] = self.func(Ph[i, :self.nfunc], *self.indparams, **self.indparams_dict)
         return torch.from_numpy(rows).to(self.dev)
 
     @on_device
@@ -643,94 +601,83 @@ class Population:
         return allsum, nb, self.world
 
     def _data_chisq_local(self, P, fuse=None, moment_ok=False):
-        nb = P.shape[0]
         self._part_is_moment = False
-        st = _lib.stream_ptr()
         if self.wlike:
-            out = self._workspace(('dwt', nb), (1, nb))
-            ws_bytes = _lib.load().mc3b_dwt_workspace(nb, self.ndata)
-            ws = self._workspace(('dwtws', nb), (max(ws_bytes, 8)//8,))
-            if self.kind == 'builtin':
-                _lib.call('mc3b_dwt_chisq', self.func.model_id, P.data_ptr(),
-                          _lib.ld(P), nb, self.npars, self.nmodel,
-                          self.d_x.data_ptr(), None, 0, self.d_data.data_ptr(),
-                          self.ndata, ws.data_ptr(), out.data_ptr(), st)
-            elif self.kind == 'cuda':
-                # the model is evaluated inside the D4 kernels of its fp64 module: no rows
-                _lib.call('mc3b_user_model_dwt_chisq', self.jit_eval, P.data_ptr(), _lib.ld(P), nb,
-                          self.npars, self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst,
-                          self.d_data.data_ptr(), self.ndata, ws.data_ptr(), out.data_ptr(), st)
-            else:
-                m = self._model_rows(P)
-                _lib.call('mc3b_dwt_chisq', -1, P.data_ptr(), _lib.ld(P), nb,
-                          self.npars, 0, None, m.data_ptr(), _lib.ld(m),
-                          self.d_data.data_ptr(), self.ndata, ws.data_ptr(),
-                          out.data_ptr(), st)
-            self.launches += 2
-            return out, nb, 1
+            return self._wavelet_chisq(P)
         if self.kind in ('builtin', 'cuda'):
-            moment = bool(getattr(self, 'use_moment', False)) and self.d_fold is not None \
-                and (fuse is not None or moment_ok)
-            spec = moment and self.moment.spectral
-            ns = self._plan(nb, 2 if spec else 1 if moment else 0)
-            part = self._workspace(('part', nb, ns), (ns, nb))
-            self._last_part = part
-            o = _lib.ChisqOpts()
-            o.plan_chains = self._plan_chains(nb) if self.plan_chains else 0
-            o.uniform_sigma = 1 if self.usig else 0
-            if self.seg is not None:
-                o.tile_x, o.dx = self.d_tile_x.data_ptr(), self.seg['dx']
-                o.ntiles = self.seg['starts'].size
-            if self.d_fold is not None:
-                o.folded = self.d_fold.data_ptr()
-                if (not os.environ.get('MC3B_NO_FOLD_CONSTS') or moment) and not spec:
-                    o.work = self._workspace(('foldk', nb), (_lib.FOLD_WORK, nb)).data_ptr()
-                    self.launches += 1
-                if moment:
-                    o.moment = ctypes.pointer(self.moment)
-                    self._part_is_moment = fuse is None
-            if fuse is not None:
-                o.c_off, o.gen, o.zrow0, adv = fuse
-                o.advance = 1 if adv else 0
-                o.fuse = ctypes.pointer(self.S)
-                o.fuse_done = self.fuse_done.data_ptr()
-            if self.kind == 'cuda':
-                _lib.call('mc3b_user_model_chisq_consts', self.jit, P.data_ptr(), _lib.ld(P), nb,
-                          self.k_xptrs, len(self.k_xs), _lib.ptr(self.k_kc), self.nconst,
-                          self.k_d.data_ptr(), self.k_w.data_ptr(),
-                          self.ndata, part.data_ptr(), nb, ns, ctypes.byref(o), st)
-            else:
-                _lib.call('mc3b_model_chisq_ex', self.chisq_model_id, self.dtype,
-                          P.data_ptr(), _lib.ld(P), nb, self.nmodel,
-                          self.k_x.data_ptr(), self.k_d.data_ptr(),
-                          self.k_w.data_ptr(), self.ndata, part.data_ptr(), nb, ns,
-                          ctypes.byref(o), st)
-            self.launches += 1
-            return part, nb, ns
-        m = self._model_rows(P)
+            return self._model_chisq(P, fuse, moment_ok)
+        nb, m = P.shape[0], self._model_rows(P)
         out = self._workspace(('rows', nb), (1, nb))
-        _lib.call('mc3b_chisq_batch', m.data_ptr(), _lib.ld(m), nb,
-                  self.d_data.data_ptr(), self.d_uncert.data_ptr(), self.ndata,
-                  out.data_ptr(), st)
+        _lib.call('mc3b_chisq_batch', m.data_ptr(), _lib.ld(m), nb, self.d_data.data_ptr(),
+                  self.d_uncert.data_ptr(), self.ndata, out.data_ptr(), _lib.stream_ptr())
         self.launches += 1
         return out, nb, 1
+
+    def _wavelet_chisq(self, P):
+        """The wavelet likelihood (csrc/dwt.cu): one row of sums."""
+        nb = P.shape[0]
+        st = _lib.stream_ptr()
+        out = self._workspace(('dwt', nb), (1, nb))
+        ws_bytes = _lib.load().mc3b_dwt_workspace(nb, self.ndata)
+        ws = self._workspace(('dwtws', nb), (max(ws_bytes, 8)//8,))
+        if self.kind == 'builtin':
+            _lib.call('mc3b_dwt_chisq', self.func.model_id, P.data_ptr(), _lib.ld(P), nb, self.npars, self.nmodel,
+                      self.d_x.data_ptr(), None, 0, self.d_data.data_ptr(), self.ndata, ws.data_ptr(),
+                      out.data_ptr(), st)
+        elif self.kind == 'cuda':
+            # the model is evaluated inside the D4 kernels of its fp64 module: no rows
+            _lib.call('mc3b_user_model_dwt_chisq', self.jit_eval, P.data_ptr(), _lib.ld(P), nb,
+                      self.npars, self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst,
+                      self.d_data.data_ptr(), self.ndata, ws.data_ptr(), out.data_ptr(), st)
+        else:
+            m = self._model_rows(P)
+            _lib.call('mc3b_dwt_chisq', -1, P.data_ptr(), _lib.ld(P), nb, self.npars, 0, None, m.data_ptr(),
+                      _lib.ld(m), self.d_data.data_ptr(), self.ndata, ws.data_ptr(), out.data_ptr(), st)
+        self.launches += 2
+        return out, nb, 1
+
+    def _model_chisq(self, P, fuse, moment_ok):
+        """The model + chi-squared kernel of a built-in or CUDA model in the population's form."""
+        nb = P.shape[0]
+        moment = self.use_moment and (fuse is not None or moment_ok)
+        spec = moment and self.spectral is not None
+        ns = self._plan(nb, 2 if spec else 1 if moment else 0)
+        part = self._last_part = self._workspace(('part', nb, ns), (ns, nb))
+        o = _lib.ChisqOpts()
+        o.plan_chains = self._plan_chains(nb) if self.plan_chains else 0
+        o.uniform_sigma = 1 if self.usig else 0
+        if self.seg is not None:
+            o.tile_x, o.dx, o.ntiles = self.d_tile_x.data_ptr(), self.seg['dx'], self.seg['starts'].size
+        if self.d_fold is not None:
+            o.folded = self.d_fold.data_ptr()
+            if (not os.environ.get('MC3B_NO_FOLD_CONSTS') or moment) and not spec:
+                o.work = self._workspace(('foldk', nb), (_lib.FOLD_WORK, nb)).data_ptr()
+                self.launches += 1
+        if moment:
+            o.moment = ctypes.pointer(self.moment)
+            self._part_is_moment = fuse is None
+        if fuse is not None:
+            o.c_off, o.gen, o.zrow0, adv = fuse
+            o.advance = 1 if adv else 0
+            o.fuse = ctypes.pointer(self.S)
+            o.fuse_done = self.fuse_done.data_ptr()
+        if self.kind == 'cuda':
+            _lib.call('mc3b_user_model_chisq_consts', self.jit, P.data_ptr(), _lib.ld(P), nb, self.k_xptrs,
+                      len(self.k_xs), _lib.ptr(self.k_kc), self.nconst, self.k_d.data_ptr(), self.k_w.data_ptr(),
+                      self.ndata, part.data_ptr(), nb, ns, ctypes.byref(o), _lib.stream_ptr())
+        else:
+            _lib.call('mc3b_model_chisq_ex', self.chisq_model_id, self.dtype, P.data_ptr(), _lib.ld(P), nb,
+                      self.nmodel, self.k_x.data_ptr(), self.k_d.data_ptr(), self.k_w.data_ptr(), self.ndata,
+                      part.data_ptr(), nb, ns, ctypes.byref(o), _lib.stream_ptr())
+        self.launches += 1
+        return part, nb, ns
 
     @on_device
     def model_eval(self, fpar):
         """Built-in or CUDA model at one parameter vector over the (device-resident)
         abscissa, as a host array (chain.py:316-319 `func(params, *indparams)`)."""
         P = torch.as_tensor(np.atleast_2d(np.asarray(fpar, dtype=np.double)), device=self.dev)
-        out = torch.empty((1, self.ndata), dtype=torch.float64, device=self.dev)
-        if self.kind == 'cuda':
-            _lib.call('mc3b_user_model_eval_consts', self.jit_eval, P.data_ptr(), P.shape[1], 1,
-                      self.d_xptrs, len(self.d_xs), _lib.ptr(self.d_kc), self.nconst, self.ndata,
-                      out.data_ptr(), _lib.stream_ptr())
-        else:
-            _lib.call('mc3b_model_eval', self.func.model_id, P.data_ptr(), P.shape[1], 1,
-                      self.nmodel, self.d_x.data_ptr(), self.ndata, out.data_ptr(),
-                      _lib.stream_ptr())
-        self.launches += 1
-        return to_host(out[0])
+        return to_host(self._model_rows(P)[0])
 
     @on_device
     def chisq(self, P):
@@ -921,7 +868,7 @@ class Population:
             use_graph = self.kind in ('builtin', 'cuda') and not heavy and not \
                 (self.world > 1 and self.shard == 'chains' and self.sampler == 'snooker'
                  and self.p2p is None)
-        if getattr(self, 'use_moment', False):
+        if self.use_moment:
             # the persistent small-population kernel never runs the moment form, and
             # unfused generations write no guard records
             self._moment_policy(ngen, self.fused and not (use_graph and self.small))
@@ -1055,7 +1002,7 @@ class Population:
         if self.shard == 'data' or self.world == 1:
             return
         K = self.thinned_done()
-        k0 = getattr(self, '_gathered_k', 0)      # thinned steps complete everywhere
+        k0 = self._gathered_k
         if K <= k0:
             return
         lo = self.M0 + k0*self.nchains
@@ -1101,7 +1048,7 @@ class Population:
         ev.synchronize()
         h = host.numpy()
         nf = self.nfree
-        numaccept = int(round(h[:, 0].sum())) + getattr(self, 'resumed_accept', 0)
+        numaccept = int(round(h[:, 0].sum())) + self.resumed_accept
         outbounds = np.rint(h[:, 4 + nf:4 + 2*nf].sum(axis=0)).astype(int)
         best_chisq = -2.0*self.best_log_post0
         bestp = np.copy(self.bestp0)
